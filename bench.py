@@ -16,7 +16,10 @@ sides of its own x-interval; per-cell partial sums / arg-max come home through O
 (every GPU owns a full 1024x1024 shard of a wider grid) is measured in the same run and reported as `other_scaling`;
 `--scaling weak|strong` forces one mode for `value`.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c4|c3|c2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c4|c3|c2] [--dump-outputs DIR]
+
+`--dump-outputs DIR` writes what the last timed step returned to its caller as DIR/<name>.npy (float64, at most 64 MB in
+all); the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -55,6 +58,18 @@ POSTERIOR_TRAFFIC_C4_1GPU = 18.883344e9 + 39.72864e6
 CHOL_TRAFFIC_C4_1GPU = 96.788829e6 + 46.284102e6
 DGEMM_PEAK_TFLOPS = 35.41   # cuBLAS DGEMM 8192^3 measured on this pool's B200 (profiles/r01_dgemm_peak.json);
 #                             MEASURED_PEAKS.json carries no FP64 figure.  DMMA issue peak: 37.15 (r01_fp64_pipes.log)
+DUMP_LIMIT = 64 << 20       # bytes written by --dump-outputs, all arrays together
+
+
+def dump_outputs(path, arrays):
+    """Writes every array as path/<name>.npy in float64."""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit(f"bench: --dump-outputs would write {total} bytes, more than {DUMP_LIMIT}")
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
 
 
 def make_workload(name, world=1, rank=0, scaling="weak"):
@@ -290,10 +305,10 @@ def run_ours(args):
             self.eng.refactor(check=False)         # the reference refits every iteration (simulator.py:888-891): factor stale
             if world == 1:
                 loss, cent, axy, mv, _, _ = self.state.step(self.model, w["pos"], w["cen"])
-                out = (loss, cent, axy)
+                out = (loss, cent, axy, mv)
             else:
                 loss, cent, idx, mv = self.state.step(self.model, w["pos"], w["cen"])
-                out = (loss, cent, idx)
+                out = (loss, cent, idx, mv)
             if timed and self.eng.profile_events[1].query():
                 try:
                     self.chol_ms.append(self.eng.profile_events[0].elapsed_time(self.eng.profile_events[1]))
@@ -321,6 +336,10 @@ def run_ours(args):
     clocks = sampler.result()
     chk = min(npts, 1 << 16)
     mu_timed, var_timed = arm.state.mu[:chk].cpu().numpy(), arm.state.var[:chk].cpu().numpy()      # results of the last TIMED step
+    if args.dump_outputs and rank == 0:         # N > 1: mu / var of rank 0's grid slice, the merged per-cell results
+        dump_outputs(args.dump_outputs, {"mu": arm.state.mu.cpu().numpy(), "var": arm.state.var.cpu().numpy(), "loss": out[0],
+                                         "centroids": out[1], "argmax_xy" if world == 1 else "argmax_index": out[2],
+                                         "max_var": out[3]})
     plan = eng._fplan[1] if eng._fplan is not None else None
 
     # the other scaling mode at N > 1, reported inside the same line (never as `value`)
@@ -589,6 +608,8 @@ def run_ours(args):
 C5 = dict(n=64, agents=8, iterations=120, lattice=6, sigma_n=0.1, total_runs=512,
           desc="c5: replicate sweep, independent periodic_hmf runs on 64x64 (4096-point) grids, 8 agents, 120 iterations, "
                "36-point lofi prior lattice (512 runs in the full sweep; a step is ONE whole run)")
+C5_AGENT_COLS = ("X", "Y", "XMax", "YMax", "VarMax", "Var0", "XCentroid", "YCentroid", "ProbExplore", "Explore", "Distance")
+C5_DUMP_RUNS = 256          # --dump-outputs keeps the logs of at most this many runs: 512 whole runs exceed DUMP_LIMIT
 
 
 def c5_inputs():
@@ -599,6 +620,20 @@ def c5_inputs():
     near = np.argmin(((xy[None, :, :] - lat[:, None, :]) ** 2).sum(axis=2), axis=1)
     prior_arr = np.column_stack((lat, 0.8 * truth_arr[near, 2] + 0.02))
     return truth_arr, prior_arr
+
+
+def c5_log_arrays(logs):
+    """The (loss_log, agent_log, sample_log) rows of the timed runs as arrays, for a fixed, seeded sample of at most
+    C5_DUMP_RUNS runs: runs[R'] (the sampled run indices), loss[R', T], agent[R', T, A, 11] (the numeric columns of an
+    agent row, in C5_AGENT_COLS order), samples[S, 6] (run index, Iteration, Agent, X, Y, Sample)."""
+    R, T = len(logs), len(logs[0][0])
+    runs = np.arange(R) if R <= C5_DUMP_RUNS else np.sort(np.random.default_rng(0).choice(R, C5_DUMP_RUNS, replace=False))
+    num = lambda v: np.nan if isinstance(v, str) else float(v)       # noqa: E731   ("NA" cells of the reference's rows)
+    loss = [[num(r["Loss"]) for r in logs[k][0]] for k in runs]
+    agent = [[[num(r[c]) for c in C5_AGENT_COLS] for r in logs[k][1]] for k in runs]
+    samples = [[k] + [num(r[c]) for c in ("Iteration", "Agent", "X", "Y", "Sample")] for k in runs for r in logs[k][2]]
+    return {"runs": runs, "loss": np.array(loss), "agent": np.array(agent).reshape(len(runs), T, -1, len(C5_AGENT_COLS)),
+            "samples": np.array(samples).reshape(-1, 6)}
 
 
 def run_c5(args):
@@ -675,6 +710,8 @@ def run_c5(args):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
     clocks = sampler.result()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, c5_log_arrays(logs))
     # the device loop alone, eager launches vs ONE CUDA graph replay (capture excluded), on fresh state each
     from mfgp_coverage_b200._batched import BatchedRuns
     loop_ms = {}
@@ -741,10 +778,16 @@ def main():
     ap.add_argument("--workload", default="c4", choices=sorted(WORKLOADS) + ["c5"])
     ap.add_argument("--scaling", default="strong", choices=["weak", "strong"],
                     help="N > 1: the fixed grid split over the GPUs (strong, default: BASELINE config 4) or a fixed per-GPU shard (weak)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned to DIR/<name>.npy (float64, at most 64 MB in all; --impl ours)")
     args = ap.parse_args()
     args.scaling_given = any(a.startswith("--scaling") for a in sys.argv[1:])
     if args.steps is None:      # c5: a step is one whole run and the runs of a rank are stepped together -> the full sweep
         args.steps = max(1, C5["total_runs"] // max(1, int(os.environ.get("WORLD_SIZE", "1")))) if args.workload == "c5" else 5
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the device path (--impl ours)")
     if args.workload == "c5":
         run_c5(args)
     elif args.impl == "reference":

@@ -1,12 +1,11 @@
 """The deterministic Choi tour planner that replaces mlrose's genetic algorithm (reference simulator.py:415-454): the CPU
-statement oracle/tsp.py (properties + optimality on small clusters + the LIVE reference routed through it) and, on the
-GPU, bit-identical tours from choi_tsp_tours (csrc/tsp.cu)."""
+statement oracle/tsp.py (properties + optimality on small clusters) and, on the GPU, bit-identical tours from
+choi_tsp_tours (csrc/tsp.cu)."""
 import itertools
 
 import numpy as np
 import pytest
 
-from oracle import reference_live as rl
 from oracle import tsp as otsp
 from tests import synth
 
@@ -55,20 +54,6 @@ def test_small_clusters_reach_the_optimal_closed_tour():
     assert np.all(steps > 0) or np.all(steps < 0)                 # convex position: the optimal tour is the hull order
     square = np.array([[0.0, 0.0], [1.0, 1.0], [1.0, 0.0], [0.0, 1.0]])
     assert abs(otsp.tour_length(square, otsp.plan_tour(square)) - 4.0) <= 1e-15
-
-
-@pytest.mark.skipif(not rl.available(), reason="/root/reference not present")
-def test_live_reference_compute_sample_tsp_runs_through_the_planner():
-    """The unmodified reference's compute_sample_tsp (simulator.py:415-454), with its mlrose import served by
-    oracle/refshim/mlrose, returns exactly the oracle's tours (cluster[solution] indexing included)."""
-    sim, _ = rl.load()
-    rng = np.random.default_rng(2)
-    clusters = _clusters(rng, (0, 1, 2, 7, 19), on_grid=True)
-    ref = sim.compute_sample_tsp(clusters)
-    mine = otsp.compute_sample_tsp(clusters)
-    assert len(ref) == len(mine) == 5
-    for a, b in zip(ref, mine):
-        assert a.shape == b.shape and np.array_equal(a, b)
 
 
 @pytest.mark.gpu

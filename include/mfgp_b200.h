@@ -317,7 +317,7 @@ int64_t choi_greedy(const double* Xs, int64_t G, double* Vc, int64_t ldv, int64_
  * Logs: log_loss[iterations], log_agent[iterations, A, 11] (X, Y, XMax, YMax, VarMax, Var0, XCentroid, YCentroid, ProbExplore,
  * Explore, Distance: the reference's agent row), log_sample[max_samples, 5] (Iteration, Agent, X, Y, Sample). */
 typedef struct mfgp_batch {
-    int64_t runs, G, nx, ny, A, NL, cap, algo /* 0 lloyd, 1 periodic, 2 todescato */, iterations, max_samples;
+    int64_t runs, G, nx, ny, A, NL, cap, algo /* 0 lloyd, 1 periodic, 2 todescato, 3 choi */, iterations, max_samples;
     double xmin, xmax, ymin, ymax, eps, tie_tol, amax_rel;
     const double* xy; const double* f; const double* ux; const double* uy;
     double* Xt; double* y; double* W; double* z;
@@ -329,6 +329,14 @@ typedef struct mfgp_batch {
     int32_t* Ncur; int32_t* knew; int32_t* status; int32_t* noise_used; int32_t* nsamples; int32_t* ties;
     const double* noise; const double* unif;
     double* log_loss; double* log_agent; double* log_sample;
+    /* Choi only (algo 3; NULL otherwise).  Planner: q[G] per run (variance reduction |W psi_g|^2 of the rows in use),
+     * picks[cap] (grid indices of the period's picks in selection order, planned rows Ncur + k), nplan (picks so far),
+     * plan_state (0 planning, 1 done, 2 stopped at cap: grow the buffers, reset to 0, resume), pmask[cap] (cells of each
+     * pick, bit c = agent c), ccount[A] (picks per cell), cties (picks within TIE_TOL/10 of a bisector in this period).
+     * Tours: tour_off[runs*A+1] (tour of (run r, agent c) = tour[tour_off[r*A+c] .. tour_off[r*A+c+1]), grid indices),
+     * tour_cur[runs*A] (next entry to visit). */
+    double* q; int64_t* picks; int32_t* nplan; int32_t* plan_state; int32_t* pmask; int32_t* ccount; int32_t* cties;
+    int32_t* tour_off; int32_t* tour_cur; int64_t* tour;
 } mfgp_batch;
 
 /* One iteration of every run: take the exploring agents' samples (:698-713), append them to the model by a block-bordered
@@ -337,6 +345,28 @@ typedef struct mfgp_batch {
  * write the log rows (:740-768), decide (:771-775, :942-943) and move (:777-782).  Three launches, no host involvement
  * between iterations: the whole run can be captured in one CUDA graph.  b_host / p_host are read on the host. */
 int mfgp_batch_step(const mfgp_batch* b_host, const mfgp_params* p_host, int64_t iteration, void* stream);
+
+/* ---- batched Choi (algo 3): per period plan (compute_sample_points :326-374), cluster (compute_sample_clusters :377-412)
+ *      and tours (compute_sample_tsp :415-454) for every run, then the period's iterations through mfgp_batch_step ---- */
+
+/* Start of a period: q[g] = |W psi_g|^2 over the rows [0, Ncur) of every run, nplan = 0, plan_state = 0 (1 for a stopped run). */
+int mfgp_batch_choi_begin(const mfgp_batch* b_host, const mfgp_params* p_host, void* stream);
+
+/* `rounds` pick rounds without a host synchronisation.  A round advances every planning run by one pick: first-index arg-max
+ * of k(0) - q with the tie rule of cov_argmax; if it exceeds `threshold`, the pick is appended to the run's factor as the
+ * temporary row Ncur + nplan (bordered update; Ncur, z, mu and var are not touched) and q += v^2 with v the new row of
+ * W Psi.  A run whose rows would exceed cap stops with plan_state 2; a non-positive pivot sets status (as the stepper). */
+int mfgp_batch_choi_plan(const mfgp_batch* b_host, const mfgp_params* p_host, double threshold, int64_t rounds, void* stream);
+
+/* Cells of every pick in the partition seeded by cen (device-clipped bounded Voronoi cells; nearest seed, the crossings
+ * test within TIE_TOL of a bisector): pmask, ccount, cties. */
+int mfgp_batch_choi_cluster(const mfgp_batch* b_host, void* stream);
+
+/* Tours of all runs x agents: the clusters (picks of a cell in selection order) are gathered at b->tour_off (the caller's
+ * prefix sum of ccount, n_total entries, largest n_max) into pts[n_total,2] / gidx[n_total], ordered by choi_tsp_tours
+ * into ord[n_total] (work / work_bytes: as choi_tsp_tours), and stored as grid indices in b->tour; tour_cur = tour_off. */
+int mfgp_batch_choi_tours(const mfgp_batch* b_host, int64_t n_total, int64_t n_max, double* pts, int64_t* gidx, int32_t* ord,
+                          void* work, int64_t work_bytes, void* stream);
 
 /* ---- hyper-parameter training: replaces SFGP.likelihood / MFGP.likelihood gaussian_process.py:81-105, :344-384 and the
  *      autograd gradient behind SFGP.train / MFGP.train :107-119, :386-399 ------------------------------------------- */

@@ -29,7 +29,9 @@ class MfgpBatch(Structure):      # struct mfgp_batch (include/mfgp_b200.h)
                [(n, c_double) for n in ("xmin", "xmax", "ymin", "ymax", "eps", "tie_tol", "amax_rel")] + \
                [(n, c_void_p) for n in ("xy", "f", "ux", "uy", "Xt", "y", "W", "z", "TxL", "TyL", "TxH", "TyH", "mu", "var", "pos",
                                         "prev", "cen", "pos_idx", "prob", "explore", "Ncur", "knew", "status", "noise_used",
-                                        "nsamples", "ties", "noise", "unif", "log_loss", "log_agent", "log_sample")]
+                                        "nsamples", "ties", "noise", "unif", "log_loss", "log_agent", "log_sample",
+                                        "q", "picks", "nplan", "plan_state", "pmask", "ccount", "cties", "tour_off", "tour_cur",
+                                        "tour")]
 
 
 # name -> (restype, argtypes); this table is also what tests/test_abi.py checks against include/mfgp_b200.h
@@ -127,6 +129,11 @@ SIGNATURES = {
                               POINTER(MfgpParams), c_double, c_double, c_int64, POINTER(c_int64), c_void_p, c_int64,
                               c_void_p]),
     "mfgp_batch_step": (c_int, [POINTER(MfgpBatch), POINTER(MfgpParams), c_int64, c_void_p]),
+    "mfgp_batch_choi_begin": (c_int, [POINTER(MfgpBatch), POINTER(MfgpParams), c_void_p]),
+    "mfgp_batch_choi_plan": (c_int, [POINTER(MfgpBatch), POINTER(MfgpParams), c_double, c_int64, c_void_p]),
+    "mfgp_batch_choi_cluster": (c_int, [POINTER(MfgpBatch), c_void_p]),
+    "mfgp_batch_choi_tours": (c_int, [POINTER(MfgpBatch), c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int64,
+                                      c_void_p]),
     "mfgp_nlml_workspace_bytes": (c_int64, [c_int64]),
     "mfgp_nlml_grad": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_int64, c_int64,
                                POINTER(MfgpParams), c_void_p, c_void_p, c_int64, c_void_p]),

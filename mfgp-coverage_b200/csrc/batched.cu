@@ -49,6 +49,9 @@ struct BatchArgs {
     int* ties;                                                           // [runs][iterations]
     const double* noise; const double* unif;                             // [runs][max_samples], [runs][iterations][A]
     double* log_loss; double* log_agent; double* log_sample;             // [runs][it], [runs][it][A][BT_LOGC], [runs][max_samples][5]
+    double* q; long long* picks; int* nplan; int* plan_state;            // Choi planner: [runs][G], [runs][cap], [runs], [runs]
+    int* pmask; int* ccount; int* cties;                                 // Choi clusters: [runs][cap], [runs][A], [runs]
+    int* tour_off; int* tour_cur; long long* tour;                       // Choi tours: [runs*A+1], [runs*A], [tour_off[runs*A]]
 };
 
 __device__ __forceinline__ double warp_sum_d(double v) {
@@ -470,18 +473,267 @@ __global__ void __launch_bounds__(BT_THREADS) batch_coverage_kernel(BatchArgs a,
         row[6] = cx; row[7] = cy; row[8] = a.prob[r * A + i]; row[9] = (double)a.explore[r * A + i]; row[10] = dist;
         int ex = 0;
         double pr = 0.0;
+        long long tgi = -1;
         if (a.algo == 1) { ex = ((it / 5) % 2 == 0) ? 1 : 0; pr = (double)ex; }
         else if (a.algo == 2) {
             pr = sqrt(mv / (a.p.k0 * (double)A));              // todescato_prob, simulator.py:457-467
             ex = a.unif[((int64_t)r * a.iterations + it) * A + i] < pr ? 1 : 0;
         }
+        else if (a.algo == 3) {          // Choi: explore while the tour has points left, visit its next point (simulator.choi)
+            const int k = r * A + i, cur = a.tour_cur[k];
+            ex = cur < a.tour_off[k + 1] ? 1 : 0;
+            pr = (double)ex;
+            if (ex) { tgi = a.tour[cur]; a.tour_cur[k] = cur + 1; }
+        }
         a.prob[r * A + i] = pr;
         a.explore[r * A + i] = ex;
         prev[2 * i] = px; prev[2 * i + 1] = py;
         if (a.algo == 0 || !ex) { pos[2 * i] = cx; pos[2 * i + 1] = cy; a.pos_idx[r * A + i] = -1; }
+        else if (a.algo == 3) { pos[2 * i] = a.xy[2 * tgi]; pos[2 * i + 1] = a.xy[2 * tgi + 1]; a.pos_idx[r * A + i] = tgi; }
         else { pos[2 * i] = axm; pos[2 * i + 1] = aym; a.pos_idx[r * A + i] = gi; }
         cen[2 * i] = cx; cen[2 * i + 1] = cy;
     }
+}
+
+
+// ---- Choi (algo 3): the per-period planner, clusters and tours of every run ---------------------------------------------------
+// The greedy planner of compute_sample_points (simulator.py:326-374) picks arg-max_g (k0 - q[g]) until it is <= threshold,
+// each pick conditioning a COPY of the model on one more hifi point.  Here a pick is appended to the run's own factor as the
+// temporary row Ncur + k (q = 1 case of the bordered update of batch_append_kernel); Ncur does not move, so the run's model is
+// unchanged and the next real sample overwrites the row.  The planner's variance is k0 - q with q = |W psi|^2 accumulated from
+// a recomputation at the period start, never the stepper's decremented var: far from the data q ~ ulp(k0), and the first
+// index of the top 1-ulp plateau is what the reference picks (argmax.cuh).
+
+// cross-covariance of training row n of run r with grid point (ix, iy), from the axis tables (batch_posterior_kernel)
+__device__ __forceinline__ double bt_psi(const BatchArgs& a, int r, int n, int ix, int iy) {
+    const int64_t t = (int64_t)r * a.cap + n;
+    double psi = 0.0;
+    if (n >= a.NL) psi = a.p.s_H * (a.TxH[t * a.nx + ix] * a.TyH[t * a.ny + iy]);
+    if (a.p.multi) psi = fma(n < a.NL ? a.p.rho * a.p.s_L : a.p.rho2 * a.p.s_L, a.TxL[t * a.nx + ix] * a.TyL[t * a.ny + iy], psi);
+    return psi;
+}
+
+constexpr int CQ_ROWS = 8;
+
+// period start: q[g] = |W psi_g|^2 over the rows [0, Ncur) of the run; rows of W in CQ_ROWS-row strips, psi recomputed per strip
+__global__ void __launch_bounds__(BT_THREADS) batch_choi_q_kernel(BatchArgs a) {
+    const int r = blockIdx.y;
+    const int g = blockIdx.x * BT_THREADS + threadIdx.x;
+    if (blockIdx.x == 0 && threadIdx.x == 0) { a.nplan[r] = 0; a.plan_state[r] = a.status[r] != 0 ? 1 : 0; }
+    if (g >= a.G) return;
+    const int N = a.Ncur[r], cap = a.cap, ix = g / a.ny, iy = g % a.ny;
+    const double* W = a.W + (int64_t)r * cap * cap;
+    double q = 0.0;
+    for (int n0 = 0; n0 < N; n0 += CQ_ROWS) {
+        const int hi = min(n0 + CQ_ROWS, N);
+        double acc[CQ_ROWS];
+#pragma unroll
+        for (int j = 0; j < CQ_ROWS; j++) acc[j] = 0.0;
+        for (int m = 0; m < hi; m++) {
+            const double psi = bt_psi(a, r, m, ix, iy);
+#pragma unroll
+            for (int j = 0; j < CQ_ROWS; j++)
+                if (n0 + j < hi && m <= n0 + j) acc[j] = fma(__ldg(W + (int64_t)(n0 + j) * cap + m), psi, acc[j]);
+        }
+#pragma unroll
+        for (int j = 0; j < CQ_ROWS; j++)
+            if (n0 + j < hi) q = fma(acc[j], acc[j], q);
+    }
+    a.q[(int64_t)r * a.G + g] = q;
+}
+
+// one pick of every planning run: arg-max, bordered append of the pick as row n = Ncur + k, q += v^2 with v = W[n, :] psi
+__global__ void __launch_bounds__(BT_THREADS) batch_choi_pick_kernel(BatchArgs a, double threshold) {
+    extern __shared__ __align__(16) double csm[];      // kv[cap] (covariance with rows < n), l[cap] = W kv, w[cap] = new row of W
+    __shared__ double s_v[BT_THREADS / 32];
+    __shared__ long long s_i[BT_THREADS / 32];
+    __shared__ double s_ci;
+    __shared__ int s_go;
+    const int r = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarp = BT_THREADS / 32;
+    if (a.plan_state[r] != 0 || a.status[r] != 0) return;
+    const int cap = a.cap, k = a.nplan[r], n = a.Ncur[r] + k;
+    const TieRule tol{a.p.k0, a.amax_rel};
+    double* q = a.q + (int64_t)r * a.G;
+    ArgMax best{0.0, -1};
+    for (int g = tid; g < a.G; g += BT_THREADS) best = argmax_combine(best, ArgMax{a.p.k0 - q[g], (long long)g}, tol);
+    best = argmax_warp(best, tol);
+    if (lane == 0) { s_v[warp] = best.v; s_i[warp] = best.i; }
+    __syncthreads();
+    if (tid == 0) {
+        for (int w = 1; w < nwarp; w++) best = argmax_combine(best, ArgMax{s_v[w], s_i[w]}, tol);
+        int go = 0;
+        if (!(best.v > threshold)) a.plan_state[r] = 1;                   // while max var > threshold (:345)
+        else if (n + 1 > cap) a.plan_state[r] = 2;                       // the host grows the buffers and resumes
+        else { a.picks[(int64_t)r * cap + k] = best.i; go = 1; }
+        s_go = go;
+        s_i[0] = best.i;
+    }
+    __syncthreads();
+    if (!s_go) return;
+    const long long pick = s_i[0];
+    const double xs = a.xy[2 * pick], ys = a.xy[2 * pick + 1];
+    double* Xt = a.Xt + (int64_t)r * cap * 2;
+    double* W = a.W + (int64_t)r * cap * cap;
+    double* kv = csm;
+    double* lv = csm + cap;
+    double* wn = csm + 2 * cap;
+    const int pix = (int)(pick / a.ny), piy = (int)(pick % a.ny);      // the pick is a grid point: its covariances are table entries
+    for (int m = tid; m < n; m += BT_THREADS) kv[m] = bt_psi(a, r, m, pix, piy);
+    __syncthreads();
+    for (int nn = warp; nn < n; nn += nwarp) {          // l = W kv: a warp per row
+        const double* wr = W + (int64_t)nn * cap;
+        double s = 0.0;
+        for (int m = lane; m <= nn; m += 32) s = fma(wr[m], kv[m], s);
+        s = warp_sum_d(s);
+        if (lane == 0) lv[nn] = s;
+    }
+    __syncthreads();
+    if (warp == 0) {          // d^2 = k(x, x) + noise_H + jitter - l.l; np.linalg.cholesky raises on a non-positive pivot
+        double s = 0.0;
+        for (int m = lane; m < n; m += 32) s = fma(lv[m], lv[m], s);
+        s = warp_sum_d(s);
+        if (lane == 0) {
+            const double xh = xs / a.p.l_H, yh = ys / a.p.l_H;
+            double kk = rbf_scaled(xh, yh, xh, yh, a.p.s_H);
+            if (a.p.multi) {
+                const double xl = xs / a.p.l_L, yl = ys / a.p.l_L;
+                kk = __dadd_rn(__dmul_rn(a.p.rho2, rbf_scaled(xl, yl, xl, yl, a.p.s_L)), kk);
+            }
+            kk = kk + a.p.noise_H;
+            kk = kk + a.p.jitter;
+            const double d2 = kk - s;
+            if (!(d2 > 0.0)) { a.status[r] = n + 1; s_ci = 0.0; }
+            else s_ci = 1.0 / sqrt(d2);
+        }
+    }
+    __syncthreads();
+    const double ci = s_ci;
+    if (ci == 0.0) return;
+    for (int m = tid; m < n; m += BT_THREADS) {        // W[n][m] = -ci sum_{nn >= m} l[nn] W[nn][m]
+        double t = 0.0;
+        for (int nn = m; nn < n; nn++) t = fma(lv[nn], W[(int64_t)nn * cap + m], t);
+        const double w = -(ci * t);
+        wn[m] = w;
+        W[(int64_t)n * cap + m] = w;
+    }
+    if (tid == 0) {
+        wn[n] = ci;
+        W[(int64_t)n * cap + n] = ci;
+        Xt[2 * n] = xs; Xt[2 * n + 1] = ys;
+        a.nplan[r] = k + 1;
+    }
+    for (int i = tid; i < a.nx + a.ny; i += BT_THREADS) {      // axis-table rows of the pick (batch_append_kernel)
+        const bool isx = i < a.nx;
+        const double u = isx ? a.ux[i] : a.uy[i - a.nx], U = isx ? xs : ys;
+        const double dH = u / a.p.l_H - U / a.p.l_H;
+        const int64_t row = (int64_t)r * cap + n;
+        if (isx) a.TxH[row * a.nx + i] = exp(-0.5 * (dH * dH)); else a.TyH[row * a.ny + (i - a.nx)] = exp(-0.5 * (dH * dH));
+        if (a.p.multi) {
+            const double dL = u / a.p.l_L - U / a.p.l_L;
+            if (isx) a.TxL[row * a.nx + i] = exp(-0.5 * (dL * dL)); else a.TyL[row * a.ny + (i - a.nx)] = exp(-0.5 * (dL * dL));
+        }
+    }
+    __syncthreads();
+    for (int g = tid; g < a.G; g += BT_THREADS) {
+        const int ix = g / a.ny, iy = g % a.ny;
+        double v = 0.0;
+        for (int m = 0; m <= n; m++) v = fma(wn[m], bt_psi(a, r, m, ix, iy), v);
+        q[g] += v * v;
+    }
+}
+
+// cells of the period's picks in the partition seeded by the centroids (simulator.py:651-653, :377-412): nearest seed, and
+// within TIE_TOL of a bisector the crossings test against the device-clipped cells (pass 1 of batch_coverage_kernel).  A pick
+// in no cell is dropped, a pick in several cells joins each of them.  Hard ties (gap <= TIE_TOL/10) are counted: there the
+// reference's Qhull vertices decide, and the host re-runs such runs on the single-run path.
+__global__ void __launch_bounds__(BT_THREADS) batch_choi_cluster_kernel(BatchArgs a) {
+    __shared__ double s_seed[BT_MAXA][2];
+    __shared__ double s_poly[BT_MAXA][2 * BC_MAXV];
+    __shared__ int s_cnt[BT_MAXA];
+    __shared__ double s_buf[BT_THREADS / 32][256];
+    __shared__ int s_ties, s_bad;
+    const int r = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarp = BT_THREADS / 32;
+    const int A = a.A, cap = a.cap;
+    const int k = a.status[r] == 0 ? a.nplan[r] : 0;
+    if (tid < 2 * A) s_seed[tid >> 1][tid & 1] = a.cen[(int64_t)r * A * 2 + tid];
+    if (tid == 0) { s_ties = 0; s_bad = 0; }
+    __syncthreads();
+    const double h = 0.5 * a.eps;
+    for (int i = warp; i < A && k > 0; i += nwarp) {
+        bool overflow = false;
+        int which = 0;
+        const int nv = vc_clip_cell(&s_seed[0][0], A, i, a.xmin - h, a.xmax + h, a.ymin - h, a.ymax + h, s_buf[warp], lane, overflow, which);
+        const double* px = s_buf[warp] + 128 * which;
+        const double* py = px + 64;
+        if (nv > BC_MAXV) overflow = true;
+        for (int v = lane; v < nv && v < BC_MAXV; v += 32) { s_poly[i][2 * v] = px[v]; s_poly[i][2 * v + 1] = py[v]; }
+        if (lane == 0) {
+            s_cnt[i] = nv < BC_MAXV ? nv : BC_MAXV;
+            if (overflow) s_bad = 1;
+        }
+        __syncwarp();
+    }
+    __syncthreads();
+    int hard = 0;
+    for (int j = tid; j < k; j += BT_THREADS) {
+        const long long g = a.picks[(int64_t)r * cap + j];
+        const double x = a.xy[2 * g], y = a.xy[2 * g + 1];
+        double best = DBL_MAX, second = DBL_MAX;
+        int bi = 0;
+        for (int c = 0; c < A; c++) {
+            const double dx = x - s_seed[c][0], dy = y - s_seed[c][1];
+            const double d = fma(dx, dx, dy * dy);
+            if (d < best) { second = best; best = d; bi = c; }
+            else if (d < second) second = d;
+        }
+        const double gap = second - best;
+        unsigned mask = 0;
+        if (gap > a.tie_tol) {
+            mask = 1u << bi;
+        } else {
+            if (!(gap > 0.1 * a.tie_tol)) hard++;
+            for (int c = 0; c < A; c++)
+                if (crossings_inside(s_poly[c], s_cnt[c], x, y)) mask |= 1u << c;
+        }
+        a.pmask[(int64_t)r * cap + j] = (int)mask;
+    }
+    if (hard) atomicAdd(&s_ties, hard);
+    __syncthreads();
+    for (int c = warp; c < A; c += nwarp) {
+        int cn = 0;
+        for (int j = lane; j < k; j += 32) cn += (a.pmask[(int64_t)r * cap + j] >> c) & 1;
+        cn = __reduce_add_sync(0xffffffffu, cn);
+        if (lane == 0) a.ccount[r * A + c] = cn;
+    }
+    if (tid == 0) {
+        a.cties[r] = s_ties;
+        if (s_bad) a.status[r] = -5;
+    }
+}
+
+// cluster (r, c) = the picks of run r in cell c, in selection order, at tour_off[r*A + c]: coordinates for the tour planner
+__global__ void batch_choi_gather_kernel(BatchArgs a, double* pts, long long* gidx) {
+    const int rc = blockIdx.x * blockDim.x + threadIdx.x;
+    if (rc >= a.runs * a.A) return;
+    const int r = rc / a.A, c = rc % a.A, cap = a.cap;
+    int o = a.tour_off[rc];
+    a.tour_cur[rc] = o;
+    if (a.ccount[rc] == 0) return;
+    const int k = a.nplan[r];
+    for (int j = 0; j < k; j++)
+        if ((a.pmask[(int64_t)r * cap + j] >> c) & 1) {
+            const long long g = a.picks[(int64_t)r * cap + j];
+            pts[2 * (int64_t)o] = a.xy[2 * g]; pts[2 * (int64_t)o + 1] = a.xy[2 * g + 1];
+            gidx[o++] = g;
+        }
+}
+
+// tour of (r, c) as grid indices in visiting order (ord: local indices from tsp_tours_kernel)
+__global__ void batch_choi_order_kernel(BatchArgs a, const long long* gidx, const int32_t* ord) {
+    const int rc = blockIdx.x * blockDim.x + threadIdx.x;
+    if (rc >= a.runs * a.A) return;
+    const int o0 = a.tour_off[rc], o1 = a.tour_off[rc + 1];
+    for (int t = o0; t < o1; t++) a.tour[t] = gidx[o0 + ord[t]];
 }
 
 }  // namespace mfgp
@@ -496,11 +748,12 @@ extern "C" {
 
 /* struct mfgp_batch: include/mfgp_b200.h */
 
-int mfgp_batch_step(const mfgp_batch* b, const mfgp_params* p_host, int64_t iteration, void* stream) {
-    if (!b || !p_host || b->runs <= 0 || b->A <= 0 || b->A > BT_MAXA || b->G <= 0 || b->nx * b->ny != b->G || b->cap <= 0 ||
-        iteration < 0 || iteration >= b->iterations)
-        return MFGP_ERR_INVALID;
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
+static bool batch_valid(const mfgp_batch* b, const mfgp_params* p_host) {
+    return b && p_host && b->runs > 0 && b->A > 0 && b->A <= BT_MAXA && b->G > 0 && b->nx * b->ny == b->G && b->cap > 0 &&
+           b->algo >= 0 && b->algo <= 3 && (b->algo != 3 || (b->tour_off && b->tour_cur));
+}
+
+static BatchArgs batch_args(const mfgp_batch* b, const mfgp_params* p_host) {
     BatchArgs a{};
     a.runs = (int)b->runs; a.G = (int)b->G; a.nx = (int)b->nx; a.ny = (int)b->ny; a.A = (int)b->A; a.NL = (int)b->NL;
     a.cap = (int)b->cap; a.algo = (int)b->algo; a.iterations = (int)b->iterations; a.max_samples = (int)b->max_samples;
@@ -512,6 +765,16 @@ int mfgp_batch_step(const mfgp_batch* b, const mfgp_params* p_host, int64_t iter
     a.Ncur = b->Ncur; a.knew = b->knew; a.status = b->status; a.noise_used = b->noise_used; a.nsamples = b->nsamples;
     a.ties = b->ties; a.noise = b->noise; a.unif = b->unif; a.log_loss = b->log_loss; a.log_agent = b->log_agent;
     a.log_sample = b->log_sample;
+    a.q = b->q; a.picks = reinterpret_cast<long long*>(b->picks); a.nplan = b->nplan; a.plan_state = b->plan_state;
+    a.pmask = b->pmask; a.ccount = b->ccount; a.cties = b->cties; a.tour_off = b->tour_off; a.tour_cur = b->tour_cur;
+    a.tour = reinterpret_cast<long long*>(b->tour);
+    return a;
+}
+
+int mfgp_batch_step(const mfgp_batch* b, const mfgp_params* p_host, int64_t iteration, void* stream) {
+    if (!batch_valid(b, p_host) || iteration < 0 || iteration >= b->iterations) return MFGP_ERR_INVALID;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const BatchArgs a = batch_args(b, p_host);
     if (a.algo != 0) {
         const size_t smem = sizeof(double) * 2 * (size_t)a.A * (size_t)a.cap;
         if (smem > 200 * 1024) return MFGP_ERR_INVALID;
@@ -531,6 +794,61 @@ int mfgp_batch_step(const mfgp_batch* b, const mfgp_params* p_host, int64_t iter
     if (msmem > 160 * 1024) return MFGP_ERR_INVALID;
     MFGP_CUDA_CHECK(cudaFuncSetAttribute(batch_coverage_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msmem));
     batch_coverage_kernel<<<a.runs, BT_THREADS, msmem, st>>>(a, (int)iteration);
+    MFGP_LAUNCH_CHECK();
+    return MFGP_OK;
+}
+
+
+static bool choi_valid(const mfgp_batch* b, const mfgp_params* p_host) {
+    return batch_valid(b, p_host) && b->algo == 3 && b->q && b->picks && b->nplan && b->plan_state && b->pmask && b->ccount &&
+           b->cties;
+}
+
+int mfgp_batch_choi_begin(const mfgp_batch* b, const mfgp_params* p_host, void* stream) {
+    if (!choi_valid(b, p_host)) return MFGP_ERR_INVALID;
+    const BatchArgs a = batch_args(b, p_host);
+    batch_choi_q_kernel<<<dim3((unsigned)((a.G + BT_THREADS - 1) / BT_THREADS), (unsigned)a.runs), BT_THREADS, 0,
+                          static_cast<cudaStream_t>(stream)>>>(a);
+    MFGP_LAUNCH_CHECK();
+    return MFGP_OK;
+}
+
+int mfgp_batch_choi_plan(const mfgp_batch* b, const mfgp_params* p_host, double threshold, int64_t rounds, void* stream) {
+    if (!choi_valid(b, p_host) || rounds < 0) return MFGP_ERR_INVALID;
+    const BatchArgs a = batch_args(b, p_host);
+    const size_t smem = sizeof(double) * 3 * (size_t)a.cap;
+    if (smem > 200 * 1024) return MFGP_ERR_INVALID;
+    MFGP_CUDA_CHECK(cudaFuncSetAttribute(batch_choi_pick_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    for (int64_t i = 0; i < rounds; i++) {
+        batch_choi_pick_kernel<<<a.runs, BT_THREADS, smem, static_cast<cudaStream_t>(stream)>>>(a, threshold);
+        MFGP_LAUNCH_CHECK();
+    }
+    return MFGP_OK;
+}
+
+int mfgp_batch_choi_cluster(const mfgp_batch* b, void* stream) {
+    mfgp_params dummy{};
+    if (!b || !choi_valid(b, &dummy)) return MFGP_ERR_INVALID;
+    const BatchArgs a = batch_args(b, &dummy);
+    batch_choi_cluster_kernel<<<a.runs, BT_THREADS, 0, static_cast<cudaStream_t>(stream)>>>(a);
+    MFGP_LAUNCH_CHECK();
+    return MFGP_OK;
+}
+
+int mfgp_batch_choi_tours(const mfgp_batch* b, int64_t n_total, int64_t n_max, double* pts, int64_t* gidx, int32_t* ord,
+                          void* work, int64_t work_bytes, void* stream) {
+    mfgp_params dummy{};
+    if (!b || !choi_valid(b, &dummy) || n_total < 0 || n_max < 0 || n_max > n_total) return MFGP_ERR_INVALID;
+    if (n_total > 0 && (!pts || !gidx || !ord || !b->tour)) return MFGP_ERR_INVALID;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const BatchArgs a = batch_args(b, &dummy);
+    const int nrc = a.runs * a.A;
+    batch_choi_gather_kernel<<<(nrc + 127) / 128, 128, 0, st>>>(a, pts, reinterpret_cast<long long*>(gidx));
+    MFGP_LAUNCH_CHECK();
+    if (n_total == 0) return MFGP_OK;
+    const int rc = choi_tsp_tours(pts, b->tour_off, nrc, n_total, n_max, ord, nullptr, work, work_bytes, stream);
+    if (rc != MFGP_OK) return rc;
+    batch_choi_order_kernel<<<(nrc + 127) / 128, 128, 0, st>>>(a, reinterpret_cast<const long long*>(gidx), ord);
     MFGP_LAUNCH_CHECK();
     return MFGP_OK;
 }

@@ -49,18 +49,19 @@ def run_sim(args):
     return loss_log_t, agent_log_t, sample_log_t
 
 
-# MFGP_BATCHED=1 (or runner.BATCHED = True, or run(batched=True)): the replicate simulations of lloyd / periodic / todescato
-# experiments are stepped TOGETHER on the device (simulator.run_batched: three kernel launches advance every run by one
-# iteration) instead of one host loop per simulation.  The random streams are consumed exactly as the sequential loop
-# consumes them: per simulation the 2 A start coordinates, then (todescato) one uniform per agent and iteration.
+# MFGP_BATCHED=1 (or runner.BATCHED = True, or run(batched=True)): the replicate simulations of lloyd / periodic / todescato /
+# choi experiments are stepped TOGETHER on the device (simulator.run_batched: three kernel launches advance every run by one
+# iteration; Choi plans all runs' tours on the device once per period) instead of one host loop per simulation.  The random
+# streams are consumed exactly as the sequential loop consumes them: per simulation the 2 A start coordinates, then
+# (todescato) one uniform per agent and iteration.
 BATCHED = os.environ.get("MFGP_BATCHED", "0") == "1"
 BATCH_RUNS = 512          # simulations per device batch (state: ~4 MB per run at 64x64 points, 520 samples)
 
 
 def _batchable(args):
     algos = {a[1] for a in args}
-    return len(args) > 1 and len(algos) == 1 and not any("choi" in a for a in algos) and \
-        any(k in next(iter(algos)) for k in ("todescato", "lloyd", "periodic")) and all(a[10] is None for a in args)
+    return len(args) > 1 and len(algos) == 1 and \
+        any(k in next(iter(algos)) for k in ("choi", "todescato", "lloyd", "periodic")) and all(a[10] is None for a in args)
 
 
 def run_sims_batched(args):

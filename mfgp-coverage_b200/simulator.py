@@ -609,15 +609,18 @@ def todescato(title, sim_num, iterations, agents, positions, truth, sigma_n, pri
 def run_batched(algo, sim_nums, iterations, agents, positions, truth, sigma_n, prior, hyp, uniforms=None, noise=None,
                 noise_rngs=None, exact_tie_loss=False, use_graph=False):
     """Many independent runs of ONE experiment stepped together on the device (config c5, the replicate sweeps of
-    runner.py:100, :131-147): `algo` in ("lloyd", "periodic", "todescato"), `positions[R, A, 2]` the runs' start positions
-    (updated in place to the final ones, like the single-run functions do).  Returns a list of R (loss_log, agent_log,
-    sample_log) triples with the reference's row schemas.  See _batched.BatchedRuns for the random-number and tie
-    conventions; `exact_tie_loss=True` re-evaluates the losses that involve exact bisector ties with Qhull cells."""
+    runner.py:100, :131-147): `algo` names lloyd, periodic, todescato or choi (as runner.run_sim dispatches), `positions[R, A,
+    2]` the runs' start positions (updated in place to the final ones, like the single-run functions do).  Returns a list of R
+    (loss_log, agent_log, sample_log) triples with the reference's row schemas.  See _batched.BatchedRuns for the
+    random-number and tie conventions; `exact_tie_loss=True` re-evaluates the losses that involve exact bisector ties with
+    Qhull cells.  Choi runs come back to the host once per period, so `use_graph` is not available for them."""
     from ._batched import BatchedRuns
     kind = "choi" if "choi" in algo else ("todescato" if "todescato" in algo else ("lloyd" if "lloyd" in algo else
                                           ("periodic" if "periodic" in algo else None)))
-    if kind is None or kind == "choi":
-        raise ValueError("run_batched supports lloyd, periodic and todescato")
+    if kind is None:
+        raise ValueError("run_batched supports lloyd, periodic, todescato and choi")
+    if kind == "choi" and use_graph:
+        raise ValueError("Choi runs return to the host once per period: use_graph is not available for them")
     truth_arr = np.vstack(truth.values.tolist()) if hasattr(truth, "values") else np.asarray(truth, dtype=np.float64)
     prior_arr = None
     if prior is not None and len(prior) > 0:

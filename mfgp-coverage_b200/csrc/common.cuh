@@ -1,7 +1,8 @@
-// Shared device helpers for libmfgp_b200 (sm_100a): FP64 tensor-core MMA, cp.async staging, error plumbing.
+// Shared device helpers for libmfgp_b200 (sm_100a): FP64 tensor-core MMA, cp.async / TMA staging, error plumbing.
 #pragma once
 #include <cstdint>
 #include <cstdio>
+#include <cuda.h>
 #include <cuda_runtime.h>
 
 #include "../../include/mfgp_b200.h"
@@ -47,6 +48,68 @@ __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commi
 template <int N>
 __device__ __forceinline__ void cp_async_wait() {
     asm volatile("cp.async.wait_group %0;\n" ::"n"(N));
+}
+
+// ---- mbarrier / TMA primitives (PTX) ----------------------------------------------------------------------------------
+__device__ __forceinline__ uint32_t smem_u32(const void* p) { return static_cast<uint32_t>(__cvta_generic_to_shared(p)); }
+__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;\n" ::"r"(bar), "r"(count));
+}
+__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
+    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];\n" ::"r"(bar) : "memory");
+}
+__device__ __forceinline__ void mbar_arrive_expect_tx(uint32_t bar, uint32_t bytes) {
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;\n" ::"r"(bar), "r"(bytes) : "memory");
+}
+__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
+    uint32_t done;
+    do {
+        asm volatile(
+            "{\n .reg .pred p;\n mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n selp.u32 %0, 1, 0, p;\n}\n"
+            : "=r"(done)
+            : "r"(bar), "r"(parity)
+            : "memory");
+    } while (!done);
+}
+// box of a 2D tensor map at element coordinates (c0 = column, c1 = row) -> shared memory; completion in bytes on `bar`
+__device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* map, int c0, int c1, uint32_t bar) {
+    asm volatile(
+        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];\n" ::"r"(dst),
+        "l"(map), "r"(c0), "r"(c1), "r"(bar)
+        : "memory");
+}
+
+// 2D tensor map of a row-major FP64 matrix (rows x cols, row stride ld elements) with a box of box_cols x box_rows;
+// cuTensorMapEncodeTiled through the runtime's driver entry point query (no link-time dependency on libcuda).  The base
+// must be 16-byte aligned and ld even; boxes reaching past the matrix read zeros.
+typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
+                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
+                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+inline int make_tensor_map_2d(CUtensorMap* map, const double* base, int64_t rows, int64_t cols, int64_t ld, int box_cols,
+                              int box_rows, CUtensorMapSwizzle swizzle) {
+    static EncodeTiledFn encode = nullptr;
+    if (!encode) {
+        void* fn = nullptr;
+        cudaDriverEntryPointQueryResult qres;
+        MFGP_CUDA_CHECK(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres));
+        if (qres != cudaDriverEntryPointSuccess || !fn) {
+            set_last_error("cuTensorMapEncodeTiled entry point unavailable", cudaErrorUnknown);
+            return MFGP_ERR_CUDA;
+        }
+        encode = reinterpret_cast<EncodeTiledFn>(fn);
+    }
+    const cuuint64_t gdim[2] = {(cuuint64_t)cols, (cuuint64_t)rows};       // {columns (contiguous), rows}
+    const cuuint64_t gstride[1] = {(cuuint64_t)ld * sizeof(double)};       // row pitch in bytes
+    const cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows};
+    const cuuint32_t estr[2] = {1, 1};
+    const CUresult r = encode(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 2, const_cast<double*>(base), gdim, gstride, box, estr,
+                              CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) {
+        set_last_error("cuTensorMapEncodeTiled failed", cudaErrorInvalidValue);
+        return MFGP_ERR_CUDA;
+    }
+    return MFGP_OK;
 }
 
 // ---- the RBF kernel with the reference's operation order (gaussian_process.py:75-79) -------------------------------

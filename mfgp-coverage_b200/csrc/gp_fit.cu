@@ -95,6 +95,10 @@ struct PotrfScratch {
 // BS = 64: the whole tile (s, m: 4x4 cyclic sub-blocks per thread); BS = 32: one half of the two-level form below (2x2).
 // `col0`: global index of the block's first column (for the failing-pivot report).  Ls / Wsm (optional, shared memory, row
 // stride lds_out): copies of L and of its inverse for the caller's next step.
+// Barrier of the 256 threads that work on a tile: the whole CTA of potrf_diag_kernel, the consumer warps of
+// chol_dataflow_kernel (whose ninth warp, the producer, does not take part in the epilogue).
+__device__ __forceinline__ void tile_bar() { asm volatile("bar.sync 1, 256;\n" ::: "memory"); }
+
 template <int BS>
 __device__ __forceinline__ void potrf_diag_body(const double* src, int64_t lds, double* A, int64_t ld,
                                                 double* __restrict__ Winv, int64_t ldw, int32_t* __restrict__ info, int col0,
@@ -132,7 +136,7 @@ __device__ __forceinline__ void potrf_diag_body(const double* src, int64_t lds, 
 #pragma unroll
                 for (int b = 0; b < NB; b++) dst[2 * (tc + 16 * b)] = m[jb][b];
             }
-            __syncthreads();
+            tile_bar();
             const double2* col = colAB[buf];
             const double2* row = rowAB[buf];
             double pa = col[j0].x;
@@ -181,7 +185,7 @@ __device__ __forceinline__ void potrf_diag_body(const double* src, int64_t lds, 
             }
         }
     }
-    __syncthreads();
+    tile_bar();
     if (tid < BS / 2) {          // C = chol(P) of every pair
         const double a = piv[0][tid], b = piv[1][tid], c = piv[2][tid];
         const double r1 = rsqrt(a);
@@ -190,7 +194,7 @@ __device__ __forceinline__ void potrf_diag_body(const double* src, int64_t lds, 
         fin[1][tid] = rsqrt(fma(-g, b, c));
         fin[2][tid] = g;
     }
-    __syncthreads();
+    tile_bar();
     const bool failed = bad != 0;
 #pragma unroll
     for (int a = 0; a < NB; a++)
@@ -241,6 +245,13 @@ __global__ void __launch_bounds__(256, 1) potrf_diag_kernel(double* __restrict__
 // them); a bounded spin (abort flag) guards against bugs all the same.
 // Two CTAs share an SM; while one of them runs the latency-bound tail of a chain task it raises a per-SM pause flag and
 // the other one idles between its k slabs (its DMMA traffic would otherwise stretch the chain by ~25%).
+// Warp-specialised: 8 consumer warps run the DMMA loops and the epilogues; a ninth, producer warp draws the tickets, polls
+// the tile flags and moves every slab with ONE 2D TMA copy per operand into a 3-slot ring (full / empty mbarriers), so the
+// k loop has no CTA-wide barrier and no per-thread copy issue.  The TMA boxes are 4 doubles wider than the slab: the
+// 4 columns past it land as the row padding that puts the 8 rows of a DMMA
+// fragment read on distinct bank groups, so the slabs keep the padded layout the fragment reads are laid out for.  Those 4
+// columns belong to the neighbouring k tile (Y tile, W block), whose flag has not been acquired and which another CTA may be
+// writing at that moment: the copy may read in-flight data there.  That is intended -- no padding element is ever read.
 constexpr int DF_K = 32;                 // K slab
 constexpr int DF_LDA = DF_K + 4;         // [m][k] / [n][k] slabs: rows land on distinct 8-bank groups
 constexpr int DF_LDT = PB + 4;           // [k][n] slabs and the 64x64 epilogue tiles
@@ -248,7 +259,16 @@ constexpr int DF_STAGE = PB * DF_LDA;    // doubles per operand per stage (64 x 
 constexpr int DF_TILE = PB * DF_LDT;     // one padded 64x64 tile
 constexpr int DF_NSTAGE = 3;             // slabs in flight: one slab of compute (~0.5 us) does not cover an L2 round trip under load
 constexpr int DF_SMEM_DOUBLES = DF_NSTAGE * 2 * DF_STAGE;     // 3 stages x (A, B) = 13824 doubles >= epilogue X, W, L tiles (13056)
-constexpr int DF_THREADS = 256;
+constexpr int DF_SMEM_BYTES = DF_SMEM_DOUBLES * 8 + 128;      // + slack to align the TMA destinations to 128 bytes
+constexpr int DF_THREADS = 256;                               // consumer threads
+constexpr int DF_CTA_THREADS = DF_THREADS + 32;               // + the producer warp
+constexpr uint32_t DF_MK_BYTES = PB * DF_LDA * 8;             // TMA box of an [m][k] / [n][k] slab (36 x 64 doubles)
+constexpr uint32_t DF_KN_BYTES = DF_K * DF_LDT * 8;           // TMA box of a [k][n] slab (68 x 32 doubles)
+constexpr uint32_t DF_TILE_BYTES = PB * DF_LDT * 8;           // TMA box of the epilogue's W_cc tile (68 x 64 doubles)
+// Factorisations of fewer block columns (npad <= 2048: c2, c3) are bound by the chain of diagonal blocks and run the cp.async
+// form of the kernel (chol_dataflow_cpasync_kernel).  Measured on a B200, cp.async vs TMA: N = 1024 0.298 vs 0.313 ms; N = 2048
+// R = 0 0.610 vs 0.614 ms, R = 512 0.627 vs 0.621 ms; N = 4096 7-10 % faster with TMA
+constexpr int DF_TMA_MIN_NB = 33;
 
 struct DfArgs {
     double* K; int64_t ld;
@@ -313,6 +333,13 @@ __device__ __forceinline__ int df_ld_relaxed(const int* p) {
 __device__ __forceinline__ void df_st_release(int* p, int v) {
     asm volatile("st.release.gpu.global.s32 [%0], %1;\n" ::"l"(p), "r"(v) : "memory");
 }
+// Publishes a tile: the CTA's stores of it (ordered before this thread by a barrier) are written with generic stores but read by
+// later tasks through the async proxy (TMA), so a proxy fence precedes the release of the flag (the reader adds one after its
+// acquire).  One thread, after the barrier: a fence in every thread would drain every thread's stores on the chain's path.
+__device__ __forceinline__ void df_publish(int* flag) {
+    asm volatile("fence.proxy.async.global;\n" ::: "memory");
+    df_st_release(flag, 1);
+}
 __device__ __forceinline__ void df_st_relaxed(int* p, int v) {
     asm volatile("st.relaxed.gpu.global.s32 [%0], %1;\n" ::"l"(p), "r"(v) : "memory");
 }
@@ -336,11 +363,545 @@ __device__ __forceinline__ bool df_wait(const int* f, int* ctrl, int32_t* info, 
     return ok != 0;
 }
 
-// (A warp-specialised variant -- ninth warp as producer with mbarrier hand-off, bulk copies or cp.async -- was built and
-// measured this round: correct, but 2.48 ms against 2.07 ms; one warp cannot issue the 2048 16-byte copies of a slab fast enough,
-// and 128 row-sized bulk copies per slab are slower still.  profiles/r02_chol_scheduler_experiments.txt, experiment 12.)
-__global__ void __launch_bounds__(DF_THREADS, 2) chol_dataflow_kernel(DfArgs g) {
-    extern __shared__ __align__(16) double df_smem[];
+// Output of the task in task[] (kind, column, index, aux): the tile the accumulators start from and the task writes (row stride
+// ldc), the diagonal tile of a chain task, and the flag that publishes the tile.  Derived from the shared task[] where used: held
+// in registers across the k loop, these pointers would spill.
+struct DfOut {
+    double* Ct; int64_t ldc;
+    double* Cd;
+    int* flag;
+};
+__device__ __forceinline__ DfOut df_out(const DfArgs& g, const int* task) {
+    const int kind = task[0], idx = task[2], tj = task[3];
+    const bool rhs = kind == 1, chain = kind == 2, gram = kind == 3;
+    const int c = chain ? idx - 1 : (gram ? 0 : task[1]), cc = c > 0 ? c : 0;
+    const int i = rhs ? c : idx;
+    DfOut o;
+    o.Ct = gram ? g.M + (int64_t)idx * PB * g.ldm + (int64_t)tj * PB
+                : (rhs ? g.Bm + (int64_t)c * PB * g.ldb + (int64_t)idx * PB : g.K + (int64_t)i * PB * g.ld + (int64_t)cc * PB);
+    o.ldc = gram ? g.ldm : (rhs ? g.ldb : g.ld);
+    o.Cd = g.K + (int64_t)(chain ? idx : 0) * PB * (g.ld + 1);
+    o.flag = gram ? g.flagsM + (int64_t)task[1] * g.m_tiles + idx * (idx + 1) / 2 + tj
+                  : (rhs ? g.flagsY + (int64_t)c * g.nr + idx : g.flagsL + (int64_t)i * g.nb + cc);   // chain: tile (idx, idx - 1)
+    return o;
+}
+
+// The producer's flag check for the k tiles kt0, kt0 + 1, ... of a task: lane j < 16 reads the flag of the A tile of k tile
+// kt0 + j, lane 16 + j that of its B tile (relaxed: one L2 round trip for up to 16 tiles).  Once a leading run of tiles is
+// seen ready, every lane of the run takes ONE acquire load of its flag, and __syncwarp orders those acquires before lane 0's
+// copies.  While tile kt0 is not ready only its two flags are polled (bounded spin, abort flag as in df_wait).  Returns the
+// last tile of the run (>= kt0), or -1 once the abort flag is raised.
+__device__ __forceinline__ int df_poll_tiles(const int* fa, int fas, const int* fb, int fbs, int kt0, int nk, int* ctrl, int32_t* info,
+                                          long long limit) {
+    const int lane = threadIdx.x & 31, j = lane & 15, kt = kt0 + j;
+    const int* f = lane < 16 ? fa + (int64_t)kt * fas : fb + (int64_t)kt * fbs;
+    long long t0 = 0;
+    for (int spin = 0;; spin++) {
+        const int v = (kt < nk && (spin == 0 || j == 0)) ? df_ld_relaxed(f) : 0;
+        const unsigned m = __ballot_sync(0xffffffffu, v != 0);
+        const unsigned both = m & (m >> 16) & 0xffffu;
+        const int n = __ffs(~both) - 1;          // length of the leading run of ready tiles
+        if (n > 0) {
+            if (j < n) (void)df_ld_acquire(f);
+            __syncwarp();
+            return kt0 + n - 1;
+        }
+        int stop = 0;
+        if (lane == 0) {
+            if (spin == 0) t0 = clock64();
+            else if (clock64() - t0 > limit) { atomicExch(ctrl + 1, 1); atomicExch(info, -1); }
+            stop = *reinterpret_cast<volatile int*>(ctrl + 1);
+        }
+        if (__shfl_sync(0xffffffffu, stop, 0)) return -1;
+        __nanosleep(32);
+    }
+}
+
+__global__ void __maxnreg__(112)        // 2 CTAs of 288 threads per SM: 2 x 288 x 112 <= 65536 registers
+chol_dataflow_kernel(const __grid_constant__ CUtensorMap kmap, const __grid_constant__ CUtensorMap bmap,
+                     const __grid_constant__ CUtensorMap wmap, DfArgs g) {
+    extern __shared__ __align__(128) uint8_t df_smem_raw[];
+    // TMA destinations 128-byte aligned (offsetting the shared array keeps the compiler's shared-memory loads and stores)
+    double* df_smem = reinterpret_cast<double*>(df_smem_raw + ((128u - (smem_u32(df_smem_raw) & 127u)) & 127u));
+    __shared__ int task[6];                   // kind, column, index, aux; ring slabs moved before the task, W_cc tiles loaded before it
+    __shared__ int ready_s[4];
+    __shared__ int dec_s[6];                  // the producer's ticket and ring state (below)
+    __shared__ int abort_s;                   // the producer met the abort flag in the k loop (read after the loop's barrier)
+    __shared__ __align__(8) unsigned long long df_bars[2 * DF_NSTAGE + 1];     // full[slot], empty[slot], W_cc tile
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const bool producer = warp == DF_THREADS / 32;
+    const uint32_t bar_full = smem_u32(&df_bars[0]), bar_empty = smem_u32(&df_bars[DF_NSTAGE]);
+    const uint32_t bar_w = smem_u32(&df_bars[2 * DF_NSTAGE]);
+    if (tid == 0) {
+        for (int q = 0; q < DF_NSTAGE; q++) { mbar_init(bar_full + 8 * q, 1); mbar_init(bar_empty + 8 * q, DF_THREADS / 32); }
+        mbar_init(bar_w, 1);
+        abort_s = 0;
+        dec_s[0] = -1; dec_s[1] = 0; dec_s[2] = 1; dec_s[3] = 1; dec_s[4] = 0; dec_s[5] = 0;
+        asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
+    }
+    // 8 warps as 4 x 2; a warp owns the 8x8 tiles (row tile (warp>>1) + 4x, column tile (warp&1) + 2y), x < 2, y < 4 --
+    // interleaved, so that the triangular products of the chain task (W_cc lower, S symmetric) skip about the same share
+    // of DMMAs in every warp
+    const int wm = (warp >> 1) * 8, wn = (warp & 1) * 8;
+    const int gq = lane >> 2, tq = lane & 3;
+    double* As0 = df_smem;
+    double* Bs0 = df_smem + DF_NSTAGE * DF_STAGE;
+    auto my_pause = [&]() {                   // this SM's pause flag (re-derived: a pointer held across the loop costs registers)
+        unsigned smid;
+        asm volatile("mov.u32 %0, %%smid;\n" : "=r"(smid));
+        return g.pause + smid;
+    };
+    // diagnostics (MFGP_DF_TRACE=1): SM clocks this CTA's thread 0 spent waiting (tile flags, slabs), in k loops, and in total
+#ifdef MFGP_DF_ACCOUNTING       // build with -DMFGP_DF_ACCOUNTING for profiles/tools/cta_account.py (costs ~10 registers)
+    long long t_wait = 0, t_loop = 0, t_begin = clock64(), t_mark = 0;
+    int n_tasks = 0;
+    const bool tracing = g.trace != nullptr;
+#else
+    long long t_wait = 0, t_loop = 0, t_begin = 0, t_mark = 0;
+    int n_tasks = 0;
+    constexpr bool tracing = false;
+#endif
+    // producer lane 0's state, kept in shared memory (it is touched once per task; registers are the consumers' budget):
+    // a Gram ticket claimed before it became runnable; the decoder's column, next chain task to place and its first ticket;
+    // the slabs this CTA has moved so far (ring slot = gs % 3, phase = gs / 3) and the W_cc tiles (phase of bar_w)
+    int& held_m = dec_s[0];
+    int& dec_c = dec_s[1];
+    int& dec_dnext = dec_s[2];
+    int& dec_base = dec_s[3];
+
+    for (;;) {
+        if (!producer) asm volatile("fence.proxy.async.shared::cta;\n" ::: "memory");   // epilogue stores before the next TMA writes
+        __syncthreads();                      // the previous task is done with shared memory and task[]
+        if (producer && lane == 0) {
+            int c = 0, kind = -1, idx = 0, aux = 0;
+            int t = -1;
+            if (g.M == nullptr) {
+                t = atomicAdd(g.ctrl, 1);
+            } else {
+                // Two queues.  Critical = the factorisation and the substitution (ticket order as below); Gram = the tiles of
+                // M = Y^T Y per group of block rows.  A CTA takes a Gram ticket only when (a) every task the group's rows depend on
+                // has been DRAWN (a critical ticket of a later column was handed out), so that it cannot starve them of CTAs,
+                // (b) the rows are factored (no waiting inside the task) and (c) the critical queue is at least m_lead block
+                // columns ahead of the chain -- or when the critical queue is empty.  A ticket claimed too early (a race at a
+                // group boundary) is HELD while the CTA goes on with critical tasks, so no CTA ever waits on an undrawn task.
+                for (;;) {
+                    const int front = df_ld_relaxed(g.ctrl + 3), drawn = df_ld_relaxed(g.ctrl + 4);
+                    const bool crit_left = df_ld_relaxed(g.ctrl) < g.total;
+                    auto runnable = [&](int tm) {
+                        int kb_, ke_;
+                        df_group_rows(tm / g.m_tiles, g.nb, g.mg, g.m_full, kb_, ke_);
+                        const int last_row = ke_ - 1;
+                        return !crit_left || (drawn > last_row && last_row + 2 <= front);
+                    };
+                    if (held_m < 0) {
+                        const int tm = df_ld_relaxed(g.ctrl + 2);
+                        if (tm < g.m_total && runnable(tm) && (!crit_left || drawn - front >= g.m_lead)) {
+                            const int got = atomicAdd(g.ctrl + 2, 1);
+                            if (got < g.m_total) held_m = got;
+                        }
+                    }
+                    if (held_m >= 0 && runnable(held_m)) {
+                        kind = 3; c = held_m / g.m_tiles; idx = held_m % g.m_tiles;
+                        int ti = 0;
+                        while ((ti + 1) * (ti + 2) / 2 <= idx) ti++;
+                        aux = idx - ti * (ti + 1) / 2;        // tile (ti, aux), aux <= ti
+                        idx = ti;
+                        held_m = -1;
+                        break;
+                    }
+                    if (crit_left) {
+                        t = atomicAdd(g.ctrl, 1);
+                        if (t < g.total) break;
+                        t = -1;
+                        continue;
+                    }
+                    if (held_m < 0 && df_ld_relaxed(g.ctrl + 2) >= g.m_total) break;      // both queues are empty
+                }
+            }
+            if (t == 0) {
+                kind = 2; idx = 0;            // chain task 0: the first diagonal block
+            } else if (t > 0 && t < g.total) {
+                // Ticket order: per block column c -- the chain tasks PLACED there, the tiles (i, c) below the sub-diagonal, the
+                // Y tiles of block row c.  Chain task d (k loop of d - 1 tile pairs: the longest task of its column) is placed
+                // d / chain_la columns AHEAD of column d - 1, so that its accumulation is done by the time W_{d-1} arrives; it
+                // then waits on a few tiles with later tickets, which the other CTAs go on drawing (at most nb / chain_la + 1
+                // CTAs can ever be in that state).  Measured at N = 4096 with 1344 right-hand sides: 2.47 -> 2.12 ms.  Pulling
+                // the near-diagonal tiles forward as well made it slower (2.14 .. 2.41 ms): they crowd out the bulk.
+                // (a CTA's tickets only grow: the scan resumes at the column of its previous ticket -- dec_c, dec_dnext, dec_base)
+                for (;;) {
+                    int nchain = 0;
+                    while (dec_dnext + nchain < g.nb) {
+                        const int d = dec_dnext + nchain;
+                        const int place = max(0, d - 1 - (g.chain_la > 0 ? d / g.chain_la : 0));
+                        if (place != dec_c) break;
+                        nchain++;
+                    }
+                    const int ntile = g.nb - dec_c - 2 > 0 ? g.nb - dec_c - 2 : 0;
+                    const int n = nchain + ntile + g.nr;
+                    if (t < dec_base + n) {
+                        const int tl = t - dec_base;
+                        c = dec_c;
+                        if (tl < nchain) { kind = 2; idx = dec_dnext + tl; }
+                        else if (tl < nchain + ntile) { kind = 0; idx = c + 2 + (tl - nchain); }
+                        else { kind = 1; idx = tl - nchain - ntile; }
+                        break;
+                    }
+                    dec_base += n; dec_c++; dec_dnext += nchain;
+                }
+                if (g.M != nullptr) atomicMax(g.ctrl + 4, c);
+            }
+            task[3] = aux;
+            task[0] = kind; task[1] = c; task[2] = idx;
+            task[4] = dec_s[4]; task[5] = dec_s[5];
+        }
+        __syncthreads();
+        const int kind = task[0], idx = task[2];
+        if (kind < 0) {
+            if (tracing && tid == 0) {
+                unsigned long long tg;
+                asm volatile("mov.u64 %0, %%globaltimer;\n" : "=l"(tg));
+                long long* o = g.trace + 1024 * 16 + (int64_t)blockIdx.x * 8;
+                o[0] = t_wait; o[1] = t_loop; o[2] = clock64() - t_begin; o[3] = n_tasks; o[4] = (long long)tg; o[5] = my_pause() - g.pause;
+            }
+            return;
+        }
+        n_tasks++;
+        const bool rhs = kind == 1, chain = kind == 2, gram = kind == 3;
+        const bool bkn = rhs || gram;                                    // B operand stored [k][n] (rows of Y)
+        // c = block column whose diagonal inverse finishes the task; i = block row of the A operand / output tile
+        // (Gram task: task[1] = group of block rows, tile (idx, task[3]) of M)
+        const int c = chain ? idx - 1 : (gram ? 0 : task[1]);
+        const int i = rhs ? c : idx;
+        const int gi = gram ? task[1] : 0, tj = task[3];
+        int kb = 0, ke_g = 0;                                            // Gram task: block rows [kb, ke_g) of Y
+        if (gram) df_group_rows(gi, g.nb, g.mg, g.m_full, kb, ke_g);
+        const int nk = gram ? ke_g - kb : (chain ? (idx > 0 ? idx - 1 : 0) : c);      // k tiles accumulated before the epilogue
+        const int* fa = gram ? g.flagsY + (int64_t)kb * g.nr + idx : g.flagsL + (int64_t)i * g.nb;   // A tile of k tile kt ready
+        const int* fb = gram ? g.flagsY + (int64_t)kb * g.nr + tj
+                             : (rhs ? g.flagsY + idx : g.flagsL + (int64_t)(c > 0 ? c : 0) * g.nb);  // Y_k,r (stride nr) or L_c,k
+        const int fas = gram ? g.nr : 1, fbs = bkn ? g.nr : 1;
+        const int nslab = nk * (PB / DF_K);
+        if (gram && gi > 0) {                         // the tile's sum over the earlier groups must be final
+            if (tracing) t_mark = clock64();
+            if (producer) {
+                const bool w = df_wait(df_out(g, task).flag - g.m_tiles, g.ctrl, g.info, g.spin_limit);
+                if (lane == 0) ready_s[2] = w ? 1 : 0;
+            }
+            __syncthreads();
+            if (tracing) t_wait += clock64() - t_mark;
+            if (ready_s[2] == 0) return;              // abort raised (uniform)
+        }
+
+        if (producer) {
+            // ---- producer: flags -> one TMA copy per operand of slab s into ring slot (task[4] + s) % 3 ----------------------
+            // operands of the k loop: A = L_i,k ([m][k]) or Y_k,ti ([k][m]);  B = L_c,k ([n][k], transposed product) or Y_k,r ([k][n])
+            const CUtensorMap* amap = gram ? &bmap : &kmap;
+            const CUtensorMap* bsrc = bkn ? &bmap : &kmap;
+            const int a_col = gram ? idx * PB : 0, a_row = gram ? kb * PB : i * PB;           // + s * DF_K on the k axis
+            const int b_col = gram ? tj * PB : (rhs ? idx * PB : 0);
+            const int b_row = gram ? kb * PB : (rhs ? 0 : (c > 0 ? c : 0) * PB);
+            const uint32_t bytes = (gram ? DF_KN_BYTES : DF_MK_BYTES) + (bkn ? DF_KN_BYTES : DF_MK_BYTES);
+            int ready_kt = -1, paused = 0;
+            for (int s = 0; s < nslab; s++) {
+                const bool fresh = (s >> 1) > ready_kt;           // tiles newly acquired for this slab
+                if (fresh) {
+                    const int r = df_poll_tiles(fa, fas, fb, fbs, s >> 1, nk, g.ctrl, g.info, g.spin_limit);
+                    if (r < 0) {                      // abort: keep the ring moving (the consumers must not be left waiting)
+                        if (lane == 0) abort_s = 1;
+                        ready_kt = nk;
+                    } else {
+                        ready_kt = r;
+                    }
+                }
+                if (lane == 0) {
+                    const unsigned gs = (unsigned)task[4] + s;
+                    const int slot = gs % DF_NSTAGE;
+                    // the SM's other CTA is in a chain tail: the flag is cleared at the end of every chain task that set it, and the
+                    // abort flag ends the wait as well (this thread feeds the consumers: a hang here would hang them on full[slot])
+                    while (paused && df_ld_relaxed(my_pause()) && !*reinterpret_cast<volatile int*>(g.ctrl + 1)) __nanosleep(200);
+                    if (gs >= DF_NSTAGE) mbar_wait(bar_empty + 8 * slot, ((gs / DF_NSTAGE) + 1) & 1);
+                    if (fresh) asm volatile("fence.proxy.async.global;\n" ::: "memory");   // acquired tiles -> reads by the TMA engine
+                    const uint32_t fbar = bar_full + 8 * slot;
+                    mbar_arrive_expect_tx(fbar, bytes);
+                    const int k0 = s * DF_K;
+                    tma_load_2d(smem_u32(As0 + slot * DF_STAGE), amap, gram ? a_col : k0, gram ? a_row + k0 : a_row, fbar);
+                    tma_load_2d(smem_u32(Bs0 + slot * DF_STAGE), bsrc, bkn ? b_col : k0, bkn ? b_row + k0 : b_row, fbar);
+                    paused = df_ld_relaxed(my_pause());   // (sampled one slab ahead: the load is off the critical path)
+                }
+            }
+            if (lane == 0) dec_s[4] += nslab;
+            __syncthreads();                          // the consumers are out of the last slab: the ring is free
+            if (abort_s) return;
+            if (gram || (chain && idx == 0)) continue;
+            // the epilogue's W_cc tile, into the Ws region of the consumers' epilogue
+            const bool w = df_wait(g.flagsL + (int64_t)c * g.nb + c, g.ctrl, g.info, g.spin_limit);
+            if (lane == 0) {
+                ready_s[3] = w ? 1 : 0;
+                dec_s[5]++;
+                if (w) {
+                    if (chain) df_st_relaxed(my_pause(), 1);
+                    asm volatile("fence.proxy.async.global;\n" ::: "memory");
+                    mbar_arrive_expect_tx(bar_w, DF_TILE_BYTES);
+                    tma_load_2d(smem_u32(df_smem + DF_TILE), &wmap, c * PB, c * PB, bar_w);
+                } else {
+                    mbar_arrive(bar_w);               // release the consumers, who then see ready_s[3] == 0
+                }
+            }
+            if (!w) return;
+            continue;
+        }
+
+        // ---- consumers ----
+        // The accumulators START at minus the tile they will be subtracted from (A_ic or B_cr; chain tasks: also A_dd), so the
+        // global reads of those tiles happen here, at the head of the task, instead of on the critical tail behind the flag.
+        // (Gram task: at plus the tile's sum over the earlier groups, once that is flagged.)
+        const bool has_tile = gram ? gi > 0 : !(chain && idx == 0);
+        double acc[2][4][2], acc2[2][4][2];
+        const DfOut in = df_out(g, task);
+#pragma unroll
+        for (int x = 0; x < 2; x++)
+#pragma unroll
+            for (int y = 0; y < 4; y++) {
+                const int r = wm + x * 32 + gq, cc = wn + y * 16 + tq * 2;
+                double2 v = make_double2(0.0, 0.0), d = make_double2(0.0, 0.0);
+                if (has_tile) v = *reinterpret_cast<const double2*>(in.Ct + (int64_t)r * in.ldc + cc);
+                if (chain) d = *reinterpret_cast<const double2*>(in.Cd + (int64_t)r * g.ld + cc);
+                acc[x][y][0] = gram ? v.x : -v.x; acc[x][y][1] = gram ? v.y : -v.y;
+                acc2[x][y][0] = -d.x; acc2[x][y][1] = -d.y;
+            }
+
+        auto compute = [&](int slot) {                // one 64 x 64 x 32 slab out of ring slot `slot`
+            const double* As = As0 + slot * DF_STAGE;
+            const double* Bs = Bs0 + slot * DF_STAGE;
+#pragma unroll
+            for (int kk = 0; kk < DF_K; kk += 4) {
+                double a[2], b[4];
+#pragma unroll
+                for (int x = 0; x < 2; x++)
+                    a[x] = gram ? As[(kk + tq) * DF_LDT + wm + x * 32 + gq] : As[(wm + x * 32 + gq) * DF_LDA + kk + tq];
+#pragma unroll
+                for (int y = 0; y < 4; y++)
+                    b[y] = bkn ? Bs[(kk + tq) * DF_LDT + wn + y * 16 + gq] : Bs[(wn + y * 16 + gq) * DF_LDA + kk + tq];
+#pragma unroll
+                for (int x = 0; x < 2; x++)
+#pragma unroll
+                    for (int y = 0; y < 4; y++) dmma884(acc[x][y][0], acc[x][y][1], a[x], b[y]);
+                if (chain) {                          // diagonal tile (i, i): L_ik L_ik^T out of the same A slab, lower tiles only
+#pragma unroll
+                    for (int y = 0; y < 4; y++) b[y] = As[(wn + y * 16 + gq) * DF_LDA + kk + tq];
+#pragma unroll
+                    for (int x = 0; x < 2; x++)
+#pragma unroll
+                        for (int y = 0; y < 4; y++)
+                            if (wn + y * 16 < wm + x * 32 + 8) dmma884(acc2[x][y][0], acc2[x][y][1], a[x], b[y]);
+                }
+            }
+        };
+        // k loop: wait for the slab, DMMA loop, hand the ring slot back -- no CTA-wide barrier
+        const long long t_loop0 = tracing ? clock64() : 0;
+        const unsigned gs0 = task[4];
+        for (int s = 0; s < nslab; s++) {
+            const unsigned gs = gs0 + s;
+            const int slot = gs % DF_NSTAGE;
+            if (tracing) t_mark = clock64();
+            mbar_wait(bar_full + 8 * slot, (gs / DF_NSTAGE) & 1);
+            if (tracing) t_wait += clock64() - t_mark;
+            compute(slot);
+            __syncwarp();
+            if (lane == 0) mbar_arrive(bar_empty + 8 * slot);
+        }
+        __syncthreads();                              // every warp is out of the last slab: shared memory is free for the epilogue
+        if (abort_s) return;                          // abort raised in the k loop (uniform: written before the barrier)
+
+        // ---- epilogue (consumer warps only; tile_bar) ----
+        if (tracing) t_loop += clock64() - t_loop0;
+        if (chain) df_stamp(g.trace, idx, 0);
+        double* Xs = df_smem;                 // [64][68]  X = C - acc   (later: the diagonal tile S)
+        double* Ws = df_smem + DF_TILE;       // [64][68]  W_cc (TMA, issued by the producer)
+        double* Ls = df_smem + 2 * DF_TILE;   // [64][68]  L_{i,c} of a chain task
+        const DfOut out = df_out(g, task);
+        double* const Ct = out.Ct;
+        const int64_t ldc = out.ldc;
+        double* const Cd = out.Cd;
+        if (gram) {                                   // the tile's sum over groups 0 .. gi, back in place
+#pragma unroll
+            for (int x = 0; x < 2; x++)
+#pragma unroll
+                for (int y = 0; y < 4; y++) {
+                    const int r = wm + x * 32 + gq, cc = wn + y * 16 + tq * 2;
+                    double2 v;
+                    v.x = acc[x][y][0]; v.y = acc[x][y][1];
+                    *reinterpret_cast<double2*>(Ct + (int64_t)r * ldc + cc) = v;
+                }
+        } else if (!(chain && idx == 0)) {
+#pragma unroll
+            for (int x = 0; x < 2; x++)
+#pragma unroll
+                for (int y = 0; y < 4; y++) {
+                    const int r = wm + x * 32 + gq, cc = wn + y * 16 + tq * 2;
+                    Xs[r * DF_LDT + cc] = -acc[x][y][0];              // X = C - sum (the accumulator started at -C)
+                    Xs[r * DF_LDT + cc + 1] = -acc[x][y][1];
+                    acc[x][y][0] = acc[x][y][1] = 0.0;
+                }
+            if (tracing) t_mark = clock64();
+            tile_bar();                               // X is in shared memory
+            if (chain) df_stamp(g.trace, idx, 1);
+            mbar_wait(bar_w, task[5] & 1);            // W_cc is final (the producer acquired its flag) and in shared memory
+            if (tracing) t_wait += clock64() - t_mark;
+            if (ready_s[3] == 0) return;              // abort raised (uniform: written before the producer's arrival)
+            if (chain) df_stamp(g.trace, idx, 2);
+#pragma unroll 4
+            for (int kk = 0; kk < PB; kk += 4) {
+                double a[2], b[4];
+                if (!rhs) {       // L_ic = X W_cc^T :  A = X [m][k],  B = W_cc [n][k] (lower triangular: k < n0 + 8)
+#pragma unroll
+                    for (int x = 0; x < 2; x++) a[x] = Xs[(wm + x * 32 + gq) * DF_LDT + kk + tq];
+#pragma unroll
+                    for (int y = 0; y < 4; y++) b[y] = (kk < wn + y * 16 + 8) ? Ws[(wn + y * 16 + gq) * DF_LDT + kk + tq] : 0.0;
+#pragma unroll
+                    for (int x = 0; x < 2; x++)
+#pragma unroll
+                        for (int y = 0; y < 4; y++)
+                            if (kk < wn + y * 16 + 8) dmma884(acc[x][y][0], acc[x][y][1], a[x], b[y]);
+                    continue;
+                } else {          // Y_cr = W_cc X :    A = W_cc [m][k],  B = X [k][n]
+#pragma unroll
+                    for (int x = 0; x < 2; x++) a[x] = Ws[(wm + x * 32 + gq) * DF_LDT + kk + tq];
+#pragma unroll
+                    for (int y = 0; y < 4; y++) b[y] = Xs[(kk + tq) * DF_LDT + wn + y * 16 + gq];
+                }
+#pragma unroll
+                for (int x = 0; x < 2; x++)
+#pragma unroll
+                    for (int y = 0; y < 4; y++) dmma884(acc[x][y][0], acc[x][y][1], a[x], b[y]);
+            }
+#pragma unroll
+            for (int x = 0; x < 2; x++)
+#pragma unroll
+                for (int y = 0; y < 4; y++) {
+                    const int r = wm + x * 32 + gq, cc = wn + y * 16 + tq * 2;
+                    double2 v;
+                    v.x = acc[x][y][0]; v.y = acc[x][y][1];
+                    *reinterpret_cast<double2*>(Ct + (int64_t)r * ldc + cc) = v;
+                    if (chain) { Ls[r * DF_LDT + cc] = v.x; Ls[r * DF_LDT + cc + 1] = v.y; }
+                }
+        }
+        if (chain) {
+            double* Wd = g.W + (int64_t)idx * PB * (g.ldw + 1);
+            df_stamp(g.trace, idx, 3);
+            if (idx > 0) {
+                tile_bar();                           // L_{i,c} complete in shared memory; X is free
+#pragma unroll 4
+                for (int kk = 0; kk < PB; kk += 4) {  // acc2 += L_ic L_ic^T
+                    double a[2], b[4];
+#pragma unroll
+                    for (int x = 0; x < 2; x++) a[x] = Ls[(wm + x * 32 + gq) * DF_LDT + kk + tq];
+#pragma unroll
+                    for (int y = 0; y < 4; y++) b[y] = Ls[(wn + y * 16 + gq) * DF_LDT + kk + tq];
+#pragma unroll
+                    for (int x = 0; x < 2; x++)
+#pragma unroll
+                        for (int y = 0; y < 4; y++)
+                            if (wn + y * 16 < wm + x * 32 + 8) dmma884(acc2[x][y][0], acc2[x][y][1], a[x], b[y]);
+                }
+            }
+#pragma unroll
+            for (int x = 0; x < 2; x++)
+#pragma unroll
+                for (int y = 0; y < 4; y++) {
+                    const int r = wm + x * 32 + gq, cc = wn + y * 16 + tq * 2;
+                    Xs[r * DF_LDT + cc] = -acc2[x][y][0];             // S = A_dd - sum (acc2 started at -A_dd)
+                    Xs[r * DF_LDT + cc + 1] = -acc2[x][y][1];
+                }
+            if (idx > 0) {                            // publish the sub-diagonal tile before the long factor step
+                tile_bar();                           // (release by one thread after the barrier covers the CTA's writes)
+                if (tid == 0) df_publish(out.flag);
+            } else {
+                tile_bar();
+            }
+            df_stamp(g.trace, idx, 4);
+            // Two-level factor + inverse of the 64x64 diagonal tile S (in Xs): the pair-step sweep is latency-bound per step, and a
+            // 32x32 block needs half the steps at half the work per step, so  [S11 .; S21 S22] -> L11, W11 = L11^-1 (sweep);
+            // L21 = S21 W11^T; S22 -= L21 L21^T; L22, W22 (sweep); W21 = -W22 (L21 W11), the four small products on DMMA.
+            {
+                PotrfScratch* sc = reinterpret_cast<PotrfScratch*>(Ws);       // W_cc is spent
+                constexpr int H = PB / 2, LO = DF_LDT;
+                double* L11s = Ls;                       // rows 0..31 of the Ls region: [L11 | W11]
+                double* W11s = Ls + H;
+                double* L21s = Ls + H * LO;              // rows 32..63: [L21 | T = L21 W11]
+                double* Tsm = Ls + H * LO + H;
+                double* W22s = Xs;                       // S11 is consumed by then
+                // 32x32x32 products on DMMA: warp w owns row tile w >> 1 and the column tiles 2 (w & 1), 2 (w & 1) + 1
+                const int m0 = (warp >> 1) * 8, n0 = (warp & 1) * 16;
+                auto mm32 = [&](const double* A, const double* B, bool b_nk, double (&c)[2][2]) {
+                    c[0][0] = c[0][1] = c[1][0] = c[1][1] = 0.0;
+#pragma unroll
+                    for (int kk = 0; kk < H; kk += 4) {
+                        const double av = A[(m0 + gq) * LO + kk + tq];
+#pragma unroll
+                        for (int j = 0; j < 2; j++) {
+                            const double bv = b_nk ? B[(n0 + 8 * j + gq) * LO + kk + tq] : B[(kk + tq) * LO + n0 + 8 * j + gq];
+                            dmma884(c[j][0], c[j][1], av, bv);
+                        }
+                    }
+                };
+                double c[2][2];
+                potrf_diag_body<H>(Xs, LO, Cd, g.ld, Wd, g.ldw, g.info, idx * PB, sc, L11s, W11s, LO);
+                tile_bar();
+                mm32(Xs + H * LO, W11s, true, c);                    // L21 = S21 W11^T  (W11's upper part is stored as zeros)
+#pragma unroll
+                for (int j = 0; j < 2; j++) {
+                    const int r = m0 + gq, cc = n0 + 8 * j + tq * 2;
+                    *reinterpret_cast<double2*>(Cd + (int64_t)(H + r) * g.ld + cc) = make_double2(c[j][0], c[j][1]);
+                    L21s[r * LO + cc] = c[j][0]; L21s[r * LO + cc + 1] = c[j][1];
+                }
+                tile_bar();
+                mm32(L21s, L21s, true, c);                           // S22 -= L21 L21^T
+#pragma unroll
+                for (int j = 0; j < 2; j++) {
+                    const int r = m0 + gq, cc = n0 + 8 * j + tq * 2;
+                    Xs[(H + r) * LO + H + cc] -= c[j][0]; Xs[(H + r) * LO + H + cc + 1] -= c[j][1];
+                }
+                tile_bar();
+                potrf_diag_body<H>(Xs + H * LO + H, LO, Cd + (int64_t)H * g.ld + H, g.ld, Wd + (int64_t)H * g.ldw + H, g.ldw, g.info,
+                                   idx * PB + H, sc, nullptr, W22s, LO);
+                tile_bar();
+                mm32(L21s, W11s, false, c);                          // T = L21 W11
+#pragma unroll
+                for (int j = 0; j < 2; j++) {
+                    const int r = m0 + gq, cc = n0 + 8 * j + tq * 2;
+                    Tsm[r * LO + cc] = c[j][0]; Tsm[r * LO + cc + 1] = c[j][1];
+                }
+                tile_bar();
+                mm32(W22s, Tsm, false, c);                           // W21 = -W22 T;  W12 = 0
+#pragma unroll
+                for (int j = 0; j < 2; j++) {
+                    const int r = m0 + gq, cc = n0 + 8 * j + tq * 2;
+                    *reinterpret_cast<double2*>(Wd + (int64_t)(H + r) * g.ldw + cc) = make_double2(-c[j][0], -c[j][1]);
+                    *reinterpret_cast<double2*>(Wd + (int64_t)r * g.ldw + H + cc) = make_double2(0.0, 0.0);
+                }
+            }
+            df_stamp(g.trace, idx, 5);
+        }
+        tile_bar();
+        if (tid == 0) {
+            df_publish(chain ? g.flagsL + (int64_t)idx * g.nb + idx : out.flag);     // covers the tile stores of every thread before the barrier
+            if (chain) {
+                df_st_relaxed(my_pause(), 0);
+                if (g.M != nullptr) atomicMax(g.ctrl + 3, idx + 1);       // diagonal blocks factored (the Gram queue's gate)
+            }
+        }
+        if (chain) df_stamp(g.trace, idx, 6);
+    }
+}
+
+// The same tasks with the k loop of the 256-thread form: every thread stages its share of each slab with 16-byte cp.async and
+// the CTA meets at one barrier per slab.  Used below DF_TMA_MIN_NB block columns, where the chain of diagonal blocks sets the
+// time: its per-column hop is ~0.9 us shorter here than in the producer-warp kernel (which runs at <= 112 registers), and that
+// outweighs the k-loop throughput the TMA ring gains (profiles/r03_chol_tma_ab.txt).
+__global__ void __launch_bounds__(DF_THREADS, 2) chol_dataflow_cpasync_kernel(DfArgs g) {
+    extern __shared__ __align__(16) double df_smem_c[];
+    double* df_smem = df_smem_c;
     __shared__ int task[4];
     __shared__ int ready_s[4];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -937,11 +1498,28 @@ int side_for_current_device(SideStream** out) {
 }  // namespace
 
 namespace {
-struct DfScratch {        // diagnostics (MFGP_DF_TRACE=1) and the cached SM count only; no data-path state
+// A tensor map of chol_dataflow_kernel, kept while the next call passes the same buffer and shape (a step refactors the same
+// buffers, so the maps are encoded once).
+struct DfMap {
+    const double* base = nullptr;
+    int64_t rows = 0, cols = 0, ld = 0;
+    CUtensorMap map;
+};
+int df_cached_map(DfMap& m, const double* base, int64_t rows, int64_t cols, int64_t ld, int box_cols, int box_rows) {
+    if (m.base == base && m.rows == rows && m.cols == cols && m.ld == ld) return MFGP_OK;
+    m.base = nullptr;
+    const int rc = make_tensor_map_2d(&m.map, base, rows, cols, ld, box_cols, box_rows, CU_TENSOR_MAP_SWIZZLE_NONE);
+    if (rc) return rc;
+    m.base = base; m.rows = rows; m.cols = cols; m.ld = ld;
+    return MFGP_OK;
+}
+
+struct DfScratch {        // diagnostics (MFGP_DF_TRACE=1), the cached SM count and tensor maps; no data-path state
     long long* trace = nullptr;
     int trace_nb = 0;
     int trace_grid = 0;
     int sms = 0;
+    DfMap kmap, bmap, wmap;
 };
 DfScratch g_df[16];
 
@@ -993,13 +1571,29 @@ int chol_dataflow(double* K, int64_t npad, int64_t ld, double* W, int64_t ldw, i
     static const int chain_la = [] { const char* e = getenv("MFGP_DF_CHAIN_LA"); return e ? atoi(e) : 5; }();
     a.chain_la = chain_la;
     a.spin_limit = 4000000000LL;      // ~2 s of SM clocks: only a bug can get there
-    constexpr int smem = DF_SMEM_DOUBLES * sizeof(double);
+    // TMA operands: boxes of [m][k] slabs of K / L (36 x 64), [k][n] slabs of B / Y (68 x 32) and the W_cc tile (68 x 64);
+    // rows must start 16-byte aligned
+    auto aligned = [](const void* p, int64_t l) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0 && (l & 1) == 0; };
+    if (!aligned(K, ld) || !aligned(W, ldw) || (nr > 0 && !aligned(Bm, ldb))) return MFGP_ERR_INVALID;
     static const int occ = [] { const char* e = getenv("MFGP_DF_OCC"); return e ? atoi(e) : 2; }();
-    MFGP_CUDA_CHECK(cudaFuncSetAttribute(chol_dataflow_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     int grid = (occ < 1 ? 1 : occ) * sc.sms;
     if (grid > a.total + a.m_total) grid = a.total + a.m_total;
     sc.trace_grid = grid < 1024 ? grid : 1024;
-    chol_dataflow_kernel<<<grid, DF_THREADS, smem, st>>>(a);
+    if (nb < DF_TMA_MIN_NB) {         // chain-bound: the cp.async kernel's shorter hop per block column wins
+        constexpr int smem_c = DF_SMEM_DOUBLES * sizeof(double);
+        MFGP_CUDA_CHECK(cudaFuncSetAttribute(chol_dataflow_cpasync_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_c));
+        chol_dataflow_cpasync_kernel<<<grid, DF_THREADS, smem_c, st>>>(a);
+        MFGP_LAUNCH_CHECK();
+        return MFGP_OK;
+    }
+    int rc = df_cached_map(sc.kmap, K, npad, npad, ld, DF_LDA, PB);
+    if (!rc) rc = df_cached_map(sc.wmap, W, npad, npad, ldw, DF_LDT, PB);
+    if (!rc && nr > 0) rc = df_cached_map(sc.bmap, Bm, npad, R, ldb, DF_LDT, DF_K);
+    if (rc) return rc;
+    constexpr int smem = DF_SMEM_BYTES;
+    MFGP_CUDA_CHECK(cudaFuncSetAttribute(chol_dataflow_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    // (without right-hand sides no task reads the B / Y map)
+    chol_dataflow_kernel<<<grid, DF_CTA_THREADS, smem, st>>>(sc.kmap.map, nr > 0 ? sc.bmap.map : sc.kmap.map, sc.wmap.map, a);
     MFGP_LAUNCH_CHECK();
     return MFGP_OK;
 }

@@ -61,32 +61,9 @@ struct PostArgs {
     DevParams p;
 };
 
-// ---- mbarrier / TMA / setmaxnreg primitives (PTX) ---------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return static_cast<uint32_t>(__cvta_generic_to_shared(p)); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;\n" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];\n" ::"r"(bar) : "memory");
-}
+// ---- setmaxnreg / expect-tx primitives (PTX; mbarrier and TMA: common.cuh) --------------------------------------------
 __device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {   // adds to the tx-count, no arrival
     asm volatile("mbarrier.expect_tx.relaxed.cta.shared::cta.b64 [%0], %1;\n" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    uint32_t done;
-    do {
-        asm volatile(
-            "{\n .reg .pred p;\n mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n selp.u32 %0, 1, 0, p;\n}\n"
-            : "=r"(done)
-            : "r"(bar), "r"(parity)
-            : "memory");
-    } while (!done);
-}
-__device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* map, int c0, int c1, uint32_t bar) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];\n" ::"r"(dst),
-        "l"(map), "r"(c0), "r"(c1), "r"(bar)
-        : "memory");
 }
 template <int R>
 __device__ __forceinline__ void reg_alloc() { asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;\n" ::"n"(R)); }
@@ -644,35 +621,9 @@ __global__ void grid_tables_kernel(const double* __restrict__ u, int nu, int axi
     TH[(int64_t)iu * ldt + n] = vh;
 }
 
-// cuTensorMapEncodeTiled through the runtime's driver entry point query (no link-time dependency on libcuda)
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
+// 16 doubles (128 B) x 256 (or 64) rows of W per box; out-of-range rows read as zero
 static int make_w_tensor_map(CUtensorMap* map, const double* W, int64_t npad, int64_t ldw, int box_rows = P_BM / 2) {
-    static EncodeTiledFn encode = nullptr;
-    if (!encode) {
-        void* fn = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        MFGP_CUDA_CHECK(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres));
-        if (qres != cudaDriverEntryPointSuccess || !fn) {
-            set_last_error("cuTensorMapEncodeTiled entry point unavailable", cudaErrorUnknown);
-            return MFGP_ERR_CUDA;
-        }
-        encode = reinterpret_cast<EncodeTiledFn>(fn);
-    }
-    const cuuint64_t gdim[2] = {(cuuint64_t)npad, (cuuint64_t)npad};       // {columns (contiguous), rows}
-    const cuuint64_t gstride[1] = {(cuuint64_t)ldw * sizeof(double)};      // row pitch in bytes
-    const cuuint32_t box[2] = {(cuuint32_t)P_BK, (cuuint32_t)box_rows};    // 16 doubles (128 B) x 256 (or 64) rows
-    const cuuint32_t estr[2] = {1, 1};
-    const CUresult r = encode(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 2, const_cast<double*>(W), gdim, gstride, box, estr,
-                              CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);          // out-of-range rows read as zero
-    if (r != CUDA_SUCCESS) {
-        set_last_error("cuTensorMapEncodeTiled failed", cudaErrorInvalidValue);
-        return MFGP_ERR_CUDA;
-    }
-    return MFGP_OK;
+    return make_tensor_map_2d(map, W, npad, npad, ldw, P_BK, box_rows, CU_TENSOR_MAP_SWIZZLE_128B);
 }
 
 }  // namespace mfgp

@@ -157,8 +157,7 @@ int64_t mfgp_factored_workspace_bytes(int64_t npad, int64_t ncols, int64_t ny, i
  *   mfgp_build_train_cov  ->  mfgp_factored_prepare (B = [B_L | B_H | y - mean], mfgp_factored_rhs_cols columns)
  *   ->  mfgp_cholesky_solve (K -> L in place, diagonal-block inverses into W, Ball -> L^-1 Ball: ONE persistent
  *       tile-dataflow kernel, chol_dataflow_kernel in csrc/gp_fit.cu; its ticket counter and ready flags live in `work`,
- *       mfgp_cholesky_solve_workspace_bytes(npad, R) bytes of caller memory, so the call is re-entrant per work buffer.
- *       MFGP_CHOL=chain in the environment selects the older launch-per-panel implementation)
+ *       mfgp_cholesky_solve_workspace_bytes(npad, R) bytes of caller memory, so the call is re-entrant per work buffer)
  *   ->  mfgp_posterior_grid_factored_solved (steps 4-6; z_out receives the whitened observations).
  * Neither the explicit inverse (mfgp_tri_inverse) nor the product W B is formed; run mfgp_tri_inverse afterwards only if W
  * is needed (dense posterior, mfgp_cholesky_append, choi_greedy).  Same geometry / order arguments and the same `work`

@@ -3,7 +3,6 @@
 #include "common.cuh"
 #include "gemm_f64.cuh"
 #include <cstdlib>
-#include <cstring>
 
 namespace mfgp {
 
@@ -95,8 +94,8 @@ struct PotrfScratch {
 // BS = 64: the whole tile (s, m: 4x4 cyclic sub-blocks per thread); BS = 32: one half of the two-level form below (2x2).
 // `col0`: global index of the block's first column (for the failing-pivot report).  Ls / Wsm (optional, shared memory, row
 // stride lds_out): copies of L and of its inverse for the caller's next step.
-// Barrier of the 256 threads that work on a tile: the whole CTA of potrf_diag_kernel, the consumer warps of
-// chol_dataflow_kernel (whose ninth warp, the producer, does not take part in the epilogue).
+// Barrier of the 256 threads that work on a tile: the whole CTA of potrf_diag_kernel and chol_dataflow_cpasync_kernel, the
+// consumer warps of chol_dataflow_kernel (whose ninth warp, the producer, does not take part in the epilogue).
 __device__ __forceinline__ void tile_bar() { asm volatile("bar.sync 1, 256;\n" ::: "memory"); }
 
 template <int BS>
@@ -245,7 +244,9 @@ __global__ void __launch_bounds__(256, 1) potrf_diag_kernel(double* __restrict__
 // them); a bounded spin (abort flag) guards against bugs all the same.
 // Two CTAs share an SM; while one of them runs the latency-bound tail of a chain task it raises a per-SM pause flag and
 // the other one idles between its k slabs (its DMMA traffic would otherwise stretch the chain by ~25%).
-// Warp-specialised: 8 consumer warps run the DMMA loops and the epilogues; a ninth, producer warp draws the tickets, polls
+// Two forms of the kernel run the same task body (below) with different k loops.  chol_dataflow_cpasync_kernel: 256 threads
+// stage each slab with cp.async and meet at one barrier per slab.  chol_dataflow_kernel, warp-specialised: 8 consumer warps
+// run the DMMA loops and the epilogues; a ninth, producer warp draws the tickets, polls
 // the tile flags and moves every slab with ONE 2D TMA copy per operand into a 3-slot ring (full / empty mbarriers), so the
 // k loop has no CTA-wide barrier and no per-thread copy issue.  The TMA boxes are 4 doubles wider than the slab: the
 // 4 columns past it land as the row padding that puts the 8 rows of a DMMA
@@ -333,11 +334,13 @@ __device__ __forceinline__ int df_ld_relaxed(const int* p) {
 __device__ __forceinline__ void df_st_release(int* p, int v) {
     asm volatile("st.release.gpu.global.s32 [%0], %1;\n" ::"l"(p), "r"(v) : "memory");
 }
-// Publishes a tile: the CTA's stores of it (ordered before this thread by a barrier) are written with generic stores but read by
-// later tasks through the async proxy (TMA), so a proxy fence precedes the release of the flag (the reader adds one after its
-// acquire).  One thread, after the barrier: a fence in every thread would drain every thread's stores on the chain's path.
+// Publishes a tile: one thread releases its flag after a barrier that orders the CTA's stores of it.  kTma: the tiles are read
+// by later tasks through the async proxy (TMA, chol_dataflow_kernel), so a proxy fence precedes the release (the reader adds
+// one after its acquire); in one thread, after the barrier, because a fence in every thread would drain every thread's stores
+// on the chain's path.  The cp.async form reads the tiles with generic loads and releases without the fence.
+template <bool kTma>
 __device__ __forceinline__ void df_publish(int* flag) {
-    asm volatile("fence.proxy.async.global;\n" ::: "memory");
+    if constexpr (kTma) asm volatile("fence.proxy.async.global;\n" ::: "memory");
     df_st_release(flag, 1);
 }
 __device__ __forceinline__ void df_st_relaxed(int* p, int v) {
@@ -361,29 +364,6 @@ __device__ __forceinline__ bool df_wait(const int* f, int* ctrl, int32_t* info, 
     ok = __shfl_sync(0xffffffffu, ok, 0);
     __syncwarp();                 // shuffles carry no memory ordering: order lane 0's acquire before the other lanes' tile loads
     return ok != 0;
-}
-
-// Output of the task in task[] (kind, column, index, aux): the tile the accumulators start from and the task writes (row stride
-// ldc), the diagonal tile of a chain task, and the flag that publishes the tile.  Derived from the shared task[] where used: held
-// in registers across the k loop, these pointers would spill.
-struct DfOut {
-    double* Ct; int64_t ldc;
-    double* Cd;
-    int* flag;
-};
-__device__ __forceinline__ DfOut df_out(const DfArgs& g, const int* task) {
-    const int kind = task[0], idx = task[2], tj = task[3];
-    const bool rhs = kind == 1, chain = kind == 2, gram = kind == 3;
-    const int c = chain ? idx - 1 : (gram ? 0 : task[1]), cc = c > 0 ? c : 0;
-    const int i = rhs ? c : idx;
-    DfOut o;
-    o.Ct = gram ? g.M + (int64_t)idx * PB * g.ldm + (int64_t)tj * PB
-                : (rhs ? g.Bm + (int64_t)c * PB * g.ldb + (int64_t)idx * PB : g.K + (int64_t)i * PB * g.ld + (int64_t)cc * PB);
-    o.ldc = gram ? g.ldm : (rhs ? g.ldb : g.ld);
-    o.Cd = g.K + (int64_t)(chain ? idx : 0) * PB * (g.ld + 1);
-    o.flag = gram ? g.flagsM + (int64_t)task[1] * g.m_tiles + idx * (idx + 1) / 2 + tj
-                  : (rhs ? g.flagsY + (int64_t)c * g.nr + idx : g.flagsL + (int64_t)i * g.nb + cc);   // chain: tile (idx, idx - 1)
-    return o;
 }
 
 // The producer's flag check for the k tiles kt0, kt0 + 1, ... of a task: lane j < 16 reads the flag of the A tile of k tile
@@ -417,6 +397,418 @@ __device__ __forceinline__ int df_poll_tiles(const int* fa, int fas, const int* 
     }
 }
 
+// ---- the task body, shared by both forms of the kernel ----------------------------------------------------------------
+// chol_dataflow_kernel (producer warp, TMA ring) and chol_dataflow_cpasync_kernel (256 threads, cp.async ring) differ in how the
+// slabs and the W_cc tile reach shared memory and in how the CTA synchronises around them; they draw, decode, accumulate and
+// finish their tasks through the functions below, which synchronise the 256 computing threads with tile_bar().
+
+// Draws the CTA's next task into task[0..3] = kind (0: tile of L, 1: tile of Y, 2: chain task, 3: Gram task; -1: both queues
+// are empty), column, index, aux.  Called by one thread of the CTA, whose state across calls is held_m (a Gram ticket claimed
+// before it became runnable; initially -1) and the decoder's column, next chain task to place and that column's first ticket
+// (dec_c, dec_dnext, dec_base; initially 0, 1, 1).
+__device__ __forceinline__ void df_next_task(const DfArgs& g, int& held_m, int& dec_c, int& dec_dnext, int& dec_base, int* task) {
+    int c = 0, kind = -1, idx = 0, aux = 0;
+    int t = -1;
+    if (g.M == nullptr) {
+        t = atomicAdd(g.ctrl, 1);
+    } else {
+        // Two queues.  Critical = the factorisation and the substitution (ticket order as below); Gram = the tiles of
+        // M = Y^T Y per group of block rows.  A CTA takes a Gram ticket only when (a) every task the group's rows depend on
+        // has been DRAWN (a critical ticket of a later column was handed out), so that it cannot starve them of CTAs,
+        // (b) the rows are factored (no waiting inside the task) and (c) the critical queue is at least m_lead block
+        // columns ahead of the chain -- or when the critical queue is empty.  A ticket claimed too early (a race at a
+        // group boundary) is HELD while the CTA goes on with critical tasks, so no CTA ever waits on an undrawn task.
+        for (;;) {
+            const int front = df_ld_relaxed(g.ctrl + 3), drawn = df_ld_relaxed(g.ctrl + 4);
+            const bool crit_left = df_ld_relaxed(g.ctrl) < g.total;
+            auto runnable = [&](int tm) {
+                int kb_, ke_;
+                df_group_rows(tm / g.m_tiles, g.nb, g.mg, g.m_full, kb_, ke_);
+                const int last_row = ke_ - 1;
+                return !crit_left || (drawn > last_row && last_row + 2 <= front);
+            };
+            if (held_m < 0) {
+                const int tm = df_ld_relaxed(g.ctrl + 2);
+                if (tm < g.m_total && runnable(tm) && (!crit_left || drawn - front >= g.m_lead)) {
+                    const int got = atomicAdd(g.ctrl + 2, 1);
+                    if (got < g.m_total) held_m = got;
+                }
+            }
+            if (held_m >= 0 && runnable(held_m)) {
+                kind = 3; c = held_m / g.m_tiles; idx = held_m % g.m_tiles;
+                int ti = 0;
+                while ((ti + 1) * (ti + 2) / 2 <= idx) ti++;
+                aux = idx - ti * (ti + 1) / 2;        // tile (ti, aux), aux <= ti
+                idx = ti;
+                held_m = -1;
+                break;
+            }
+            if (crit_left) {
+                t = atomicAdd(g.ctrl, 1);
+                if (t < g.total) break;
+                t = -1;
+                continue;
+            }
+            if (held_m < 0 && df_ld_relaxed(g.ctrl + 2) >= g.m_total) break;      // both queues are empty
+        }
+    }
+    if (t == 0) {
+        kind = 2; idx = 0;            // chain task 0: the first diagonal block
+    } else if (t > 0 && t < g.total) {
+        // Ticket order: per block column c -- the chain tasks PLACED there, the tiles (i, c) below the sub-diagonal, the
+        // Y tiles of block row c.  Chain task d (k loop of d - 1 tile pairs: the longest task of its column) is placed
+        // d / chain_la columns AHEAD of column d - 1, so that its accumulation is done by the time W_{d-1} arrives; it
+        // then waits on a few tiles with later tickets, which the other CTAs go on drawing (at most nb / chain_la + 1
+        // CTAs can ever be in that state).  Measured at N = 4096 with 1344 right-hand sides: 2.47 -> 2.12 ms.  Pulling
+        // the near-diagonal tiles forward as well made it slower (2.14 .. 2.41 ms): they crowd out the bulk.
+        // (a CTA's tickets only grow: the scan resumes at the column of its previous ticket -- dec_c, dec_dnext, dec_base)
+        for (;;) {
+            int nchain = 0;
+            while (dec_dnext + nchain < g.nb) {
+                const int d = dec_dnext + nchain;
+                const int place = max(0, d - 1 - (g.chain_la > 0 ? d / g.chain_la : 0));
+                if (place != dec_c) break;
+                nchain++;
+            }
+            const int ntile = g.nb - dec_c - 2 > 0 ? g.nb - dec_c - 2 : 0;
+            const int n = nchain + ntile + g.nr;
+            if (t < dec_base + n) {
+                const int tl = t - dec_base;
+                c = dec_c;
+                if (tl < nchain) { kind = 2; idx = dec_dnext + tl; }
+                else if (tl < nchain + ntile) { kind = 0; idx = c + 2 + (tl - nchain); }
+                else { kind = 1; idx = tl - nchain - ntile; }
+                break;
+            }
+            dec_base += n; dec_c++; dec_dnext += nchain;
+        }
+        if (g.M != nullptr) atomicMax(g.ctrl + 4, c);
+    }
+    task[3] = aux;
+    task[0] = kind; task[1] = c; task[2] = idx;
+}
+
+__device__ __forceinline__ unsigned df_smid() {
+    unsigned smid;
+    asm volatile("mov.u32 %0, %%smid;\n" : "=r"(smid));
+    return smid;
+}
+// This SM's pause flag (re-derived where used: a pointer held across the k loop costs registers)
+__device__ __forceinline__ int* df_pause_flag(const DfArgs& g) { return g.pause + df_smid(); }
+
+// Per-CTA accounting (MFGP_DF_ACCOUNTING builds): SM clocks spent waiting (tile flags, slabs), in k loops and in total, the
+// number of tasks, the exit time and the SM
+__device__ __forceinline__ void df_exit_record(const DfArgs& g, long long t_wait, long long t_loop, long long t_begin, int n_tasks) {
+    unsigned long long tg;
+    asm volatile("mov.u64 %0, %%globaltimer;\n" : "=l"(tg));
+    long long* o = g.trace + 1024 * 16 + (int64_t)blockIdx.x * 8;
+    o[0] = t_wait; o[1] = t_loop; o[2] = clock64() - t_begin; o[3] = n_tasks; o[4] = (long long)tg; o[5] = df_smid();
+}
+
+// Geometry of the task in task[].  c = block column whose diagonal inverse finishes the task; i = block row of the A operand /
+// output tile (Gram task: task[1] = group gi of block rows [kb, kb + nk) of Y, tile (idx, tj) of M).  The k loop accumulates nk
+// k tiles in nslab slabs; the A / B tiles of k tile kt are flagged ready at fa[kt * fas] / fb[kt * fbs].
+struct DfTask {
+    int kind, idx, c, i, gi, tj, kb, nk, nslab, fas, fbs;
+    bool rhs, chain, gram, bkn;                  // bkn: B operand stored [k][n] (rows of Y)
+    const int* fa;
+    const int* fb;
+};
+__device__ __forceinline__ DfTask df_task(const DfArgs& g, const int* task) {
+    DfTask t;
+    t.kind = task[0]; t.idx = task[2]; t.tj = task[3];
+    t.rhs = t.kind == 1; t.chain = t.kind == 2; t.gram = t.kind == 3; t.bkn = t.rhs || t.gram;
+    t.c = t.chain ? t.idx - 1 : (t.gram ? 0 : task[1]);
+    t.i = t.rhs ? t.c : t.idx;
+    t.gi = t.gram ? task[1] : 0;
+    int ke = 0;
+    t.kb = 0;
+    if (t.gram) df_group_rows(t.gi, g.nb, g.mg, g.m_full, t.kb, ke);
+    t.nk = t.gram ? ke - t.kb : (t.chain ? (t.idx > 0 ? t.idx - 1 : 0) : t.c);
+    t.nslab = t.nk * (PB / DF_K);
+    t.fa = t.gram ? g.flagsY + (int64_t)t.kb * g.nr + t.idx : g.flagsL + (int64_t)t.i * g.nb;         // Y_k,idx or L_i,k
+    t.fb = t.gram ? g.flagsY + (int64_t)t.kb * g.nr + t.tj
+                  : (t.rhs ? g.flagsY + t.idx : g.flagsL + (int64_t)(t.c > 0 ? t.c : 0) * g.nb);   // Y_k,r (stride nr) or L_c,k
+    t.fas = t.gram ? g.nr : 1;
+    t.fbs = t.bkn ? g.nr : 1;
+    return t;
+}
+
+// Output of the task in task[]: the tile the accumulators start from and the task writes (row stride ldc), the diagonal tile of
+// a chain task, and the flag that publishes the tile.  Derived from the shared task[] where used: held in registers across the
+// k loop, these pointers would spill.
+struct DfOut {
+    double* Ct; int64_t ldc;
+    double* Cd;
+    int* flag;
+};
+__device__ __forceinline__ DfOut df_out(const DfArgs& g, const int* task) {
+    const int kind = task[0], idx = task[2], tj = task[3];
+    const bool rhs = kind == 1, chain = kind == 2, gram = kind == 3;
+    const int c = chain ? idx - 1 : (gram ? 0 : task[1]), cc = c > 0 ? c : 0;
+    const int i = rhs ? c : idx;
+    DfOut o;
+    o.Ct = gram ? g.M + (int64_t)idx * PB * g.ldm + (int64_t)tj * PB
+                : (rhs ? g.Bm + (int64_t)c * PB * g.ldb + (int64_t)idx * PB : g.K + (int64_t)i * PB * g.ld + (int64_t)cc * PB);
+    o.ldc = gram ? g.ldm : (rhs ? g.ldb : g.ld);
+    o.Cd = g.K + (int64_t)(chain ? idx : 0) * PB * (g.ld + 1);
+    o.flag = gram ? g.flagsM + (int64_t)task[1] * g.m_tiles + idx * (idx + 1) / 2 + tj
+                  : (rhs ? g.flagsY + (int64_t)c * g.nr + idx : g.flagsL + (int64_t)i * g.nb + cc);   // chain: tile (idx, idx - 1)
+    return o;
+}
+
+// The 256 computing threads' share of a task's 64x64 tiles, as DMMA accumulator fragments: acc the output tile, acc2 the
+// diagonal tile of a chain task.  8 warps as 4 x 2; a warp owns the 8x8 tiles (row tile (warp>>1) + 4x, column tile (warp&1) + 2y),
+// x < 2, y < 4 -- interleaved, so that the triangular products of the chain task (W_cc lower, S symmetric) skip about the same
+// share of DMMAs in every warp.  The epilogue's shared memory: X (later the diagonal tile S) at smem, W_cc at smem + DF_TILE,
+// L_{i,c} of a chain task at smem + 2 DF_TILE, each [64][68].
+struct DfTile {
+    int wm, wn, gq, tq;
+    double acc[2][4][2], acc2[2][4][2];
+
+    // tid: the kernel's threadIdx.x, whose range the compiler knows from the kernel's launch bounds (the 256-thread kernel
+    // then drops the DMMAs of the triangular products that no warp runs)
+    __device__ __forceinline__ explicit DfTile(int tid) {
+        const int lane = tid & 31, warp = tid >> 5;
+        wm = (warp >> 1) * 8; wn = (warp & 1) * 8;
+        gq = lane >> 2; tq = lane & 3;
+    }
+
+    // The accumulators START at minus the tile they will be subtracted from (A_ic or B_cr; chain tasks: also A_dd), so the
+    // global reads of those tiles happen here, at the head of the task, instead of on the critical tail behind the flag.
+    // (Gram task: at plus the tile's sum over the earlier groups, once that is flagged.)
+    __device__ __forceinline__ void start(const DfArgs& g, const int* task, const DfTask& tk) {
+        const bool has_tile = tk.gram ? tk.gi > 0 : !(tk.chain && tk.idx == 0);
+        const DfOut in = df_out(g, task);
+#pragma unroll
+        for (int x = 0; x < 2; x++)
+#pragma unroll
+            for (int y = 0; y < 4; y++) {
+                const int r = wm + x * 32 + gq, cc = wn + y * 16 + tq * 2;
+                double2 v = make_double2(0.0, 0.0), d = make_double2(0.0, 0.0);
+                if (has_tile) v = *reinterpret_cast<const double2*>(in.Ct + (int64_t)r * in.ldc + cc);
+                if (tk.chain) d = *reinterpret_cast<const double2*>(in.Cd + (int64_t)r * g.ld + cc);
+                acc[x][y][0] = tk.gram ? v.x : -v.x; acc[x][y][1] = tk.gram ? v.y : -v.y;
+                acc2[x][y][0] = -d.x; acc2[x][y][1] = -d.y;
+            }
+    }
+
+    // One 64 x 64 x 32 slab of the k loop out of shared memory (A at As, B at Bs)
+    __device__ __forceinline__ void slab(const double* As, const double* Bs, const DfTask& tk) {
+#pragma unroll
+        for (int kk = 0; kk < DF_K; kk += 4) {
+            double a[2], b[4];
+#pragma unroll
+            for (int x = 0; x < 2; x++)
+                a[x] = tk.gram ? As[(kk + tq) * DF_LDT + wm + x * 32 + gq] : As[(wm + x * 32 + gq) * DF_LDA + kk + tq];
+#pragma unroll
+            for (int y = 0; y < 4; y++)
+                b[y] = tk.bkn ? Bs[(kk + tq) * DF_LDT + wn + y * 16 + gq] : Bs[(wn + y * 16 + gq) * DF_LDA + kk + tq];
+#pragma unroll
+            for (int x = 0; x < 2; x++)
+#pragma unroll
+                for (int y = 0; y < 4; y++) dmma884(acc[x][y][0], acc[x][y][1], a[x], b[y]);
+            if (tk.chain) {                           // diagonal tile (i, i): L_ik L_ik^T out of the same A slab, lower tiles only
+#pragma unroll
+                for (int y = 0; y < 4; y++) b[y] = As[(wn + y * 16 + gq) * DF_LDA + kk + tq];
+#pragma unroll
+                for (int x = 0; x < 2; x++)
+#pragma unroll
+                    for (int y = 0; y < 4; y++)
+                        if (wn + y * 16 < wm + x * 32 + 8) dmma884(acc2[x][y][0], acc2[x][y][1], a[x], b[y]);
+            }
+        }
+    }
+
+    // Gram task: the tile's sum over groups 0 .. gi, back in place
+    __device__ __forceinline__ void store(double* Ct, int64_t ldc) const {
+#pragma unroll
+        for (int x = 0; x < 2; x++)
+#pragma unroll
+            for (int y = 0; y < 4; y++) {
+                const int r = wm + x * 32 + gq, cc = wn + y * 16 + tq * 2;
+                double2 v;
+                v.x = acc[x][y][0]; v.y = acc[x][y][1];
+                *reinterpret_cast<double2*>(Ct + (int64_t)r * ldc + cc) = v;
+            }
+    }
+
+    // X = C - sum into shared memory (the accumulator started at -C); the accumulator is free for the solve product
+    __device__ __forceinline__ void stage_x(double* smem) {
+        double* Xs = smem;
+#pragma unroll
+        for (int x = 0; x < 2; x++)
+#pragma unroll
+            for (int y = 0; y < 4; y++) {
+                const int r = wm + x * 32 + gq, cc = wn + y * 16 + tq * 2;
+                Xs[r * DF_LDT + cc] = -acc[x][y][0];
+                Xs[r * DF_LDT + cc + 1] = -acc[x][y][1];
+                acc[x][y][0] = acc[x][y][1] = 0.0;
+            }
+    }
+
+    // With X and W_cc in shared memory: the output tile L_ic = X W_cc^T or Y_cr = W_cc X, stored in place (chain task: also
+    // into the L region for the tail)
+    __device__ __forceinline__ void solve(double* smem, const DfTask& tk, const DfOut& out) {
+        const double* Xs = smem;
+        const double* Ws = smem + DF_TILE;
+        double* Ls = smem + 2 * DF_TILE;
+#pragma unroll 4
+        for (int kk = 0; kk < PB; kk += 4) {
+            double a[2], b[4];
+            if (!tk.rhs) {    // L_ic = X W_cc^T :  A = X [m][k],  B = W_cc [n][k] (lower triangular: k < n0 + 8)
+#pragma unroll
+                for (int x = 0; x < 2; x++) a[x] = Xs[(wm + x * 32 + gq) * DF_LDT + kk + tq];
+#pragma unroll
+                for (int y = 0; y < 4; y++) b[y] = (kk < wn + y * 16 + 8) ? Ws[(wn + y * 16 + gq) * DF_LDT + kk + tq] : 0.0;
+#pragma unroll
+                for (int x = 0; x < 2; x++)
+#pragma unroll
+                    for (int y = 0; y < 4; y++)
+                        if (kk < wn + y * 16 + 8) dmma884(acc[x][y][0], acc[x][y][1], a[x], b[y]);
+                continue;
+            } else {          // Y_cr = W_cc X :    A = W_cc [m][k],  B = X [k][n]
+#pragma unroll
+                for (int x = 0; x < 2; x++) a[x] = Ws[(wm + x * 32 + gq) * DF_LDT + kk + tq];
+#pragma unroll
+                for (int y = 0; y < 4; y++) b[y] = Xs[(kk + tq) * DF_LDT + wn + y * 16 + gq];
+            }
+#pragma unroll
+            for (int x = 0; x < 2; x++)
+#pragma unroll
+                for (int y = 0; y < 4; y++) dmma884(acc[x][y][0], acc[x][y][1], a[x], b[y]);
+        }
+#pragma unroll
+        for (int x = 0; x < 2; x++)
+#pragma unroll
+            for (int y = 0; y < 4; y++) {
+                const int r = wm + x * 32 + gq, cc = wn + y * 16 + tq * 2;
+                double2 v;
+                v.x = acc[x][y][0]; v.y = acc[x][y][1];
+                *reinterpret_cast<double2*>(out.Ct + (int64_t)r * out.ldc + cc) = v;
+                if (tk.chain) { Ls[r * DF_LDT + cc] = v.x; Ls[r * DF_LDT + cc + 1] = v.y; }
+            }
+    }
+
+    // 32x32x32 product on DMMA, c = A B^T (b_nk) or A B, row stride DF_LDT: warp w owns row tile w >> 1 and the column tiles
+    // 2 (w & 1), 2 (w & 1) + 1
+    __device__ __forceinline__ void mm32(const double* A, const double* B, bool b_nk, double (&c)[2][2]) const {
+        constexpr int H = PB / 2, LO = DF_LDT;
+        const int m0 = wm, n0 = 2 * wn;
+        c[0][0] = c[0][1] = c[1][0] = c[1][1] = 0.0;
+#pragma unroll
+        for (int kk = 0; kk < H; kk += 4) {
+            const double av = A[(m0 + gq) * LO + kk + tq];
+#pragma unroll
+            for (int j = 0; j < 2; j++) {
+                const double bv = b_nk ? B[(n0 + 8 * j + gq) * LO + kk + tq] : B[(kk + tq) * LO + n0 + 8 * j + gq];
+                dmma884(c[j][0], c[j][1], av, bv);
+            }
+        }
+    }
+
+    // Chain task d = idx, after its solve product (if d > 0): S = A_dd - sum_k L_dk L_dk^T (acc2, finished with L_{d,d-1} out of
+    // shared memory), the sub-diagonal tile published before the long factor step, then L_dd and W_dd = L_dd^-1 from S.
+    // kTma: the tiles are read through the async proxy (df_publish).
+    template <bool kTma>
+    __device__ __forceinline__ void chain_tail(const DfArgs& g, int idx, double* smem, const DfOut& out) {
+        double* Xs = smem;
+        double* Ls = smem + 2 * DF_TILE;
+        double* const Cd = out.Cd;
+        double* Wd = g.W + (int64_t)idx * PB * (g.ldw + 1);
+        df_stamp(g.trace, idx, 3);
+        if (idx > 0) {
+            tile_bar();                               // L_{i,c} complete in shared memory; X is free
+#pragma unroll 4
+            for (int kk = 0; kk < PB; kk += 4) {      // acc2 += L_ic L_ic^T
+                double a[2], b[4];
+#pragma unroll
+                for (int x = 0; x < 2; x++) a[x] = Ls[(wm + x * 32 + gq) * DF_LDT + kk + tq];
+#pragma unroll
+                for (int y = 0; y < 4; y++) b[y] = Ls[(wn + y * 16 + gq) * DF_LDT + kk + tq];
+#pragma unroll
+                for (int x = 0; x < 2; x++)
+#pragma unroll
+                    for (int y = 0; y < 4; y++)
+                        if (wn + y * 16 < wm + x * 32 + 8) dmma884(acc2[x][y][0], acc2[x][y][1], a[x], b[y]);
+            }
+        }
+#pragma unroll
+        for (int x = 0; x < 2; x++)
+#pragma unroll
+            for (int y = 0; y < 4; y++) {
+                const int r = wm + x * 32 + gq, cc = wn + y * 16 + tq * 2;
+                Xs[r * DF_LDT + cc] = -acc2[x][y][0];                 // S = A_dd - sum (acc2 started at -A_dd)
+                Xs[r * DF_LDT + cc + 1] = -acc2[x][y][1];
+            }
+        tile_bar();                                   // (release by one thread after the barrier covers the CTA's writes)
+        if (idx > 0 && threadIdx.x == 0) df_publish<kTma>(out.flag);      // the sub-diagonal tile, before the long factor step
+        df_stamp(g.trace, idx, 4);
+        // Two-level factor + inverse of the 64x64 diagonal tile S (in Xs): the pair-step sweep is latency-bound per step, and a
+        // 32x32 block needs half the steps at half the work per step, so  [S11 .; S21 S22] -> L11, W11 = L11^-1 (sweep);
+        // L21 = S21 W11^T; S22 -= L21 L21^T; L22, W22 (sweep); W21 = -W22 (L21 W11), the four small products on DMMA.
+        PotrfScratch* sc = reinterpret_cast<PotrfScratch*>(smem + DF_TILE);      // W_cc is spent
+        constexpr int H = PB / 2, LO = DF_LDT;
+        double* L11s = Ls;                           // rows 0..31 of the Ls region: [L11 | W11]
+        double* W11s = Ls + H;
+        double* L21s = Ls + H * LO;                  // rows 32..63: [L21 | T = L21 W11]
+        double* Tsm = Ls + H * LO + H;
+        double* W22s = Xs;                           // S11 is consumed by then
+        const int m0 = wm, n0 = 2 * wn;              // this thread's share of a 32x32 tile in mm32
+        double c[2][2];
+        potrf_diag_body<H>(Xs, LO, Cd, g.ld, Wd, g.ldw, g.info, idx * PB, sc, L11s, W11s, LO);
+        tile_bar();
+        mm32(Xs + H * LO, W11s, true, c);                            // L21 = S21 W11^T  (W11's upper part is stored as zeros)
+#pragma unroll
+        for (int j = 0; j < 2; j++) {
+            const int r = m0 + gq, cc = n0 + 8 * j + tq * 2;
+            *reinterpret_cast<double2*>(Cd + (int64_t)(H + r) * g.ld + cc) = make_double2(c[j][0], c[j][1]);
+            L21s[r * LO + cc] = c[j][0]; L21s[r * LO + cc + 1] = c[j][1];
+        }
+        tile_bar();
+        mm32(L21s, L21s, true, c);                                   // S22 -= L21 L21^T
+#pragma unroll
+        for (int j = 0; j < 2; j++) {
+            const int r = m0 + gq, cc = n0 + 8 * j + tq * 2;
+            Xs[(H + r) * LO + H + cc] -= c[j][0]; Xs[(H + r) * LO + H + cc + 1] -= c[j][1];
+        }
+        tile_bar();
+        potrf_diag_body<H>(Xs + H * LO + H, LO, Cd + (int64_t)H * g.ld + H, g.ld, Wd + (int64_t)H * g.ldw + H, g.ldw, g.info,
+                           idx * PB + H, sc, nullptr, W22s, LO);
+        tile_bar();
+        mm32(L21s, W11s, false, c);                                  // T = L21 W11
+#pragma unroll
+        for (int j = 0; j < 2; j++) {
+            const int r = m0 + gq, cc = n0 + 8 * j + tq * 2;
+            Tsm[r * LO + cc] = c[j][0]; Tsm[r * LO + cc + 1] = c[j][1];
+        }
+        tile_bar();
+        mm32(W22s, Tsm, false, c);                                   // W21 = -W22 T;  W12 = 0
+#pragma unroll
+        for (int j = 0; j < 2; j++) {
+            const int r = m0 + gq, cc = n0 + 8 * j + tq * 2;
+            *reinterpret_cast<double2*>(Wd + (int64_t)(H + r) * g.ldw + cc) = make_double2(-c[j][0], -c[j][1]);
+            *reinterpret_cast<double2*>(Wd + (int64_t)r * g.ldw + H + cc) = make_double2(0.0, 0.0);
+        }
+        df_stamp(g.trace, idx, 5);
+    }
+};
+
+// The end of every task: once all computing threads have stored their share, one thread publishes the output tile (chain task:
+// the diagonal block, L_dd and W_dd); a chain task also lowers the SM's pause flag and advances the Gram queue's gate.
+template <bool kTma>
+__device__ __forceinline__ void df_finish(const DfArgs& g, const DfTask& tk, int* flag) {
+    tile_bar();
+    if (threadIdx.x == 0) {
+        df_publish<kTma>(tk.chain ? g.flagsL + (int64_t)tk.idx * g.nb + tk.idx : flag);   // covers the tile stores before the barrier
+        if (tk.chain) {
+            df_st_relaxed(df_pause_flag(g), 0);
+            if (g.M != nullptr) atomicMax(g.ctrl + 3, tk.idx + 1);       // diagonal blocks factored (the Gram queue's gate)
+        }
+    }
+    if (tk.chain) df_stamp(g.trace, tk.idx, 6);
+}
+
 __global__ void __maxnreg__(112)        // 2 CTAs of 288 threads per SM: 2 x 288 x 112 <= 65536 registers
 chol_dataflow_kernel(const __grid_constant__ CUtensorMap kmap, const __grid_constant__ CUtensorMap bmap,
                      const __grid_constant__ CUtensorMap wmap, DfArgs g) {
@@ -439,18 +831,8 @@ chol_dataflow_kernel(const __grid_constant__ CUtensorMap kmap, const __grid_cons
         dec_s[0] = -1; dec_s[1] = 0; dec_s[2] = 1; dec_s[3] = 1; dec_s[4] = 0; dec_s[5] = 0;
         asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
     }
-    // 8 warps as 4 x 2; a warp owns the 8x8 tiles (row tile (warp>>1) + 4x, column tile (warp&1) + 2y), x < 2, y < 4 --
-    // interleaved, so that the triangular products of the chain task (W_cc lower, S symmetric) skip about the same share
-    // of DMMAs in every warp
-    const int wm = (warp >> 1) * 8, wn = (warp & 1) * 8;
-    const int gq = lane >> 2, tq = lane & 3;
     double* As0 = df_smem;
     double* Bs0 = df_smem + DF_NSTAGE * DF_STAGE;
-    auto my_pause = [&]() {                   // this SM's pause flag (re-derived: a pointer held across the loop costs registers)
-        unsigned smid;
-        asm volatile("mov.u32 %0, %%smid;\n" : "=r"(smid));
-        return g.pause + smid;
-    };
     // diagnostics (MFGP_DF_TRACE=1): SM clocks this CTA's thread 0 spent waiting (tile flags, slabs), in k loops, and in total
 #ifdef MFGP_DF_ACCOUNTING       // build with -DMFGP_DF_ACCOUNTING for profiles/tools/cta_account.py (costs ~10 registers)
     long long t_wait = 0, t_loop = 0, t_begin = clock64(), t_mark = 0;
@@ -462,126 +844,24 @@ chol_dataflow_kernel(const __grid_constant__ CUtensorMap kmap, const __grid_cons
     constexpr bool tracing = false;
 #endif
     // producer lane 0's state, kept in shared memory (it is touched once per task; registers are the consumers' budget):
-    // a Gram ticket claimed before it became runnable; the decoder's column, next chain task to place and its first ticket;
-    // the slabs this CTA has moved so far (ring slot = gs % 3, phase = gs / 3) and the W_cc tiles (phase of bar_w)
-    int& held_m = dec_s[0];
-    int& dec_c = dec_s[1];
-    int& dec_dnext = dec_s[2];
-    int& dec_base = dec_s[3];
+    // df_next_task's in dec_s[0..3]; the slabs this CTA has moved so far (ring slot = gs % 3, phase = gs / 3) and the W_cc
+    // tiles (phase of bar_w) in dec_s[4], dec_s[5]
 
     for (;;) {
         if (!producer) asm volatile("fence.proxy.async.shared::cta;\n" ::: "memory");   // epilogue stores before the next TMA writes
         __syncthreads();                      // the previous task is done with shared memory and task[]
         if (producer && lane == 0) {
-            int c = 0, kind = -1, idx = 0, aux = 0;
-            int t = -1;
-            if (g.M == nullptr) {
-                t = atomicAdd(g.ctrl, 1);
-            } else {
-                // Two queues.  Critical = the factorisation and the substitution (ticket order as below); Gram = the tiles of
-                // M = Y^T Y per group of block rows.  A CTA takes a Gram ticket only when (a) every task the group's rows depend on
-                // has been DRAWN (a critical ticket of a later column was handed out), so that it cannot starve them of CTAs,
-                // (b) the rows are factored (no waiting inside the task) and (c) the critical queue is at least m_lead block
-                // columns ahead of the chain -- or when the critical queue is empty.  A ticket claimed too early (a race at a
-                // group boundary) is HELD while the CTA goes on with critical tasks, so no CTA ever waits on an undrawn task.
-                for (;;) {
-                    const int front = df_ld_relaxed(g.ctrl + 3), drawn = df_ld_relaxed(g.ctrl + 4);
-                    const bool crit_left = df_ld_relaxed(g.ctrl) < g.total;
-                    auto runnable = [&](int tm) {
-                        int kb_, ke_;
-                        df_group_rows(tm / g.m_tiles, g.nb, g.mg, g.m_full, kb_, ke_);
-                        const int last_row = ke_ - 1;
-                        return !crit_left || (drawn > last_row && last_row + 2 <= front);
-                    };
-                    if (held_m < 0) {
-                        const int tm = df_ld_relaxed(g.ctrl + 2);
-                        if (tm < g.m_total && runnable(tm) && (!crit_left || drawn - front >= g.m_lead)) {
-                            const int got = atomicAdd(g.ctrl + 2, 1);
-                            if (got < g.m_total) held_m = got;
-                        }
-                    }
-                    if (held_m >= 0 && runnable(held_m)) {
-                        kind = 3; c = held_m / g.m_tiles; idx = held_m % g.m_tiles;
-                        int ti = 0;
-                        while ((ti + 1) * (ti + 2) / 2 <= idx) ti++;
-                        aux = idx - ti * (ti + 1) / 2;        // tile (ti, aux), aux <= ti
-                        idx = ti;
-                        held_m = -1;
-                        break;
-                    }
-                    if (crit_left) {
-                        t = atomicAdd(g.ctrl, 1);
-                        if (t < g.total) break;
-                        t = -1;
-                        continue;
-                    }
-                    if (held_m < 0 && df_ld_relaxed(g.ctrl + 2) >= g.m_total) break;      // both queues are empty
-                }
-            }
-            if (t == 0) {
-                kind = 2; idx = 0;            // chain task 0: the first diagonal block
-            } else if (t > 0 && t < g.total) {
-                // Ticket order: per block column c -- the chain tasks PLACED there, the tiles (i, c) below the sub-diagonal, the
-                // Y tiles of block row c.  Chain task d (k loop of d - 1 tile pairs: the longest task of its column) is placed
-                // d / chain_la columns AHEAD of column d - 1, so that its accumulation is done by the time W_{d-1} arrives; it
-                // then waits on a few tiles with later tickets, which the other CTAs go on drawing (at most nb / chain_la + 1
-                // CTAs can ever be in that state).  Measured at N = 4096 with 1344 right-hand sides: 2.47 -> 2.12 ms.  Pulling
-                // the near-diagonal tiles forward as well made it slower (2.14 .. 2.41 ms): they crowd out the bulk.
-                // (a CTA's tickets only grow: the scan resumes at the column of its previous ticket -- dec_c, dec_dnext, dec_base)
-                for (;;) {
-                    int nchain = 0;
-                    while (dec_dnext + nchain < g.nb) {
-                        const int d = dec_dnext + nchain;
-                        const int place = max(0, d - 1 - (g.chain_la > 0 ? d / g.chain_la : 0));
-                        if (place != dec_c) break;
-                        nchain++;
-                    }
-                    const int ntile = g.nb - dec_c - 2 > 0 ? g.nb - dec_c - 2 : 0;
-                    const int n = nchain + ntile + g.nr;
-                    if (t < dec_base + n) {
-                        const int tl = t - dec_base;
-                        c = dec_c;
-                        if (tl < nchain) { kind = 2; idx = dec_dnext + tl; }
-                        else if (tl < nchain + ntile) { kind = 0; idx = c + 2 + (tl - nchain); }
-                        else { kind = 1; idx = tl - nchain - ntile; }
-                        break;
-                    }
-                    dec_base += n; dec_c++; dec_dnext += nchain;
-                }
-                if (g.M != nullptr) atomicMax(g.ctrl + 4, c);
-            }
-            task[3] = aux;
-            task[0] = kind; task[1] = c; task[2] = idx;
+            df_next_task(g, dec_s[0], dec_s[1], dec_s[2], dec_s[3], task);
             task[4] = dec_s[4]; task[5] = dec_s[5];
         }
         __syncthreads();
-        const int kind = task[0], idx = task[2];
-        if (kind < 0) {
-            if (tracing && tid == 0) {
-                unsigned long long tg;
-                asm volatile("mov.u64 %0, %%globaltimer;\n" : "=l"(tg));
-                long long* o = g.trace + 1024 * 16 + (int64_t)blockIdx.x * 8;
-                o[0] = t_wait; o[1] = t_loop; o[2] = clock64() - t_begin; o[3] = n_tasks; o[4] = (long long)tg; o[5] = my_pause() - g.pause;
-            }
+        const DfTask tk = df_task(g, task);
+        if (tk.kind < 0) {
+            if (tracing && tid == 0) df_exit_record(g, t_wait, t_loop, t_begin, n_tasks);
             return;
         }
         n_tasks++;
-        const bool rhs = kind == 1, chain = kind == 2, gram = kind == 3;
-        const bool bkn = rhs || gram;                                    // B operand stored [k][n] (rows of Y)
-        // c = block column whose diagonal inverse finishes the task; i = block row of the A operand / output tile
-        // (Gram task: task[1] = group of block rows, tile (idx, task[3]) of M)
-        const int c = chain ? idx - 1 : (gram ? 0 : task[1]);
-        const int i = rhs ? c : idx;
-        const int gi = gram ? task[1] : 0, tj = task[3];
-        int kb = 0, ke_g = 0;                                            // Gram task: block rows [kb, ke_g) of Y
-        if (gram) df_group_rows(gi, g.nb, g.mg, g.m_full, kb, ke_g);
-        const int nk = gram ? ke_g - kb : (chain ? (idx > 0 ? idx - 1 : 0) : c);      // k tiles accumulated before the epilogue
-        const int* fa = gram ? g.flagsY + (int64_t)kb * g.nr + idx : g.flagsL + (int64_t)i * g.nb;   // A tile of k tile kt ready
-        const int* fb = gram ? g.flagsY + (int64_t)kb * g.nr + tj
-                             : (rhs ? g.flagsY + idx : g.flagsL + (int64_t)(c > 0 ? c : 0) * g.nb);  // Y_k,r (stride nr) or L_c,k
-        const int fas = gram ? g.nr : 1, fbs = bkn ? g.nr : 1;
-        const int nslab = nk * (PB / DF_K);
-        if (gram && gi > 0) {                         // the tile's sum over the earlier groups must be final
+        if (tk.gram && tk.gi > 0) {                   // the tile's sum over the earlier groups must be final
             if (tracing) t_mark = clock64();
             if (producer) {
                 const bool w = df_wait(df_out(g, task).flag - g.m_tiles, g.ctrl, g.info, g.spin_limit);
@@ -595,20 +875,20 @@ chol_dataflow_kernel(const __grid_constant__ CUtensorMap kmap, const __grid_cons
         if (producer) {
             // ---- producer: flags -> one TMA copy per operand of slab s into ring slot (task[4] + s) % 3 ----------------------
             // operands of the k loop: A = L_i,k ([m][k]) or Y_k,ti ([k][m]);  B = L_c,k ([n][k], transposed product) or Y_k,r ([k][n])
-            const CUtensorMap* amap = gram ? &bmap : &kmap;
-            const CUtensorMap* bsrc = bkn ? &bmap : &kmap;
-            const int a_col = gram ? idx * PB : 0, a_row = gram ? kb * PB : i * PB;           // + s * DF_K on the k axis
-            const int b_col = gram ? tj * PB : (rhs ? idx * PB : 0);
-            const int b_row = gram ? kb * PB : (rhs ? 0 : (c > 0 ? c : 0) * PB);
-            const uint32_t bytes = (gram ? DF_KN_BYTES : DF_MK_BYTES) + (bkn ? DF_KN_BYTES : DF_MK_BYTES);
+            const CUtensorMap* amap = tk.gram ? &bmap : &kmap;
+            const CUtensorMap* bsrc = tk.bkn ? &bmap : &kmap;
+            const int a_col = tk.gram ? tk.idx * PB : 0, a_row = tk.gram ? tk.kb * PB : tk.i * PB;   // + s * DF_K on the k axis
+            const int b_col = tk.gram ? tk.tj * PB : (tk.rhs ? tk.idx * PB : 0);
+            const int b_row = tk.gram ? tk.kb * PB : (tk.rhs ? 0 : (tk.c > 0 ? tk.c : 0) * PB);
+            const uint32_t bytes = (tk.gram ? DF_KN_BYTES : DF_MK_BYTES) + (tk.bkn ? DF_KN_BYTES : DF_MK_BYTES);
             int ready_kt = -1, paused = 0;
-            for (int s = 0; s < nslab; s++) {
+            for (int s = 0; s < tk.nslab; s++) {
                 const bool fresh = (s >> 1) > ready_kt;           // tiles newly acquired for this slab
                 if (fresh) {
-                    const int r = df_poll_tiles(fa, fas, fb, fbs, s >> 1, nk, g.ctrl, g.info, g.spin_limit);
+                    const int r = df_poll_tiles(tk.fa, tk.fas, tk.fb, tk.fbs, s >> 1, tk.nk, g.ctrl, g.info, g.spin_limit);
                     if (r < 0) {                      // abort: keep the ring moving (the consumers must not be left waiting)
                         if (lane == 0) abort_s = 1;
-                        ready_kt = nk;
+                        ready_kt = tk.nk;
                     } else {
                         ready_kt = r;
                     }
@@ -618,31 +898,31 @@ chol_dataflow_kernel(const __grid_constant__ CUtensorMap kmap, const __grid_cons
                     const int slot = gs % DF_NSTAGE;
                     // the SM's other CTA is in a chain tail: the flag is cleared at the end of every chain task that set it, and the
                     // abort flag ends the wait as well (this thread feeds the consumers: a hang here would hang them on full[slot])
-                    while (paused && df_ld_relaxed(my_pause()) && !*reinterpret_cast<volatile int*>(g.ctrl + 1)) __nanosleep(200);
+                    while (paused && df_ld_relaxed(df_pause_flag(g)) && !*reinterpret_cast<volatile int*>(g.ctrl + 1)) __nanosleep(200);
                     if (gs >= DF_NSTAGE) mbar_wait(bar_empty + 8 * slot, ((gs / DF_NSTAGE) + 1) & 1);
                     if (fresh) asm volatile("fence.proxy.async.global;\n" ::: "memory");   // acquired tiles -> reads by the TMA engine
                     const uint32_t fbar = bar_full + 8 * slot;
                     mbar_arrive_expect_tx(fbar, bytes);
                     const int k0 = s * DF_K;
-                    tma_load_2d(smem_u32(As0 + slot * DF_STAGE), amap, gram ? a_col : k0, gram ? a_row + k0 : a_row, fbar);
-                    tma_load_2d(smem_u32(Bs0 + slot * DF_STAGE), bsrc, bkn ? b_col : k0, bkn ? b_row + k0 : b_row, fbar);
-                    paused = df_ld_relaxed(my_pause());   // (sampled one slab ahead: the load is off the critical path)
+                    tma_load_2d(smem_u32(As0 + slot * DF_STAGE), amap, tk.gram ? a_col : k0, tk.gram ? a_row + k0 : a_row, fbar);
+                    tma_load_2d(smem_u32(Bs0 + slot * DF_STAGE), bsrc, tk.bkn ? b_col : k0, tk.bkn ? b_row + k0 : b_row, fbar);
+                    paused = df_ld_relaxed(df_pause_flag(g));   // (sampled one slab ahead: the load is off the critical path)
                 }
             }
-            if (lane == 0) dec_s[4] += nslab;
+            if (lane == 0) dec_s[4] += tk.nslab;
             __syncthreads();                          // the consumers are out of the last slab: the ring is free
             if (abort_s) return;
-            if (gram || (chain && idx == 0)) continue;
-            // the epilogue's W_cc tile, into the Ws region of the consumers' epilogue
-            const bool w = df_wait(g.flagsL + (int64_t)c * g.nb + c, g.ctrl, g.info, g.spin_limit);
+            if (tk.gram || (tk.chain && tk.idx == 0)) continue;
+            // the epilogue's W_cc tile, into the W_cc region of the consumers' epilogue
+            const bool w = df_wait(g.flagsL + (int64_t)tk.c * g.nb + tk.c, g.ctrl, g.info, g.spin_limit);
             if (lane == 0) {
                 ready_s[3] = w ? 1 : 0;
                 dec_s[5]++;
                 if (w) {
-                    if (chain) df_st_relaxed(my_pause(), 1);
+                    if (tk.chain) df_st_relaxed(df_pause_flag(g), 1);
                     asm volatile("fence.proxy.async.global;\n" ::: "memory");
                     mbar_arrive_expect_tx(bar_w, DF_TILE_BYTES);
-                    tma_load_2d(smem_u32(df_smem + DF_TILE), &wmap, c * PB, c * PB, bar_w);
+                    tma_load_2d(smem_u32(df_smem + DF_TILE), &wmap, tk.c * PB, tk.c * PB, bar_w);
                 } else {
                     mbar_arrive(bar_w);               // release the consumers, who then see ready_s[3] == 0
                 }
@@ -652,246 +932,43 @@ chol_dataflow_kernel(const __grid_constant__ CUtensorMap kmap, const __grid_cons
         }
 
         // ---- consumers ----
-        // The accumulators START at minus the tile they will be subtracted from (A_ic or B_cr; chain tasks: also A_dd), so the
-        // global reads of those tiles happen here, at the head of the task, instead of on the critical tail behind the flag.
-        // (Gram task: at plus the tile's sum over the earlier groups, once that is flagged.)
-        const bool has_tile = gram ? gi > 0 : !(chain && idx == 0);
-        double acc[2][4][2], acc2[2][4][2];
-        const DfOut in = df_out(g, task);
-#pragma unroll
-        for (int x = 0; x < 2; x++)
-#pragma unroll
-            for (int y = 0; y < 4; y++) {
-                const int r = wm + x * 32 + gq, cc = wn + y * 16 + tq * 2;
-                double2 v = make_double2(0.0, 0.0), d = make_double2(0.0, 0.0);
-                if (has_tile) v = *reinterpret_cast<const double2*>(in.Ct + (int64_t)r * in.ldc + cc);
-                if (chain) d = *reinterpret_cast<const double2*>(in.Cd + (int64_t)r * g.ld + cc);
-                acc[x][y][0] = gram ? v.x : -v.x; acc[x][y][1] = gram ? v.y : -v.y;
-                acc2[x][y][0] = -d.x; acc2[x][y][1] = -d.y;
-            }
-
-        auto compute = [&](int slot) {                // one 64 x 64 x 32 slab out of ring slot `slot`
-            const double* As = As0 + slot * DF_STAGE;
-            const double* Bs = Bs0 + slot * DF_STAGE;
-#pragma unroll
-            for (int kk = 0; kk < DF_K; kk += 4) {
-                double a[2], b[4];
-#pragma unroll
-                for (int x = 0; x < 2; x++)
-                    a[x] = gram ? As[(kk + tq) * DF_LDT + wm + x * 32 + gq] : As[(wm + x * 32 + gq) * DF_LDA + kk + tq];
-#pragma unroll
-                for (int y = 0; y < 4; y++)
-                    b[y] = bkn ? Bs[(kk + tq) * DF_LDT + wn + y * 16 + gq] : Bs[(wn + y * 16 + gq) * DF_LDA + kk + tq];
-#pragma unroll
-                for (int x = 0; x < 2; x++)
-#pragma unroll
-                    for (int y = 0; y < 4; y++) dmma884(acc[x][y][0], acc[x][y][1], a[x], b[y]);
-                if (chain) {                          // diagonal tile (i, i): L_ik L_ik^T out of the same A slab, lower tiles only
-#pragma unroll
-                    for (int y = 0; y < 4; y++) b[y] = As[(wn + y * 16 + gq) * DF_LDA + kk + tq];
-#pragma unroll
-                    for (int x = 0; x < 2; x++)
-#pragma unroll
-                        for (int y = 0; y < 4; y++)
-                            if (wn + y * 16 < wm + x * 32 + 8) dmma884(acc2[x][y][0], acc2[x][y][1], a[x], b[y]);
-                }
-            }
-        };
+        DfTile f(tid);
+        f.start(g, task, tk);
         // k loop: wait for the slab, DMMA loop, hand the ring slot back -- no CTA-wide barrier
         const long long t_loop0 = tracing ? clock64() : 0;
         const unsigned gs0 = task[4];
-        for (int s = 0; s < nslab; s++) {
+        for (int s = 0; s < tk.nslab; s++) {
             const unsigned gs = gs0 + s;
             const int slot = gs % DF_NSTAGE;
             if (tracing) t_mark = clock64();
             mbar_wait(bar_full + 8 * slot, (gs / DF_NSTAGE) & 1);
             if (tracing) t_wait += clock64() - t_mark;
-            compute(slot);
+            f.slab(As0 + slot * DF_STAGE, Bs0 + slot * DF_STAGE, tk);
             __syncwarp();
             if (lane == 0) mbar_arrive(bar_empty + 8 * slot);
         }
         __syncthreads();                              // every warp is out of the last slab: shared memory is free for the epilogue
         if (abort_s) return;                          // abort raised in the k loop (uniform: written before the barrier)
 
-        // ---- epilogue (consumer warps only; tile_bar) ----
+        // ---- epilogue (consumer warps only) ----
         if (tracing) t_loop += clock64() - t_loop0;
-        if (chain) df_stamp(g.trace, idx, 0);
-        double* Xs = df_smem;                 // [64][68]  X = C - acc   (later: the diagonal tile S)
-        double* Ws = df_smem + DF_TILE;       // [64][68]  W_cc (TMA, issued by the producer)
-        double* Ls = df_smem + 2 * DF_TILE;   // [64][68]  L_{i,c} of a chain task
+        if (tk.chain) df_stamp(g.trace, tk.idx, 0);
         const DfOut out = df_out(g, task);
-        double* const Ct = out.Ct;
-        const int64_t ldc = out.ldc;
-        double* const Cd = out.Cd;
-        if (gram) {                                   // the tile's sum over groups 0 .. gi, back in place
-#pragma unroll
-            for (int x = 0; x < 2; x++)
-#pragma unroll
-                for (int y = 0; y < 4; y++) {
-                    const int r = wm + x * 32 + gq, cc = wn + y * 16 + tq * 2;
-                    double2 v;
-                    v.x = acc[x][y][0]; v.y = acc[x][y][1];
-                    *reinterpret_cast<double2*>(Ct + (int64_t)r * ldc + cc) = v;
-                }
-        } else if (!(chain && idx == 0)) {
-#pragma unroll
-            for (int x = 0; x < 2; x++)
-#pragma unroll
-                for (int y = 0; y < 4; y++) {
-                    const int r = wm + x * 32 + gq, cc = wn + y * 16 + tq * 2;
-                    Xs[r * DF_LDT + cc] = -acc[x][y][0];              // X = C - sum (the accumulator started at -C)
-                    Xs[r * DF_LDT + cc + 1] = -acc[x][y][1];
-                    acc[x][y][0] = acc[x][y][1] = 0.0;
-                }
+        if (tk.gram) {
+            f.store(out.Ct, out.ldc);
+        } else if (!(tk.chain && tk.idx == 0)) {
+            f.stage_x(df_smem);
             if (tracing) t_mark = clock64();
             tile_bar();                               // X is in shared memory
-            if (chain) df_stamp(g.trace, idx, 1);
+            if (tk.chain) df_stamp(g.trace, tk.idx, 1);
             mbar_wait(bar_w, task[5] & 1);            // W_cc is final (the producer acquired its flag) and in shared memory
             if (tracing) t_wait += clock64() - t_mark;
             if (ready_s[3] == 0) return;              // abort raised (uniform: written before the producer's arrival)
-            if (chain) df_stamp(g.trace, idx, 2);
-#pragma unroll 4
-            for (int kk = 0; kk < PB; kk += 4) {
-                double a[2], b[4];
-                if (!rhs) {       // L_ic = X W_cc^T :  A = X [m][k],  B = W_cc [n][k] (lower triangular: k < n0 + 8)
-#pragma unroll
-                    for (int x = 0; x < 2; x++) a[x] = Xs[(wm + x * 32 + gq) * DF_LDT + kk + tq];
-#pragma unroll
-                    for (int y = 0; y < 4; y++) b[y] = (kk < wn + y * 16 + 8) ? Ws[(wn + y * 16 + gq) * DF_LDT + kk + tq] : 0.0;
-#pragma unroll
-                    for (int x = 0; x < 2; x++)
-#pragma unroll
-                        for (int y = 0; y < 4; y++)
-                            if (kk < wn + y * 16 + 8) dmma884(acc[x][y][0], acc[x][y][1], a[x], b[y]);
-                    continue;
-                } else {          // Y_cr = W_cc X :    A = W_cc [m][k],  B = X [k][n]
-#pragma unroll
-                    for (int x = 0; x < 2; x++) a[x] = Ws[(wm + x * 32 + gq) * DF_LDT + kk + tq];
-#pragma unroll
-                    for (int y = 0; y < 4; y++) b[y] = Xs[(kk + tq) * DF_LDT + wn + y * 16 + gq];
-                }
-#pragma unroll
-                for (int x = 0; x < 2; x++)
-#pragma unroll
-                    for (int y = 0; y < 4; y++) dmma884(acc[x][y][0], acc[x][y][1], a[x], b[y]);
-            }
-#pragma unroll
-            for (int x = 0; x < 2; x++)
-#pragma unroll
-                for (int y = 0; y < 4; y++) {
-                    const int r = wm + x * 32 + gq, cc = wn + y * 16 + tq * 2;
-                    double2 v;
-                    v.x = acc[x][y][0]; v.y = acc[x][y][1];
-                    *reinterpret_cast<double2*>(Ct + (int64_t)r * ldc + cc) = v;
-                    if (chain) { Ls[r * DF_LDT + cc] = v.x; Ls[r * DF_LDT + cc + 1] = v.y; }
-                }
+            if (tk.chain) df_stamp(g.trace, tk.idx, 2);
+            f.solve(df_smem, tk, out);
         }
-        if (chain) {
-            double* Wd = g.W + (int64_t)idx * PB * (g.ldw + 1);
-            df_stamp(g.trace, idx, 3);
-            if (idx > 0) {
-                tile_bar();                           // L_{i,c} complete in shared memory; X is free
-#pragma unroll 4
-                for (int kk = 0; kk < PB; kk += 4) {  // acc2 += L_ic L_ic^T
-                    double a[2], b[4];
-#pragma unroll
-                    for (int x = 0; x < 2; x++) a[x] = Ls[(wm + x * 32 + gq) * DF_LDT + kk + tq];
-#pragma unroll
-                    for (int y = 0; y < 4; y++) b[y] = Ls[(wn + y * 16 + gq) * DF_LDT + kk + tq];
-#pragma unroll
-                    for (int x = 0; x < 2; x++)
-#pragma unroll
-                        for (int y = 0; y < 4; y++)
-                            if (wn + y * 16 < wm + x * 32 + 8) dmma884(acc2[x][y][0], acc2[x][y][1], a[x], b[y]);
-                }
-            }
-#pragma unroll
-            for (int x = 0; x < 2; x++)
-#pragma unroll
-                for (int y = 0; y < 4; y++) {
-                    const int r = wm + x * 32 + gq, cc = wn + y * 16 + tq * 2;
-                    Xs[r * DF_LDT + cc] = -acc2[x][y][0];             // S = A_dd - sum (acc2 started at -A_dd)
-                    Xs[r * DF_LDT + cc + 1] = -acc2[x][y][1];
-                }
-            if (idx > 0) {                            // publish the sub-diagonal tile before the long factor step
-                tile_bar();                           // (release by one thread after the barrier covers the CTA's writes)
-                if (tid == 0) df_publish(out.flag);
-            } else {
-                tile_bar();
-            }
-            df_stamp(g.trace, idx, 4);
-            // Two-level factor + inverse of the 64x64 diagonal tile S (in Xs): the pair-step sweep is latency-bound per step, and a
-            // 32x32 block needs half the steps at half the work per step, so  [S11 .; S21 S22] -> L11, W11 = L11^-1 (sweep);
-            // L21 = S21 W11^T; S22 -= L21 L21^T; L22, W22 (sweep); W21 = -W22 (L21 W11), the four small products on DMMA.
-            {
-                PotrfScratch* sc = reinterpret_cast<PotrfScratch*>(Ws);       // W_cc is spent
-                constexpr int H = PB / 2, LO = DF_LDT;
-                double* L11s = Ls;                       // rows 0..31 of the Ls region: [L11 | W11]
-                double* W11s = Ls + H;
-                double* L21s = Ls + H * LO;              // rows 32..63: [L21 | T = L21 W11]
-                double* Tsm = Ls + H * LO + H;
-                double* W22s = Xs;                       // S11 is consumed by then
-                // 32x32x32 products on DMMA: warp w owns row tile w >> 1 and the column tiles 2 (w & 1), 2 (w & 1) + 1
-                const int m0 = (warp >> 1) * 8, n0 = (warp & 1) * 16;
-                auto mm32 = [&](const double* A, const double* B, bool b_nk, double (&c)[2][2]) {
-                    c[0][0] = c[0][1] = c[1][0] = c[1][1] = 0.0;
-#pragma unroll
-                    for (int kk = 0; kk < H; kk += 4) {
-                        const double av = A[(m0 + gq) * LO + kk + tq];
-#pragma unroll
-                        for (int j = 0; j < 2; j++) {
-                            const double bv = b_nk ? B[(n0 + 8 * j + gq) * LO + kk + tq] : B[(kk + tq) * LO + n0 + 8 * j + gq];
-                            dmma884(c[j][0], c[j][1], av, bv);
-                        }
-                    }
-                };
-                double c[2][2];
-                potrf_diag_body<H>(Xs, LO, Cd, g.ld, Wd, g.ldw, g.info, idx * PB, sc, L11s, W11s, LO);
-                tile_bar();
-                mm32(Xs + H * LO, W11s, true, c);                    // L21 = S21 W11^T  (W11's upper part is stored as zeros)
-#pragma unroll
-                for (int j = 0; j < 2; j++) {
-                    const int r = m0 + gq, cc = n0 + 8 * j + tq * 2;
-                    *reinterpret_cast<double2*>(Cd + (int64_t)(H + r) * g.ld + cc) = make_double2(c[j][0], c[j][1]);
-                    L21s[r * LO + cc] = c[j][0]; L21s[r * LO + cc + 1] = c[j][1];
-                }
-                tile_bar();
-                mm32(L21s, L21s, true, c);                           // S22 -= L21 L21^T
-#pragma unroll
-                for (int j = 0; j < 2; j++) {
-                    const int r = m0 + gq, cc = n0 + 8 * j + tq * 2;
-                    Xs[(H + r) * LO + H + cc] -= c[j][0]; Xs[(H + r) * LO + H + cc + 1] -= c[j][1];
-                }
-                tile_bar();
-                potrf_diag_body<H>(Xs + H * LO + H, LO, Cd + (int64_t)H * g.ld + H, g.ld, Wd + (int64_t)H * g.ldw + H, g.ldw, g.info,
-                                   idx * PB + H, sc, nullptr, W22s, LO);
-                tile_bar();
-                mm32(L21s, W11s, false, c);                          // T = L21 W11
-#pragma unroll
-                for (int j = 0; j < 2; j++) {
-                    const int r = m0 + gq, cc = n0 + 8 * j + tq * 2;
-                    Tsm[r * LO + cc] = c[j][0]; Tsm[r * LO + cc + 1] = c[j][1];
-                }
-                tile_bar();
-                mm32(W22s, Tsm, false, c);                           // W21 = -W22 T;  W12 = 0
-#pragma unroll
-                for (int j = 0; j < 2; j++) {
-                    const int r = m0 + gq, cc = n0 + 8 * j + tq * 2;
-                    *reinterpret_cast<double2*>(Wd + (int64_t)(H + r) * g.ldw + cc) = make_double2(-c[j][0], -c[j][1]);
-                    *reinterpret_cast<double2*>(Wd + (int64_t)r * g.ldw + H + cc) = make_double2(0.0, 0.0);
-                }
-            }
-            df_stamp(g.trace, idx, 5);
-        }
-        tile_bar();
-        if (tid == 0) {
-            df_publish(chain ? g.flagsL + (int64_t)idx * g.nb + idx : out.flag);     // covers the tile stores of every thread before the barrier
-            if (chain) {
-                df_st_relaxed(my_pause(), 0);
-                if (g.M != nullptr) atomicMax(g.ctrl + 3, idx + 1);       // diagonal blocks factored (the Gram queue's gate)
-            }
-        }
-        if (chain) df_stamp(g.trace, idx, 6);
+        if (tk.chain) f.chain_tail<true>(g, tk.idx, df_smem, out);
+        df_finish<true>(g, tk, out.flag);
     }
 }
 
@@ -900,21 +977,13 @@ chol_dataflow_kernel(const __grid_constant__ CUtensorMap kmap, const __grid_cons
 // time: its per-column hop is ~0.9 us shorter here than in the producer-warp kernel (which runs at <= 112 registers), and that
 // outweighs the k-loop throughput the TMA ring gains (profiles/r03_chol_tma_ab.txt).
 __global__ void __launch_bounds__(DF_THREADS, 2) chol_dataflow_cpasync_kernel(DfArgs g) {
-    extern __shared__ __align__(16) double df_smem_c[];
-    double* df_smem = df_smem_c;
+    extern __shared__ __align__(16) double df_smem[];
     __shared__ int task[4];
     __shared__ int ready_s[4];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    // 8 warps as 4 x 2; a warp owns the 8x8 tiles (row tile (warp>>1) + 4x, column tile (warp&1) + 2y), x < 2, y < 4 --
-    // interleaved, so that the triangular products of the chain task (W_cc lower, S symmetric) skip about the same share
-    // of DMMAs in every warp
-    const int wm = (warp >> 1) * 8, wn = (warp & 1) * 8;
-    const int gq = lane >> 2, tq = lane & 3;
     double* As0 = df_smem;
     double* Bs0 = df_smem + DF_NSTAGE * DF_STAGE;
-    unsigned smid;
-    asm volatile("mov.u32 %0, %%smid;\n" : "=r"(smid));
-    int* my_pause = g.pause + smid;
+    int* const my_pause = df_pause_flag(g);
     // diagnostics (MFGP_DF_TRACE=1): SM clocks this CTA spent waiting for tile flags, in k loops, and in total
 #ifdef MFGP_DF_ACCOUNTING       // build with -DMFGP_DF_ACCOUNTING for profiles/tools/cta_account.py (costs ~10 registers)
     long long t_wait = 0, t_loop = 0, t_begin = clock64(), t_mark = 0;
@@ -925,157 +994,35 @@ __global__ void __launch_bounds__(DF_THREADS, 2) chol_dataflow_cpasync_kernel(Df
     int n_tasks = 0;
     constexpr bool tracing = false;
 #endif
-    int held_m = -1;                          // thread 0: a Gram ticket claimed before it became runnable
-    int dec_c = 0, dec_dnext = 1, dec_base = 1;     // thread 0: ticket decoder state (column, next chain task to place, its first ticket)
+    int held_m = -1, dec_c = 0, dec_dnext = 1, dec_base = 1;      // thread 0: df_next_task's state
 
     for (;;) {
         __syncthreads();                      // the previous task is done with shared memory and task[]
-        if (tid == 0) {
-            int c = 0, kind = -1, idx = 0, aux = 0;
-            int t = -1;
-            if (g.M == nullptr) {
-                t = atomicAdd(g.ctrl, 1);
-            } else {
-                // Two queues.  Critical = the factorisation and the substitution (ticket order as below); Gram = the tiles of
-                // M = Y^T Y per group of block rows.  A CTA takes a Gram ticket only when (a) every task the group's rows depend on
-                // has been DRAWN (a critical ticket of a later column was handed out), so that it cannot starve them of CTAs,
-                // (b) the rows are factored (no waiting inside the task) and (c) the critical queue is at least m_lead block
-                // columns ahead of the chain -- or when the critical queue is empty.  A ticket claimed too early (a race at a
-                // group boundary) is HELD while the CTA goes on with critical tasks, so no CTA ever waits on an undrawn task.
-                for (;;) {
-                    const int front = df_ld_relaxed(g.ctrl + 3), drawn = df_ld_relaxed(g.ctrl + 4);
-                    const bool crit_left = df_ld_relaxed(g.ctrl) < g.total;
-                    auto runnable = [&](int tm) {
-                        int kb_, ke_;
-                        df_group_rows(tm / g.m_tiles, g.nb, g.mg, g.m_full, kb_, ke_);
-                        const int last_row = ke_ - 1;
-                        return !crit_left || (drawn > last_row && last_row + 2 <= front);
-                    };
-                    if (held_m < 0) {
-                        const int tm = df_ld_relaxed(g.ctrl + 2);
-                        if (tm < g.m_total && runnable(tm) && (!crit_left || drawn - front >= g.m_lead)) {
-                            const int got = atomicAdd(g.ctrl + 2, 1);
-                            if (got < g.m_total) held_m = got;
-                        }
-                    }
-                    if (held_m >= 0 && runnable(held_m)) {
-                        kind = 3; c = held_m / g.m_tiles; idx = held_m % g.m_tiles;
-                        int ti = 0;
-                        while ((ti + 1) * (ti + 2) / 2 <= idx) ti++;
-                        aux = idx - ti * (ti + 1) / 2;        // tile (ti, aux), aux <= ti
-                        idx = ti;
-                        held_m = -1;
-                        break;
-                    }
-                    if (crit_left) {
-                        t = atomicAdd(g.ctrl, 1);
-                        if (t < g.total) break;
-                        t = -1;
-                        continue;
-                    }
-                    if (held_m < 0 && df_ld_relaxed(g.ctrl + 2) >= g.m_total) break;      // both queues are empty
-                }
-            }
-            if (t == 0) {
-                kind = 2; idx = 0;            // chain task 0: the first diagonal block
-            } else if (t > 0 && t < g.total) {
-                // Ticket order: per block column c -- the chain tasks PLACED there, the tiles (i, c) below the sub-diagonal, the
-                // Y tiles of block row c.  Chain task d (k loop of d - 1 tile pairs: the longest task of its column) is placed
-                // d / chain_la columns AHEAD of column d - 1, so that its accumulation is done by the time W_{d-1} arrives; it
-                // then waits on a few tiles with later tickets, which the other CTAs go on drawing (at most nb / chain_la + 1
-                // CTAs can ever be in that state).  Measured at N = 4096 with 1344 right-hand sides: 2.47 -> 2.12 ms.  Pulling
-                // the near-diagonal tiles forward as well made it slower (2.14 .. 2.41 ms): they crowd out the bulk.
-                // (a CTA's tickets only grow: the scan resumes at the column of its previous ticket -- dec_c, dec_dnext, dec_base)
-                for (;;) {
-                    int nchain = 0;
-                    while (dec_dnext + nchain < g.nb) {
-                        const int d = dec_dnext + nchain;
-                        const int place = max(0, d - 1 - (g.chain_la > 0 ? d / g.chain_la : 0));
-                        if (place != dec_c) break;
-                        nchain++;
-                    }
-                    const int ntile = g.nb - dec_c - 2 > 0 ? g.nb - dec_c - 2 : 0;
-                    const int n = nchain + ntile + g.nr;
-                    if (t < dec_base + n) {
-                        const int tl = t - dec_base;
-                        c = dec_c;
-                        if (tl < nchain) { kind = 2; idx = dec_dnext + tl; }
-                        else if (tl < nchain + ntile) { kind = 0; idx = c + 2 + (tl - nchain); }
-                        else { kind = 1; idx = tl - nchain - ntile; }
-                        break;
-                    }
-                    dec_base += n; dec_c++; dec_dnext += nchain;
-                }
-                if (g.M != nullptr) atomicMax(g.ctrl + 4, c);
-            }
-            task[3] = aux;
-            task[0] = kind; task[1] = c; task[2] = idx;
-        }
+        if (tid == 0) df_next_task(g, held_m, dec_c, dec_dnext, dec_base, task);
         __syncthreads();
-        const int kind = task[0], idx = task[2];
-        if (kind < 0) {
-            if (tracing && tid == 0) {
-                unsigned long long tg;
-                asm volatile("mov.u64 %0, %%globaltimer;\n" : "=l"(tg));
-                long long* o = g.trace + 1024 * 16 + (int64_t)blockIdx.x * 8;
-                o[0] = t_wait; o[1] = t_loop; o[2] = clock64() - t_begin; o[3] = n_tasks; o[4] = (long long)tg; o[5] = smid;
-            }
+        const DfTask tk = df_task(g, task);
+        if (tk.kind < 0) {
+            if (tracing && tid == 0) df_exit_record(g, t_wait, t_loop, t_begin, n_tasks);
             return;
         }
         n_tasks++;
-        const bool rhs = kind == 1, chain = kind == 2, gram = kind == 3;
-        const bool bkn = rhs || gram;                                    // B operand stored [k][n] (rows of Y)
-        // c = block column whose diagonal inverse finishes the task; i = block row of the A operand / output tile
-        // (Gram task: task[1] = group of block rows, tile (idx, task[3]) of M)
-        const int c = chain ? idx - 1 : (gram ? 0 : task[1]);
-        const int i = rhs ? c : idx;
-        const int gi = gram ? task[1] : 0, tj = task[3];
-        int kb = 0, ke_g = 0;                                            // Gram task: block rows [kb, ke_g) of Y
-        if (gram) df_group_rows(gi, g.nb, g.mg, g.m_full, kb, ke_g);
-        const int nk = gram ? ke_g - kb : (chain ? (idx > 0 ? idx - 1 : 0) : c);      // k tiles accumulated before the epilogue
         // operands of the k loop: A = L_i,k ([m][k]) or Y_k,ti ([k][m]);  B = L_c,k ([n][k], transposed product) or Y_k,r ([k][n])
-        const double* Ag = gram ? g.Bm + (int64_t)kb * PB * g.ldb + (int64_t)idx * PB : g.K + (int64_t)i * PB * g.ld;
-        const double* Bg = gram ? g.Bm + (int64_t)kb * PB * g.ldb + (int64_t)tj * PB
-                                : (rhs ? g.Bm + (int64_t)idx * PB : g.K + (int64_t)(c > 0 ? c : 0) * PB * g.ld);
-        const int* fa = gram ? g.flagsY + (int64_t)kb * g.nr + idx : g.flagsL + (int64_t)i * g.nb;   // A tile of k tile kt ready
-        const int* fb = gram ? g.flagsY + (int64_t)kb * g.nr + tj
-                             : (rhs ? g.flagsY + idx : g.flagsL + (int64_t)(c > 0 ? c : 0) * g.nb);  // Y_k,r (stride nr) or L_c,k
-        const int fas = gram ? g.nr : 1, fbs = bkn ? g.nr : 1;
-
-        // The accumulators START at minus the tile they will be subtracted from (A_ic or B_cr; chain tasks: also A_dd), so the
-        // global reads of those tiles happen here, at the head of the task, instead of on the critical tail behind the flag.
-        // (Gram task: at plus the tile's sum over the earlier groups, once that is flagged.)
-        double* Ct = gram ? g.M + (int64_t)idx * PB * g.ldm + (int64_t)tj * PB
-                          : (rhs ? g.Bm + (int64_t)c * PB * g.ldb + (int64_t)idx * PB
-                                 : g.K + (int64_t)i * PB * g.ld + (int64_t)(c > 0 ? c : 0) * PB);
-        const int64_t ldc = gram ? g.ldm : (rhs ? g.ldb : g.ld);
-        double* Cd = g.K + (int64_t)(chain ? idx : 0) * PB * (g.ld + 1);        // diagonal tile (idx, idx) of a chain task
-        const bool has_tile = gram ? gi > 0 : !(chain && idx == 0);
-        int* const mflag = gram ? g.flagsM + (int64_t)gi * g.m_tiles + idx * (idx + 1) / 2 + tj : nullptr;
-        const int nslab = nk * (PB / DF_K);
+        const double* Ag = tk.gram ? g.Bm + (int64_t)tk.kb * PB * g.ldb + (int64_t)tk.idx * PB : g.K + (int64_t)tk.i * PB * g.ld;
+        const double* Bg = tk.gram ? g.Bm + (int64_t)tk.kb * PB * g.ldb + (int64_t)tk.tj * PB
+                                   : (tk.rhs ? g.Bm + (int64_t)tk.idx * PB : g.K + (int64_t)(tk.c > 0 ? tk.c : 0) * PB * g.ld);
         bool ok = true;
-        if (gram && gi > 0) {
+        if (tk.gram && tk.gi > 0) {                   // the tile's sum over the earlier groups must be final
             if (tracing) t_mark = clock64();
             if (warp == 0) {
-                const bool w = df_wait(mflag - g.m_tiles, g.ctrl, g.info, g.spin_limit);
+                const bool w = df_wait(df_out(g, task).flag - g.m_tiles, g.ctrl, g.info, g.spin_limit);
                 if (lane == 0) ready_s[2] = w ? 1 : 0;
             }
             __syncthreads();
             if (tracing) t_wait += clock64() - t_mark;
             if (ready_s[2] == 0) return;              // abort raised (uniform)
         }
-        double acc[2][4][2], acc2[2][4][2];
-#pragma unroll
-        for (int x = 0; x < 2; x++)
-#pragma unroll
-            for (int y = 0; y < 4; y++) {
-                const int r = wm + x * 32 + gq, cc = wn + y * 16 + tq * 2;
-                double2 v = make_double2(0.0, 0.0), d = make_double2(0.0, 0.0);
-                if (has_tile) v = *reinterpret_cast<const double2*>(Ct + (int64_t)r * ldc + cc);
-                if (chain) d = *reinterpret_cast<const double2*>(Cd + (int64_t)r * g.ld + cc);
-                acc[x][y][0] = gram ? v.x : -v.x; acc[x][y][1] = gram ? v.y : -v.y;
-                acc2[x][y][0] = -d.x; acc2[x][y][1] = -d.y;
-            }
+        DfTile f(tid);
+        f.start(g, task, tk);
 
         // k loop: DF_NSTAGE slabs in flight.  A slab that opens a new k tile may only be staged once both operand tiles are
         // flagged ready; ONE thread samples those flags for the CTA every iteration (relaxed load, then one acquire when it
@@ -1085,7 +1032,7 @@ __global__ void __launch_bounds__(DF_THREADS, 2) chol_dataflow_cpasync_kernel(Df
             const int k0 = s * DF_K;
             double* As = As0 + (s % DF_NSTAGE) * DF_STAGE;
             double* Bs = Bs0 + (s % DF_NSTAGE) * DF_STAGE;
-            if (!gram) {
+            if (!tk.gram) {
 #pragma unroll
                 for (int e = tid; e < PB * (DF_K / 2); e += DF_THREADS) {     // 64 rows x 16 chunks of 16 bytes
                     const int r = e >> 4, q = e & 15;
@@ -1098,7 +1045,7 @@ __global__ void __launch_bounds__(DF_THREADS, 2) chol_dataflow_cpasync_kernel(Df
                     cp_async16(&As[r * DF_LDT + q * 2], Ag + (int64_t)(k0 + r) * g.ldb + q * 2, true);
                 }
             }
-            if (!bkn) {
+            if (!tk.bkn) {
 #pragma unroll
                 for (int e = tid; e < PB * (DF_K / 2); e += DF_THREADS) {
                     const int r = e >> 4, q = e & 15;
@@ -1114,43 +1061,19 @@ __global__ void __launch_bounds__(DF_THREADS, 2) chol_dataflow_cpasync_kernel(Df
             cp_async_commit();
         };
         auto sample = [&](int kt) -> int {            // both operand tiles of k tile kt flagged?  (thread 0 only)
-            if (kt >= nk) return 0;
-            if (!(df_ld_relaxed(fa + (int64_t)kt * fas) & df_ld_relaxed(fb + (int64_t)kt * fbs))) return 0;
-            return df_ld_acquire(fa + (int64_t)kt * fas) & df_ld_acquire(fb + (int64_t)kt * fbs);
+            if (kt >= tk.nk) return 0;
+            if (!(df_ld_relaxed(tk.fa + (int64_t)kt * tk.fas) & df_ld_relaxed(tk.fb + (int64_t)kt * tk.fbs))) return 0;
+            return df_ld_acquire(tk.fa + (int64_t)kt * tk.fas) & df_ld_acquire(tk.fb + (int64_t)kt * tk.fbs);
         };
         // the same in two halves: the relaxed loads are ISSUED before a slab's DMMA loop and consumed after it, so their L2
         // round trip never sits between the CTA and its barrier; only a tile newly seen ready costs the acquire
         auto peek = [&](int kt) -> int {
-            return kt < nk ? (df_ld_relaxed(fa + (int64_t)kt * fas) & df_ld_relaxed(fb + (int64_t)kt * fbs)) : 0;
+            return kt < tk.nk ? (df_ld_relaxed(tk.fa + (int64_t)kt * tk.fas) & df_ld_relaxed(tk.fb + (int64_t)kt * tk.fbs)) : 0;
         };
-        auto confirm = [&](int kt) -> int { return df_ld_acquire(fa + (int64_t)kt * fas) & df_ld_acquire(fb + (int64_t)kt * fbs); };
-        auto compute = [&](int slot) {                // one 64 x 64 x 32 slab out of ring slot `slot`
-            const double* As = As0 + slot * DF_STAGE;
-            const double* Bs = Bs0 + slot * DF_STAGE;
-#pragma unroll
-            for (int kk = 0; kk < DF_K; kk += 4) {
-                double a[2], b[4];
-#pragma unroll
-                for (int x = 0; x < 2; x++)
-                    a[x] = gram ? As[(kk + tq) * DF_LDT + wm + x * 32 + gq] : As[(wm + x * 32 + gq) * DF_LDA + kk + tq];
-#pragma unroll
-                for (int y = 0; y < 4; y++)
-                    b[y] = bkn ? Bs[(kk + tq) * DF_LDT + wn + y * 16 + gq] : Bs[(wn + y * 16 + gq) * DF_LDA + kk + tq];
-#pragma unroll
-                for (int x = 0; x < 2; x++)
-#pragma unroll
-                    for (int y = 0; y < 4; y++) dmma884(acc[x][y][0], acc[x][y][1], a[x], b[y]);
-                if (chain) {                          // diagonal tile (i, i): L_ik L_ik^T out of the same A slab, lower tiles only
-#pragma unroll
-                    for (int y = 0; y < 4; y++) b[y] = As[(wn + y * 16 + gq) * DF_LDA + kk + tq];
-#pragma unroll
-                    for (int x = 0; x < 2; x++)
-#pragma unroll
-                        for (int y = 0; y < 4; y++)
-                            if (wn + y * 16 < wm + x * 32 + 8) dmma884(acc2[x][y][0], acc2[x][y][1], a[x], b[y]);
-                }
-            }
+        auto confirm = [&](int kt) -> int {
+            return df_ld_acquire(tk.fa + (int64_t)kt * tk.fas) & df_ld_acquire(tk.fb + (int64_t)kt * tk.fbs);
         };
+        const int nslab = tk.nslab;
         int paused = 0;
         const long long t_loop0 = tracing ? clock64() : 0;
         int staged = 0, ready_kt = -1;                // tiles 0 .. ready_kt are known to be ready (uniform)
@@ -1166,8 +1089,8 @@ __global__ void __launch_bounds__(DF_THREADS, 2) chol_dataflow_cpasync_kernel(Df
                 const int kt = s >> 1;
                 if (tracing) t_mark = clock64();
                 if (warp == 0) {
-                    bool w = df_wait(fa + (int64_t)kt * fas, g.ctrl, g.info, g.spin_limit);
-                    w = df_wait(fb + (int64_t)kt * fbs, g.ctrl, g.info, g.spin_limit) && w;
+                    bool w = df_wait(tk.fa + (int64_t)kt * tk.fas, g.ctrl, g.info, g.spin_limit);
+                    w = df_wait(tk.fb + (int64_t)kt * tk.fbs, g.ctrl, g.info, g.spin_limit) && w;
                     if (lane == 0) ready_s[2] = w ? 1 : 0;
                 }
                 __syncthreads();                      // also orders warp 0's acquire before everybody's tile loads
@@ -1187,49 +1110,31 @@ __global__ void __launch_bounds__(DF_THREADS, 2) chol_dataflow_cpasync_kernel(Df
             ready_kt = max(ready_kt, ready_s[s & 1]);
             while (staged < nslab && staged <= s + DF_NSTAGE - 1 && (staged >> 1) <= ready_kt) { issue(staged); staged++; }
             const int seen = (tid == 0) ? peek(ready_kt + 1) : 0;
-            compute(s % DF_NSTAGE);
+            f.slab(As0 + (s % DF_NSTAGE) * DF_STAGE, Bs0 + (s % DF_NSTAGE) * DF_STAGE, tk);
             if (tid == 0) ready_s[(s + 1) & 1] = (seen && confirm(ready_kt + 1)) ? ready_kt + 1 : ready_kt;
         }
         __syncthreads();                              // every warp is out of the last slab: shared memory is free for the epilogue
 
         // ---- epilogue ----
         if (tracing) t_loop += clock64() - t_loop0;
-        if (chain) df_stamp(g.trace, idx, 0);
-        double* Xs = df_smem;                 // [64][68]  X = C - acc   (later: the diagonal tile S)
-        double* Ws = df_smem + DF_TILE;       // [64][68]  W_cc
-        double* Ls = df_smem + 2 * DF_TILE;   // [64][68]  L_{i,c} of a chain task
-        double* Wcc = g.W + (int64_t)(c > 0 ? c : 0) * PB * (g.ldw + 1);
-        int* myflag = gram ? mflag : (rhs ? g.flagsY + (int64_t)c * g.nr + idx : g.flagsL + (int64_t)i * g.nb + (c > 0 ? c : 0));
-        if (gram) {                                   // the tile's sum over groups 0 .. gi, back in place
-#pragma unroll
-            for (int x = 0; x < 2; x++)
-#pragma unroll
-                for (int y = 0; y < 4; y++) {
-                    const int r = wm + x * 32 + gq, cc = wn + y * 16 + tq * 2;
-                    double2 v;
-                    v.x = acc[x][y][0]; v.y = acc[x][y][1];
-                    *reinterpret_cast<double2*>(Ct + (int64_t)r * ldc + cc) = v;
-                }
-        } else if (!(chain && idx == 0)) {
-#pragma unroll
-            for (int x = 0; x < 2; x++)
-#pragma unroll
-                for (int y = 0; y < 4; y++) {
-                    const int r = wm + x * 32 + gq, cc = wn + y * 16 + tq * 2;
-                    Xs[r * DF_LDT + cc] = -acc[x][y][0];              // X = C - sum (the accumulator started at -C)
-                    Xs[r * DF_LDT + cc + 1] = -acc[x][y][1];
-                    acc[x][y][0] = acc[x][y][1] = 0.0;
-                }
+        if (tk.chain) df_stamp(g.trace, tk.idx, 0);
+        const DfOut out = df_out(g, task);
+        if (tk.gram) {
+            f.store(out.Ct, out.ldc);
+        } else if (!(tk.chain && tk.idx == 0)) {
+            f.stage_x(df_smem);
             if (tracing) t_mark = clock64();
             if (warp == 0) {
-                const bool w = df_wait(g.flagsL + (int64_t)c * g.nb + c, g.ctrl, g.info, g.spin_limit);
+                const bool w = df_wait(g.flagsL + (int64_t)tk.c * g.nb + tk.c, g.ctrl, g.info, g.spin_limit);
                 if (lane == 0) ready_s[2] = w ? 1 : 0;
             }
             __syncthreads();                          // X is in shared memory, W_cc is final (warp 0 acquired its flag)
             if (tracing) t_wait += clock64() - t_mark;
             const bool okd = ready_s[2] != 0;
-            if (chain && tid == 0) df_st_relaxed(my_pause, 1);
-            if (chain) df_stamp(g.trace, idx, 1);
+            if (tk.chain && tid == 0) df_st_relaxed(my_pause, 1);
+            if (tk.chain) df_stamp(g.trace, tk.idx, 1);
+            const double* Wcc = g.W + (int64_t)tk.c * PB * (g.ldw + 1);
+            double* Ws = df_smem + DF_TILE;
 #pragma unroll
             for (int e = tid; e < PB * (PB / 2); e += DF_THREADS) {
                 const int r = e >> 5, q = e & 31;
@@ -1239,153 +1144,14 @@ __global__ void __launch_bounds__(DF_THREADS, 2) chol_dataflow_cpasync_kernel(Df
             cp_async_wait<0>();
             __syncthreads();
             if (!okd) {                               // abort raised (uniform: okd came through shared memory)
-                if (chain && tid == 0) df_st_relaxed(my_pause, 0);
+                if (tk.chain && tid == 0) df_st_relaxed(my_pause, 0);
                 return;
             }
-            if (chain) df_stamp(g.trace, idx, 2);
-#pragma unroll 4
-            for (int kk = 0; kk < PB; kk += 4) {
-                double a[2], b[4];
-                if (!rhs) {       // L_ic = X W_cc^T :  A = X [m][k],  B = W_cc [n][k] (lower triangular: k < n0 + 8)
-#pragma unroll
-                    for (int x = 0; x < 2; x++) a[x] = Xs[(wm + x * 32 + gq) * DF_LDT + kk + tq];
-#pragma unroll
-                    for (int y = 0; y < 4; y++) b[y] = (kk < wn + y * 16 + 8) ? Ws[(wn + y * 16 + gq) * DF_LDT + kk + tq] : 0.0;
-#pragma unroll
-                    for (int x = 0; x < 2; x++)
-#pragma unroll
-                        for (int y = 0; y < 4; y++)
-                            if (kk < wn + y * 16 + 8) dmma884(acc[x][y][0], acc[x][y][1], a[x], b[y]);
-                    continue;
-                } else {          // Y_cr = W_cc X :    A = W_cc [m][k],  B = X [k][n]
-#pragma unroll
-                    for (int x = 0; x < 2; x++) a[x] = Ws[(wm + x * 32 + gq) * DF_LDT + kk + tq];
-#pragma unroll
-                    for (int y = 0; y < 4; y++) b[y] = Xs[(kk + tq) * DF_LDT + wn + y * 16 + gq];
-                }
-#pragma unroll
-                for (int x = 0; x < 2; x++)
-#pragma unroll
-                    for (int y = 0; y < 4; y++) dmma884(acc[x][y][0], acc[x][y][1], a[x], b[y]);
-            }
-#pragma unroll
-            for (int x = 0; x < 2; x++)
-#pragma unroll
-                for (int y = 0; y < 4; y++) {
-                    const int r = wm + x * 32 + gq, cc = wn + y * 16 + tq * 2;
-                    double2 v;
-                    v.x = acc[x][y][0]; v.y = acc[x][y][1];
-                    *reinterpret_cast<double2*>(Ct + (int64_t)r * ldc + cc) = v;
-                    if (chain) { Ls[r * DF_LDT + cc] = v.x; Ls[r * DF_LDT + cc + 1] = v.y; }
-                }
+            if (tk.chain) df_stamp(g.trace, tk.idx, 2);
+            f.solve(df_smem, tk, out);
         }
-        if (chain) {
-            double* Wd = g.W + (int64_t)idx * PB * (g.ldw + 1);
-            df_stamp(g.trace, idx, 3);
-            if (idx > 0) {
-                __syncthreads();                      // L_{i,c} complete in shared memory; X is free
-#pragma unroll 4
-                for (int kk = 0; kk < PB; kk += 4) {  // acc2 += L_ic L_ic^T
-                    double a[2], b[4];
-#pragma unroll
-                    for (int x = 0; x < 2; x++) a[x] = Ls[(wm + x * 32 + gq) * DF_LDT + kk + tq];
-#pragma unroll
-                    for (int y = 0; y < 4; y++) b[y] = Ls[(wn + y * 16 + gq) * DF_LDT + kk + tq];
-#pragma unroll
-                    for (int x = 0; x < 2; x++)
-#pragma unroll
-                        for (int y = 0; y < 4; y++)
-                            if (wn + y * 16 < wm + x * 32 + 8) dmma884(acc2[x][y][0], acc2[x][y][1], a[x], b[y]);
-                }
-            }
-#pragma unroll
-            for (int x = 0; x < 2; x++)
-#pragma unroll
-                for (int y = 0; y < 4; y++) {
-                    const int r = wm + x * 32 + gq, cc = wn + y * 16 + tq * 2;
-                    Xs[r * DF_LDT + cc] = -acc2[x][y][0];             // S = A_dd - sum (acc2 started at -A_dd)
-                    Xs[r * DF_LDT + cc + 1] = -acc2[x][y][1];
-                }
-            if (idx > 0) {                            // publish the sub-diagonal tile before the long factor step
-                __syncthreads();                      // (release by one thread after the barrier covers the CTA's writes)
-                if (tid == 0) df_st_release(myflag, 1);
-            } else {
-                __syncthreads();
-            }
-            df_stamp(g.trace, idx, 4);
-            // Two-level factor + inverse of the 64x64 diagonal tile S (in Xs): the pair-step sweep is latency-bound per step, and a
-            // 32x32 block needs half the steps at half the work per step, so  [S11 .; S21 S22] -> L11, W11 = L11^-1 (sweep);
-            // L21 = S21 W11^T; S22 -= L21 L21^T; L22, W22 (sweep); W21 = -W22 (L21 W11), the four small products on DMMA.
-            {
-                PotrfScratch* sc = reinterpret_cast<PotrfScratch*>(Ws);       // W_cc is spent
-                constexpr int H = PB / 2, LO = DF_LDT;
-                double* L11s = Ls;                       // rows 0..31 of the Ls region: [L11 | W11]
-                double* W11s = Ls + H;
-                double* L21s = Ls + H * LO;              // rows 32..63: [L21 | T = L21 W11]
-                double* Tsm = Ls + H * LO + H;
-                double* W22s = Xs;                       // S11 is consumed by then
-                // 32x32x32 products on DMMA: warp w owns row tile w >> 1 and the column tiles 2 (w & 1), 2 (w & 1) + 1
-                const int m0 = (warp >> 1) * 8, n0 = (warp & 1) * 16;
-                auto mm32 = [&](const double* A, const double* B, bool b_nk, double (&c)[2][2]) {
-                    c[0][0] = c[0][1] = c[1][0] = c[1][1] = 0.0;
-#pragma unroll
-                    for (int kk = 0; kk < H; kk += 4) {
-                        const double av = A[(m0 + gq) * LO + kk + tq];
-#pragma unroll
-                        for (int j = 0; j < 2; j++) {
-                            const double bv = b_nk ? B[(n0 + 8 * j + gq) * LO + kk + tq] : B[(kk + tq) * LO + n0 + 8 * j + gq];
-                            dmma884(c[j][0], c[j][1], av, bv);
-                        }
-                    }
-                };
-                double c[2][2];
-                potrf_diag_body<H>(Xs, LO, Cd, g.ld, Wd, g.ldw, g.info, idx * PB, sc, L11s, W11s, LO);
-                __syncthreads();
-                mm32(Xs + H * LO, W11s, true, c);                    // L21 = S21 W11^T  (W11's upper part is stored as zeros)
-#pragma unroll
-                for (int j = 0; j < 2; j++) {
-                    const int r = m0 + gq, cc = n0 + 8 * j + tq * 2;
-                    *reinterpret_cast<double2*>(Cd + (int64_t)(H + r) * g.ld + cc) = make_double2(c[j][0], c[j][1]);
-                    L21s[r * LO + cc] = c[j][0]; L21s[r * LO + cc + 1] = c[j][1];
-                }
-                __syncthreads();
-                mm32(L21s, L21s, true, c);                           // S22 -= L21 L21^T
-#pragma unroll
-                for (int j = 0; j < 2; j++) {
-                    const int r = m0 + gq, cc = n0 + 8 * j + tq * 2;
-                    Xs[(H + r) * LO + H + cc] -= c[j][0]; Xs[(H + r) * LO + H + cc + 1] -= c[j][1];
-                }
-                __syncthreads();
-                potrf_diag_body<H>(Xs + H * LO + H, LO, Cd + (int64_t)H * g.ld + H, g.ld, Wd + (int64_t)H * g.ldw + H, g.ldw, g.info,
-                                   idx * PB + H, sc, nullptr, W22s, LO);
-                __syncthreads();
-                mm32(L21s, W11s, false, c);                          // T = L21 W11
-#pragma unroll
-                for (int j = 0; j < 2; j++) {
-                    const int r = m0 + gq, cc = n0 + 8 * j + tq * 2;
-                    Tsm[r * LO + cc] = c[j][0]; Tsm[r * LO + cc + 1] = c[j][1];
-                }
-                __syncthreads();
-                mm32(W22s, Tsm, false, c);                           // W21 = -W22 T;  W12 = 0
-#pragma unroll
-                for (int j = 0; j < 2; j++) {
-                    const int r = m0 + gq, cc = n0 + 8 * j + tq * 2;
-                    *reinterpret_cast<double2*>(Wd + (int64_t)(H + r) * g.ldw + cc) = make_double2(-c[j][0], -c[j][1]);
-                    *reinterpret_cast<double2*>(Wd + (int64_t)r * g.ldw + H + cc) = make_double2(0.0, 0.0);
-                }
-            }
-            myflag = g.flagsL + (int64_t)idx * g.nb + idx;
-            df_stamp(g.trace, idx, 5);
-        }
-        __syncthreads();
-        if (tid == 0) {
-            df_st_release(myflag, 1);                 // cumulative: covers the tile stores of every thread before the barrier
-            if (chain) {
-                df_st_relaxed(my_pause, 0);
-                if (g.M != nullptr) atomicMax(g.ctrl + 3, idx + 1);       // diagonal blocks factored (the Gram queue's gate)
-            }
-        }
-        if (chain) df_stamp(g.trace, idx, 6);
+        if (tk.chain) f.chain_tail<false>(g, tk.idx, df_smem, out);
+        df_finish<false>(g, tk, out.flag);
     }
 }
 
@@ -1466,38 +1232,6 @@ extern "C" int mfgp_build_train_cov(const double* Xt, int64_t NL, int64_t NH, co
 }
 
 namespace {
-struct SideStream {
-    cudaStream_t st = nullptr;
-    cudaEvent_t ev_potrf[2] = {nullptr, nullptr}, ev_trsm[2] = {nullptr, nullptr}, ev_begin = nullptr, ev_end = nullptr;
-    int device = -1;
-};
-SideStream g_side[16];
-
-int side_for_current_device(SideStream** out) {
-    int dev = 0;
-    MFGP_CUDA_CHECK(cudaGetDevice(&dev));
-    if (dev < 0 || dev >= 16) return MFGP_ERR_INVALID;
-    SideStream& s = g_side[dev];
-    if (!s.st) {
-        // the latency-bound panel chain runs on this stream at the HIGHEST priority, so that its small kernels are placed
-        // ahead of the pending CTAs of the bulk right-hand-side GEMMs (which stay on the caller's stream)
-        int least = 0, greatest = 0;
-        MFGP_CUDA_CHECK(cudaDeviceGetStreamPriorityRange(&least, &greatest));
-        MFGP_CUDA_CHECK(cudaStreamCreateWithPriority(&s.st, cudaStreamNonBlocking, greatest));
-        for (int i = 0; i < 2; i++) {
-            MFGP_CUDA_CHECK(cudaEventCreateWithFlags(&s.ev_potrf[i], cudaEventDisableTiming));
-            MFGP_CUDA_CHECK(cudaEventCreateWithFlags(&s.ev_trsm[i], cudaEventDisableTiming));
-        }
-        MFGP_CUDA_CHECK(cudaEventCreateWithFlags(&s.ev_begin, cudaEventDisableTiming));
-        MFGP_CUDA_CHECK(cudaEventCreateWithFlags(&s.ev_end, cudaEventDisableTiming));
-        s.device = dev;
-    }
-    *out = &s;
-    return MFGP_OK;
-}
-}  // namespace
-
-namespace {
 // A tensor map of chol_dataflow_kernel, kept while the next call passes the same buffer and shape (a step refactors the same
 // buffers, so the maps are encoded once).
 struct DfMap {
@@ -1522,14 +1256,6 @@ struct DfScratch {        // diagnostics (MFGP_DF_TRACE=1), the cached SM count 
     DfMap kmap, bmap, wmap;
 };
 DfScratch g_df[16];
-
-bool use_panel_chain() {
-    static const int v = [] {
-        const char* e = getenv("MFGP_CHOL");
-        return (e && std::strcmp(e, "chain") == 0) ? 1 : 0;
-    }();
-    return v != 0;
-}
 
 // One launch: K -> L (lower, in place), diagonal blocks of W -> inverses of L's diagonal blocks, Bm[npad, R] -> L^-1 Bm
 // (R may be 0).  The ready flags live in `scratch` (df_scratch_bytes(npad, R) bytes of caller workspace), zeroed on `st`.
@@ -1621,7 +1347,7 @@ extern "C" int mfgp_cholesky(double* K, int64_t npad, int64_t ld, double* W, int
     if (!W && !work) return MFGP_ERR_INVALID;
     if (W && ldw < npad) return MFGP_ERR_INVALID;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (W && !use_panel_chain()) {
+    if (W) {
         if (!work) return MFGP_ERR_INVALID;
         // the tile flags sit behind the part of `work` that mfgp_tri_inverse uses (see mfgp_workspace_bytes)
         int* scratch = reinterpret_cast<int*>(static_cast<char*>(work) + npad * npad * 2 + (int64_t)PB * PB * 8 + 256);
@@ -1656,73 +1382,14 @@ extern "C" int mfgp_cholesky(double* K, int64_t npad, int64_t ld, double* W, int
 
 // Cholesky of K fused with the forward substitution of R right-hand sides: on return K holds L (lower), the diagonal
 // blocks of W hold the inverses of L's diagonal blocks, and Bm[npad, R] holds L^-1 Bm; the explicit inverse
-// (mfgp_tri_inverse) and the product W B are not needed by the factored posterior.  Default: ONE launch of
-// chol_dataflow_kernel (above).  What follows is the older launch-per-panel implementation, kept behind MFGP_CHOL=chain
-// for A/B timing: the panel chain (potrf -> panel solve -> trailing update: three small dependent kernels per 64 columns)
-// runs on an internal high-priority stream, the right-hand-side work -- Y_j = W_jj B_j and B_{>j} -= L_{>j,j} Y_j, one pair
-// of tile GEMMs per panel -- on the caller's stream; Y_j waits for potrf(j), the update for the panel solve of panel j, and
-// the caller's stream waits for the internal stream before the call returns control of Bm.
-
+// (mfgp_tri_inverse) and the product W B are not needed by the factored posterior.  ONE launch of the tile-dataflow kernel
+// (chol_dataflow, above).
 extern "C" int mfgp_cholesky_solve(double* K, int64_t npad, int64_t ld, double* W, int64_t ldw, int32_t* info, double* Bm,
                                    int64_t ldb, int64_t R, void* work, int64_t work_bytes, void* stream) {
     if (!K || !W || !info || !Bm || npad <= 0 || npad % MFGP_TILE || ld < npad || ldw < npad || R <= 0 || R % GT || ldb < R)
         return MFGP_ERR_INVALID;
-    cudaStream_t caller = static_cast<cudaStream_t>(stream);
-    if (!use_panel_chain()) {
-        if (!work || work_bytes < df_scratch_bytes(npad, R)) return MFGP_ERR_INVALID;
-        return chol_dataflow(K, npad, ld, W, ldw, info, Bm, ldb, R, nullptr, 0, static_cast<int*>(work), caller);
-    }
-    SideStream* side = nullptr;
-    int rcs = side_for_current_device(&side);
-    if (rcs) return rcs;
-    cudaStream_t st = side->st;        // panel chain: internal high-priority stream
-    cudaStream_t sb = caller;          // right-hand-side GEMMs: the caller's stream
-    MFGP_CUDA_CHECK(cudaEventRecord(side->ev_begin, caller));         // Bm and K were produced on the caller's stream
-    MFGP_CUDA_CHECK(cudaStreamWaitEvent(st, side->ev_begin, 0));
-    MFGP_CUDA_CHECK(cudaMemsetAsync(info, 0, sizeof(int32_t), st));
-    const int nb = (int)(npad / PB);
-    constexpr int POTRF_SMEM = 0;   // the factor + inverse sweep lives in registers and static shared memory
-    MFGP_CUDA_CHECK(cudaFuncSetAttribute(potrf_diag_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, POTRF_SMEM));
-    for (int j = 0; j < nb; j++) {
-        double* Ajj = K + (int64_t)j * PB * (ld + 1);
-        double* Wjj = W + (int64_t)j * PB * (ldw + 1);
-        potrf_diag_kernel<<<1, 256, POTRF_SMEM, st>>>(Ajj, ld, Wjj, ldw, info, j);
-        MFGP_LAUNCH_CHECK();
-        MFGP_CUDA_CHECK(cudaEventRecord(side->ev_potrf[j & 1], st));
-        const int rem = (int)(npad - (int64_t)(j + 1) * PB);
-        double* A21 = K + (int64_t)(j + 1) * PB * ld + (int64_t)j * PB;
-        if (rem > 0) {
-            GemmArgs t{};   // L21 = A21 * inv(L11)^T, in place
-            t.A = A21; t.lda = ld; t.B = Wjj; t.ldb = ldw; t.C = A21; t.ldc = ld;
-            t.M = rem; t.N = PB; t.K = PB; t.alpha = 1.0; t.beta = 0.0; t.mode = GEMM_GENERAL;
-            int rc = launch_gemm(t, true, 1, st);
-            if (rc) return rc;
-            MFGP_CUDA_CHECK(cudaEventRecord(side->ev_trsm[j & 1], st));
-        }
-        // caller's stream: Y_j = W_jj B_j (in place: every CTA reads only the column tile it writes)
-        double* Bj = Bm + (int64_t)j * PB * ldb;
-        MFGP_CUDA_CHECK(cudaStreamWaitEvent(sb, side->ev_potrf[j & 1], 0));
-        GemmArgs y{};
-        y.A = Wjj; y.lda = ldw; y.B = Bj; y.ldb = ldb; y.C = Bj; y.ldc = ldb;
-        y.M = PB; y.N = (int)R; y.K = PB; y.alpha = 1.0; y.beta = 0.0; y.mode = GEMM_GENERAL;
-        int rc = launch_gemm(y, false, 1, sb);
-        if (rc) return rc;
-        if (rem <= 0) break;
-        MFGP_CUDA_CHECK(cudaStreamWaitEvent(sb, side->ev_trsm[j & 1], 0));
-        GemmArgs u{};       // B_{>j} -= L_{>j,j} Y_j
-        u.A = A21; u.lda = ld; u.B = Bj; u.ldb = ldb; u.C = Bm + (int64_t)(j + 1) * PB * ldb; u.ldc = ldb;
-        u.M = rem; u.N = (int)R; u.K = PB; u.alpha = -1.0; u.beta = 1.0; u.mode = GEMM_GENERAL;
-        rc = launch_gemm(u, false, 1, sb);
-        if (rc) return rc;
-        GemmArgs s2{};  // A22 -= L21 L21^T (lower tiles)
-        s2.A = A21; s2.lda = ld; s2.B = A21; s2.ldb = ld; s2.C = K + (int64_t)(j + 1) * PB * (ld + 1); s2.ldc = ld;
-        s2.M = rem; s2.N = rem; s2.K = PB; s2.alpha = -1.0; s2.beta = 1.0; s2.mode = GEMM_SYRK_LOWER;
-        rc = launch_gemm(s2, true, 1, st);
-        if (rc) return rc;
-    }
-    MFGP_CUDA_CHECK(cudaEventRecord(side->ev_end, st));               // the caller's stream resumes when the chain is done too
-    MFGP_CUDA_CHECK(cudaStreamWaitEvent(caller, side->ev_end, 0));
-    return MFGP_OK;
+    if (!work || work_bytes < df_scratch_bytes(npad, R)) return MFGP_ERR_INVALID;
+    return chol_dataflow(K, npad, ld, W, ldw, info, Bm, ldb, R, nullptr, 0, static_cast<int*>(work), static_cast<cudaStream_t>(stream));
 }
 
 // mfgp_cholesky_solve that ALSO leaves M = Y^T Y of the solved right-hand sides (R x R, row stride ldm >= R; the 64x64 tiles on
@@ -1735,17 +1402,8 @@ extern "C" int mfgp_cholesky_solve_gram(double* K, int64_t npad, int64_t ld, dou
     if (!M) return mfgp_cholesky_solve(K, npad, ld, W, ldw, info, Bm, ldb, R, work, work_bytes, stream);
     if (!K || !W || !info || !Bm || npad <= 0 || npad % MFGP_TILE || ld < npad || ldw < npad || R <= 0 || R % GT || ldb < R || ldm < R)
         return MFGP_ERR_INVALID;
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (!use_panel_chain()) {
-        if (!work || work_bytes < df_scratch_bytes(npad, R, true)) return MFGP_ERR_INVALID;
-        return chol_dataflow(K, npad, ld, W, ldw, info, Bm, ldb, R, M, ldm, static_cast<int*>(work), st);
-    }
-    int rc = mfgp_cholesky_solve(K, npad, ld, W, ldw, info, Bm, ldb, R, work, work_bytes, stream);
-    if (rc) return rc;
-    GemmArgs gm{};
-    gm.A = Bm; gm.lda = ldb; gm.B = Bm; gm.ldb = ldb; gm.C = M; gm.ldc = ldm;
-    gm.M = (int)R; gm.N = (int)R; gm.K = (int)npad; gm.alpha = 1.0; gm.beta = 0.0; gm.mode = GEMM_SYRK_LOWER;
-    return launch_syrk_ata(gm, 1, st);
+    if (!work || work_bytes < df_scratch_bytes(npad, R, true)) return MFGP_ERR_INVALID;
+    return chol_dataflow(K, npad, ld, W, ldw, info, Bm, ldb, R, M, ldm, static_cast<int*>(work), static_cast<cudaStream_t>(stream));
 }
 
 extern "C" int mfgp_tri_inverse(const double* L, int64_t npad, int64_t ld, double* W, int64_t ldw, void* work,

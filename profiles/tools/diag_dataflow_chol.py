@@ -1,5 +1,5 @@
-"""Correctness + device time of the tiled dataflow Cholesky (+ fused forward substitution) against numpy / the panel chain.
-usage: diag_dataflow_chol.py [N=4096]     (MFGP_CHOL=chain selects the old launch-per-panel chain)"""
+"""Correctness + device time of the tiled dataflow Cholesky (+ fused forward substitution) against numpy.
+usage: diag_dataflow_chol.py [N=4096] [R list, default 0,64,1792]"""
 import sys, os, ctypes
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
 import numpy as np, torch

@@ -65,7 +65,9 @@ int mfgp_build_train_cov(const double* Xt, int64_t NL, int64_t NH, const mfgp_pa
  * blocks of W (may be NULL).  `info` (device int32): 0, 1 + index of the first non-positive pivot, or -1 (internal error:
  * the tile-dataflow kernel gave up waiting for a tile).  `work`: mfgp_workspace_bytes(npad) bytes; it holds the kernel's
  * ticket counter and per-tile ready flags, so calls that use DIFFERENT work buffers may overlap freely (other streams,
- * other host threads); a work buffer must not be shared by calls that can run concurrently. */
+ * other host threads); a work buffer must not be shared by calls that can run concurrently.  A call that returns
+ * MFGP_ERR_INVALID (odd ld / ldw / ldb / ldm, a base pointer off 16-byte alignment, a short workspace, ...) enqueues
+ * nothing: info, K, W and work keep their contents.  The same holds for mfgp_cholesky_solve[_gram] (also Bm, M). */
 int mfgp_cholesky(double* K, int64_t npad, int64_t ld, double* W, int64_t ldw, int32_t* info, void* work,
                   void* stream);
 

@@ -3,6 +3,7 @@
 #include "common.cuh"
 #include "gemm_f64.cuh"
 #include <cstdlib>
+#include <mutex>
 
 namespace mfgp {
 
@@ -1253,7 +1254,8 @@ struct DfScratch {        // diagnostics (MFGP_DF_TRACE=1), the cached SM count 
     int trace_nb = 0;
     int trace_grid = 0;
     int sms = 0;
-    DfMap kmap, bmap, wmap;
+    std::mutex map_mu;    // held from the first map lookup through the launch that copies the maps into its parameters:
+    DfMap kmap, bmap, wmap;   // otherwise another host thread could re-encode them for its own buffers in between
 };
 DfScratch g_df[16];
 
@@ -1264,6 +1266,11 @@ int chol_dataflow(double* K, int64_t npad, int64_t ld, double* W, int64_t ldw, i
     int dev = 0;
     MFGP_CUDA_CHECK(cudaGetDevice(&dev));
     if (dev < 0 || dev >= 16 || !scratch) return MFGP_ERR_INVALID;
+    // TMA operands: boxes of [m][k] slabs of K / L (36 x 64), [k][n] slabs of B / Y (68 x 32) and the W_cc tile (68 x 64);
+    // rows must start 16-byte aligned.  Checked before anything is enqueued, so a rejected call leaves info and the scratch alone
+    auto aligned = [](const void* p, int64_t l) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0 && (l & 1) == 0; };
+    // (the tiles of M are read and written as double2 by the Gram tasks of both forms)
+    if (!aligned(K, ld) || !aligned(W, ldw) || (R > 0 && !aligned(Bm, ldb)) || (M && !aligned(M, ldm))) return MFGP_ERR_INVALID;
     DfScratch& sc = g_df[dev];
     const int nb = (int)(npad / PB), nr = (int)(R / PB);
     const int64_t need = df_scratch_ints(npad, R, M != nullptr);              // ctrl, per-SM pause flags, tile flags
@@ -1297,10 +1304,6 @@ int chol_dataflow(double* K, int64_t npad, int64_t ld, double* W, int64_t ldw, i
     static const int chain_la = [] { const char* e = getenv("MFGP_DF_CHAIN_LA"); return e ? atoi(e) : 5; }();
     a.chain_la = chain_la;
     a.spin_limit = 4000000000LL;      // ~2 s of SM clocks: only a bug can get there
-    // TMA operands: boxes of [m][k] slabs of K / L (36 x 64), [k][n] slabs of B / Y (68 x 32) and the W_cc tile (68 x 64);
-    // rows must start 16-byte aligned
-    auto aligned = [](const void* p, int64_t l) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0 && (l & 1) == 0; };
-    if (!aligned(K, ld) || !aligned(W, ldw) || (nr > 0 && !aligned(Bm, ldb))) return MFGP_ERR_INVALID;
     static const int occ = [] { const char* e = getenv("MFGP_DF_OCC"); return e ? atoi(e) : 2; }();
     int grid = (occ < 1 ? 1 : occ) * sc.sms;
     if (grid > a.total + a.m_total) grid = a.total + a.m_total;
@@ -1312,6 +1315,7 @@ int chol_dataflow(double* K, int64_t npad, int64_t ld, double* W, int64_t ldw, i
         MFGP_LAUNCH_CHECK();
         return MFGP_OK;
     }
+    std::lock_guard<std::mutex> lock(sc.map_mu);
     int rc = df_cached_map(sc.kmap, K, npad, npad, ld, DF_LDA, PB);
     if (!rc) rc = df_cached_map(sc.wmap, W, npad, npad, ldw, DF_LDT, PB);
     if (!rc && nr > 0) rc = df_cached_map(sc.bmap, Bm, npad, R, ldb, DF_LDT, DF_K);

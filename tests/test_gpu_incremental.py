@@ -6,6 +6,7 @@ import random
 import numpy as np
 import pytest
 import torch
+from scipy.linalg import solve_triangular
 
 from oracle import algorithms as oalg
 from oracle import gp as ogp
@@ -22,17 +23,40 @@ def _oracle(hyp, X_L, y_L, X_H, y_H, xy):
     return om, om.predict(xy)
 
 
+def _check_model(m, om, p, mu, var, mu_o, var_o):
+    """Posterior, L, z = L^-1 (y - mean) and W = L^-1 (all rows up to N = 2048, a seeded sample of 256 above) of the
+    device model against the oracle's refit."""
+    assert np.max(np.abs(var - var_o)) <= TOL * p.k0
+    assert np.max(np.abs(mu - mu_o)) <= TOL * max(1.0, np.max(np.abs(mu_o)))
+    L = m.factor()
+    assert np.max(np.abs(L - om.L)) <= 1e-10 * np.max(np.abs(om.L))
+    N = om.L.shape[0]
+    e = m.engine
+    e.ensure_factor()
+    zref = solve_triangular(om.L, ogp.centered_y(om.p, om.y_L, om.y_H)[:, 0], lower=True)
+    assert np.max(np.abs(e.z[:N].cpu().numpy() - zref)) <= TOL * max(1.0, np.max(np.abs(zref)))
+    rows = np.arange(N) if N <= 2048 else np.sort(np.random.default_rng(N).choice(N, 256, replace=False))
+    W = torch.tril(e.W[:N, :N]).cpu().numpy()[rows]
+    assert np.max(np.abs(W @ om.L - np.eye(N)[rows])) <= 1e-9
+
+
 @pytest.mark.parametrize("n,N0,adds,multi,separable", [
     (40, 30, [3, 0, 5, 1, 40, 7], True, True),         # inside one 64-block, across the 64 boundary, empty appends
     (40, 128, [64, 64, 1], True, False),               # block-aligned starts, general (non-separable) posterior path
     (48, 500, [8, 8, 70, 130], True, True),            # across the 512-row block of the posterior kernel, multi-block appends
     (40, 20, [5, 60, 9], False, True),                 # single fidelity
     (32, 120, [200], True, True),                      # one large append spanning several 64-blocks
+    (64, 2100, [1, 63, 130], True, True),              # past 2048 rows (TMA form of the fit), capacity 2112 -> 3200
+    (72, 4096, [64], True, True),                      # a c4 model taking its first samples: capacity 4096 -> 6144
 ])
 def test_append_and_incremental_posterior_match_refit(n, N0, adds, multi, separable):
+    """Past 2048 rows the split-K products of the append run 16-way, W is checked on sampled rows and the posterior on a
+    seeded subset of the grid; the grown model is then refactored from scratch through the fused path (mfgp_cholesky_solve_gram
+    on ld = capacity) and checked against the oracle as well."""
     from mfgp_coverage_b200 import simulator as sim
     from mfgp_coverage_b200._coverage import CoverageGrid
     xy = synth.grid(n)
+    sub = np.arange(xy.shape[0]) if xy.shape[0] <= 2500 else np.sort(np.random.default_rng(n).choice(xy.shape[0], 512, replace=False))
     f = synth.truth_function(xy)
     total = N0 + sum(adds)
     X_L, y_L, X_H, y_H = synth.training_set(xy, f, total + (total // 3 if multi else 0), multi=multi)
@@ -62,14 +86,8 @@ def test_append_and_incremental_posterior_match_refit(n, N0, adds, multi, separa
         nh += k
         m.predict_device(grid.xy, mu, var, grid=grid)
         launches.append(nat.lib().mfgp_launch_count() - l0)
-        om, (mu_o, var_o) = _oracle(hyp, X_L, y_L, X_H[:nh], y_H[:nh], xy)
-        assert np.max(np.abs(var.cpu().numpy() - var_o)) <= TOL * p.k0
-        assert np.max(np.abs(mu.cpu().numpy() - mu_o)) <= TOL * max(1.0, np.max(np.abs(mu_o)))
-        L = m.factor()
-        assert np.max(np.abs(L - om.L)) <= 1e-10 * np.max(np.abs(om.L))
-        N = om.L.shape[0]
-        W = torch.tril(m.engine.W[:N, :N]).cpu().numpy()
-        assert np.max(np.abs(W @ om.L - np.eye(N))) <= 1e-9
+        om, (mu_o, var_o) = _oracle(hyp, X_L, y_L, X_H[:nh], y_H[:nh], xy[sub])
+        _check_model(m, om, p, mu.cpu().numpy()[sub], var.cpu().numpy()[sub], mu_o, var_o)
     # an empty append costs nothing on the device (the reference refits even then)
     for k, nl in zip(adds, launches):
         if k == 0:
@@ -78,6 +96,14 @@ def test_append_and_incremental_posterior_match_refit(n, N0, adds, multi, separa
     mu2, var2 = m.predict(xy)
     assert np.max(np.abs(var2 - var.cpu().numpy())) <= 1e-11 * p.k0
     assert np.max(np.abs(mu2[:, 0] - mu.cpu().numpy())) <= 1e-11 * max(1.0, np.max(np.abs(mu2)))
+    if N0 > 2048:
+        e = m.engine
+        e.defer_fit = True
+        e.refactor(check=False)
+        mu3, var3 = torch.empty_like(mu), torch.empty_like(var)
+        m.predict_device(grid.xy, mu3, var3, grid=grid)
+        assert e._w_partial and e.cap > e.npad          # the fused fit ran, on leading dimension cap
+        _check_model(m, om, p, mu3.cpu().numpy()[sub], var3.cpu().numpy()[sub], mu_o, var_o)
 
 
 def test_incremental_survives_capacity_growth_and_deepcopy():

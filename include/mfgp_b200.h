@@ -134,7 +134,8 @@ int mfgp_posterior_grid_update(int64_t ny, int64_t g_lo, int64_t G, const double
  * into ONE product W B with R = ryL*rxL' + ryH*rxH' (~2.5k) columns plus per-column 64x64 Gram matrices: ~4e10 MAC
  * instead of 8.8e12 at 1 M points / N = 4096, same mean and variance to ~2e-14 k(0).  Nothing of the training covariance
  * is approximated.  Outputs are flat over the requested columns: mu / var / qred[(ix-ix0)*ny + iy].  ryL, ryH multiples
- * of 4, ryL + ryH <= 64, every order <= 64; single fidelity: rxL = ryL = 0.  `chunk_cols` columns are processed per
+ * of 4, every order <= 64 (both parts share one expansion of max(rxL, rxH) x max(ryL, ryH) terms); single fidelity:
+ * rxL = ryL = 0, NL = 0.  `chunk_cols` columns are processed per
  * pass (bounds the workspace).  No V cache: callers that need V (choi_greedy) use mfgp_posterior_grid. */
 int mfgp_posterior_grid_factored(const double* ux, int64_t nx, const double* uy, int64_t ny, int64_t ix0, int64_t ncols,
                                  const double* Xt, int64_t NL, int64_t NH, const double* W, int64_t npad, int64_t ldw,
@@ -163,7 +164,9 @@ int64_t mfgp_factored_workspace_bytes(int64_t npad, int64_t ncols, int64_t ny, i
  *   ->  mfgp_posterior_grid_factored_solved (steps 4-6; z_out receives the whitened observations).
  * Neither the explicit inverse (mfgp_tri_inverse) nor the product W B is formed; run mfgp_tri_inverse afterwards only if W
  * is needed (dense posterior, mfgp_cholesky_append, choi_greedy).  Same geometry / order arguments and the same `work`
- * buffer for prepare and solved. */
+ * buffer for prepare and solved.  ldY (row stride of Yall) is a multiple of 64 from the layout's own right-hand-side count
+ * (mfgp_factored_rhs_cols[_trunc]) up to mfgp_factored_rhs_cols(rxL, ryL, rxH, ryH); a larger one is MFGP_ERR_INVALID
+ * (mfgp_factored_gram_target: NULL), since the Gram route keeps M = Yall^T Yall at that stride inside `work`. */
 int64_t mfgp_factored_rhs_cols(int64_t rxL, int64_t ryL, int64_t rxH, int64_t ryH);
 int mfgp_factored_prepare(const double* ux, int64_t nx, const double* uy, int64_t ny, int64_t ix0, int64_t ncols,
                           const double* Xt, const double* y, int64_t NL, int64_t NH, int64_t npad, const mfgp_params* p_host,

@@ -25,7 +25,7 @@
 
 namespace mfgp {
 
-constexpr int F_LW = 64;             // padded number of y-expansion terms of both parts together (ryL + ryH <= 64)
+constexpr int F_LW = 64;             // padded number of y-expansion terms of the merged expansion (max(ryL, ryH) <= 64)
 constexpr int F_MAXR = 64;           // largest supported Chebyshev order per axis and part
 
 // Column layout of the right-hand sides: term (l, k) -- T_l(ty) T_k(tx) -- sits in column off[l] + k, k < kx[l].  Uniform: kx[l] =
@@ -210,6 +210,7 @@ struct GramArgs {
     double mean, k0;
     double* mu; double* var; double* qred;                     // flat outputs, index = col * ny + iy
     int pitch, nstage;                                         // shared-memory row pitch of a staged chunk (doubles), pipeline depth
+    int poison;                                                // 1: NaN-fill the dynamic shared memory first (MFGP_DEBUG_POISON_SMEM)
 };
 constexpr int G_MAXSTAGE = 6;
 
@@ -241,14 +242,16 @@ __device__ __forceinline__ void f_bulk_g2s(uint32_t dst, const void* src, uint32
 // Staging: chunks of 64 training rows of Y'(ix) ride an nstage-deep ring of bulk copies (completion on mbarriers).  The
 // shared row pitch is ry when ry = 4 (mod 8) -- fragment reads are then bank-conflict-free as they stand and the whole chunk is
 // ONE contiguous 64 ry x 8-byte copy -- else ry + 4 with one copy per row.  Columns [ry, WM) of a staged row alias the next row
-// (finite data, or the zero fill); they only ever meet the zero-padded entries of Uy.
+// (finite data, or the zero fill); they only ever meet the zero-padded entries of Uy -- but 0 * NaN is NaN, so the zero fill
+// reaches past the ring through the last row's column WM - 1 (g_ring_slack).
+__host__ __device__ constexpr int g_ring_slack(int wm, int pitch) { return wm - pitch > 8 ? wm - pitch : 8; }
 template <int WM>
 __global__ void __launch_bounds__(128) gram_eval_kernel(GramArgs a) {
     constexpr int NT = WM / 8, NTILES = NT * (NT + 1) / 2;
     constexpr int GP = WM + 2;
     extern __shared__ __align__(16) double gsm[];
     const int P = a.pitch, NST = a.nstage, ry = a.ryH;
-    const int ring = NST * G_ROWS * P + 8;          // + 8: the last row's aliased columns stay inside the (zeroed) buffer
+    const int ring = NST * G_ROWS * P + g_ring_slack(WM, P);     // the last row's aliased columns stay inside the (zeroed) buffer
     double* Ts = gsm;                               // [NST][G_ROWS][P]  ring of chunks of Y'(ix)
     double* Gs = gsm + ring;                        // [WM][WM + 2]   (row pitch even: 16-byte loads)
     double* hs = Gs + WM * GP;                      // [F_LW]
@@ -258,7 +261,9 @@ __global__ void __launch_bounds__(128) gram_eval_kernel(GramArgs a) {
     const int gq = lane >> 2, tq = lane & 3;
     const double* src = a.YpH + (int64_t)col * a.npad * ry;
     const uint32_t bar0 = f_smem_u32(bars);
-    for (int e = tid; e < ring; e += 128) Ts[e] = 0.0;
+    // zero ring; with `poison`, everything behind it up to the barriers reads NaN until written (a read of it shows in the output)
+    const int fill = a.poison ? ring + WM * GP + 2 * F_LW : ring;
+    for (int e = tid; e < fill; e += 128) Ts[e] = e < ring ? 0.0 : __longlong_as_double(-1ll);
     if (tid == 0) {
         for (int i = 0; i < NST; i++) f_mbar_init(bar0 + 8 * i, 1);
         asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
@@ -873,7 +878,10 @@ int f_tail(const FGeom& g, FLayout& L, const double* z, int64_t rows, double* Gs
     const int pitch = (ry0 % 8 == 4) ? ry0 : ry0 + 4;
     int nstage = (int)(73728 / (G_ROWS * pitch * 8));
     nstage = nstage < 2 ? 2 : (nstage > G_MAXSTAGE ? G_MAXSTAGE : nstage);
-    const size_t gsmem = sizeof(double) * ((size_t)nstage * G_ROWS * pitch + 8 + wm * (wm + 2) + 2 * F_LW) + 8 * G_MAXSTAGE + 64;
+    const size_t gsmem = sizeof(double) * ((size_t)nstage * G_ROWS * pitch + g_ring_slack(wm, pitch) + wm * (wm + 2) + 2 * F_LW) +
+                         8 * G_MAXSTAGE + 64;
+    const char* pe = getenv("MFGP_DEBUG_POISON_SMEM");          // read per call, as MFGP_GRAM: tests switch it inside one process
+    const int poison = pe && std::strcmp(pe, "1") == 0;
     MFGP_CUDA_CHECK(cudaFuncSetAttribute(gram_eval_kernel<40>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gsmem));
     MFGP_CUDA_CHECK(cudaFuncSetAttribute(gram_eval_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gsmem));
     int64_t hoff = 0;
@@ -909,7 +917,7 @@ int f_tail(const FGeom& g, FLayout& L, const double* z, int64_t rows, double* Gs
         ga.UxL = nullptr; ga.UxH = L.parts[0].Ux + c0 * L.parts[0].kpad;
         ga.kL = 0; ga.kH = L.parts[0].kpad;
         ga.mean = dp.mean_H; ga.k0 = dp.k0; ga.mu = mu; ga.var = var; ga.qred = qred;
-        ga.pitch = pitch; ga.nstage = nstage;
+        ga.pitch = pitch; ga.nstage = nstage; ga.poison = poison;
         if (narrow) gram_eval_kernel<40><<<(unsigned)cc, 128, gsmem, st>>>(ga);
         else gram_eval_kernel<64><<<(unsigned)cc, 128, gsmem, st>>>(ga);
         MFGP_LAUNCH_CHECK();
@@ -946,6 +954,10 @@ bool f_gram_wanted(const FGeom& g, const FLayout& L, int64_t ldY) {
     const double gram = 0.5 * npad * (double)ldY * ldY + (double)round_up(g.ncols, 64) * (f.ry * (f.ry + 1) / 2) * 64.0 * nt8 * nt8;
     return !(ov == 1 || (ov == 0 && gram >= direct));
 }
+
+// Largest row stride of the solved right-hand sides: f_tail_gram keeps M, its split-K partials and G'(ix) at offsets 0, ldY^2 and
+// (MR_MAXSPLIT + 1) ldY^2 of the step-4 region, which f_carve sizes for the uniform column count Rp.
+int64_t f_max_ldY(const FLayout& L) { return round_up((int64_t)L.parts[0].ry * L.parts[0].kpad + 1, 64); }
 
 // m_ready: M (f.Yp, row stride ldY) already holds Y^T Y (mfgp_cholesky_solve_gram wrote it)
 int f_tail_gram(const FGeom& g, FLayout& L, const double* Yall, int64_t ldY, double* Gstore, double* Hz_store, double* mu,
@@ -1027,7 +1039,7 @@ int f_tail_gram(const FGeom& g, FLayout& L, const double* Yall, int64_t ldY, dou
 
 // Factored posterior for the whole columns [ix0, ix0 + ncols) of the tensor-product grid ux[nx] x uy[ny] (x-major); outputs
 // are flat over those columns: index (ix - ix0) * ny + iy.  rx*/ry*: Chebyshev orders per axis and part (ryL, ryH multiples
-// of 4, ryL + ryH <= 64, all <= 64; rxL = ryL = 0 for a single-fidelity model) -- chosen by the caller so that the factor
+// of 4, every order <= 64; rxL = ryL = 0 for a single-fidelity model) -- chosen by the caller so that the factor
 // tables are reproduced to rounding (mfgp_coverage_b200/_engine.py: chebyshev_order).
 // kx (optional, host): truncated column layout as in mfgp_factored_prepare_trunc; needs Gstore = Hz_store = NULL and takes the Gram
 // route (MFGP_GRAM=direct falls back to the uniform layout).
@@ -1138,7 +1150,7 @@ int f_solved_impl(const FGeom& g, const int32_t* kx, const double* Yall, int64_t
     if (!f_set_trunc(L, kx)) return MFGP_ERR_INVALID;
     const int64_t npad = g.npad;
     const int64_t zoff = L.tr.cols;
-    if (ldY < round_up(zoff + 1, 64)) return MFGP_ERR_INVALID;
+    if (ldY < round_up(zoff + 1, 64) || ldY > f_max_ldY(L)) return MFGP_ERR_INVALID;
     unpack_z_kernel<<<(unsigned)((npad + 255) / 256), 256, 0, st>>>(Yall, ldY, (int)zoff, (int)npad, L.zbuf);
     MFGP_LAUNCH_CHECK();
     if (z_out) MFGP_CUDA_CHECK(cudaMemcpyAsync(z_out, L.zbuf, sizeof(double) * npad, cudaMemcpyDeviceToDevice, st));
@@ -1181,7 +1193,7 @@ extern "C" double* mfgp_factored_gram_target(int64_t nx, int64_t ny, int64_t ix0
     FGeom g{nullptr, nx, nullptr, ny, ix0, ncols, nullptr, NL, NH, npad, p_host, rxL, ryL, rxH, ryH, 0.0, 1.0, 0.0, 1.0, chunk_cols};
     FLayout L;
     f_carve(g, work, L);
-    if (!f_set_trunc(L, kx) || ldY < round_up((int64_t)L.tr.cols + 1, 64)) return nullptr;
+    if (!f_set_trunc(L, kx) || ldY < round_up((int64_t)L.tr.cols + 1, 64) || ldY > f_max_ldY(L)) return nullptr;
     return f_gram_wanted(g, L, ldY) ? L.parts[0].Yp : nullptr;
 }
 

@@ -307,6 +307,31 @@ int64_t choi_greedy(const double* Xs, int64_t G, double* Vc, int64_t ldv, int64_
                     int64_t* picks_host,
                     void* work, int64_t work_bytes, void* stream);
 
+/* Grid-sharded form of choi_greedy: every rank of a process group owns the whole-column slice [base, base + G) of the
+ * grid, its V cache Vc[cap, ldv] (rows [0,n0) valid), var[G] and qred[G].  One pick is
+ *   choi_shard_append -> choi_shard_propose -> all-gather of the send slots (caller, rank order) -> choi_shard_select;
+ * planning starts with choi_shard_begin (arg-max of the slice's var + the first propose) -> all-gather -> select.
+ * A send slot is cap + 4 doubles: [value, index bits (int64), x_j, y_j, V[0:n, j - base]] of the shard's first-index
+ * arg-max (global index; -1: no candidate, or planning is done -- every rank still joins every exchange).  The select
+ * folds the `world` slots of recv[world, cap + 4] in rank order with the tie rule of choi_greedy (a tie goes to the lowest
+ * global index), applies its loop condition (value > threshold, max_picks, cap), records the pick and stages the winner's
+ * slot for the next append.  It is deterministic, so every rank that sees the same slots holds the same state.  Nothing
+ * synchronises except choi_shard_status (BLOCKING): status_host[3] = {n, picks, done}, and, if picks_host != NULL, the
+ * picks since begin (global grid indices, up to cap of them).  `work`: choi_shard_workspace_bytes(G, cap) bytes, the
+ * same buffer and the same (G, cap) for every call between two begins.  G > 0 (every shard owns at least one column). */
+int64_t choi_shard_workspace_bytes(int64_t G, int64_t cap);
+int choi_shard_begin(const double* Xs, int64_t G, int64_t base, const double* Vc, int64_t ldv, int64_t n0, int64_t cap,
+                     const double* var, const mfgp_params* p_host, double tie_rel, double* send, void* work,
+                     int64_t work_bytes, void* stream);
+int choi_shard_append(const double* Xs, int64_t G, int64_t base, double* Vc, int64_t ldv, int64_t cap, double* var,
+                      double* qred, const mfgp_params* p_host, double tie_rel, void* work, int64_t work_bytes, void* stream);
+int choi_shard_propose(const double* Xs, int64_t G, int64_t base, const double* Vc, int64_t ldv, int64_t cap,
+                       const mfgp_params* p_host, double tie_rel, double* send, void* work, int64_t work_bytes, void* stream);
+int choi_shard_select(const double* recv, int64_t world, int64_t G, int64_t cap, const mfgp_params* p_host, double threshold,
+                      double tie_rel, int64_t max_picks, void* work, int64_t work_bytes, void* stream);
+int choi_shard_status(int64_t G, int64_t cap, const void* work, int64_t work_bytes, int64_t* status_host, int64_t* picks_host,
+                      void* stream);
+
 /* ---- batched replicate stepper: the loop bodies of simulator.py periodic :618-785, todescato :788-954, lloyd :508-616 for many
  *      independent runs of one experiment (runner.py:100, :131-147 fans the replicates out over a process pool) ----------------- */
 

@@ -128,6 +128,16 @@ SIGNATURES = {
     "choi_greedy": (c_int64, [c_void_p, c_int64, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_void_p,
                               POINTER(MfgpParams), c_double, c_double, c_int64, POINTER(c_int64), c_void_p, c_int64,
                               c_void_p]),
+    "choi_shard_workspace_bytes": (c_int64, [c_int64, c_int64]),
+    "choi_shard_begin": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_int64, c_int64, c_int64, c_void_p,
+                                 POINTER(MfgpParams), c_double, c_void_p, c_void_p, c_int64, c_void_p]),
+    "choi_shard_append": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_int64, c_int64, c_void_p, c_void_p,
+                                  POINTER(MfgpParams), c_double, c_void_p, c_int64, c_void_p]),
+    "choi_shard_propose": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_int64, c_int64, POINTER(MfgpParams), c_double,
+                                   c_void_p, c_void_p, c_int64, c_void_p]),
+    "choi_shard_select": (c_int, [c_void_p, c_int64, c_int64, c_int64, POINTER(MfgpParams), c_double, c_double, c_int64,
+                                  c_void_p, c_int64, c_void_p]),
+    "choi_shard_status": (c_int, [c_int64, c_int64, c_void_p, c_int64, POINTER(c_int64), POINTER(c_int64), c_void_p]),
     "mfgp_batch_step": (c_int, [POINTER(MfgpBatch), POINTER(MfgpParams), c_int64, c_void_p]),
     "mfgp_batch_choi_begin": (c_int, [POINTER(MfgpBatch), POINTER(MfgpParams), c_void_p]),
     "mfgp_batch_choi_plan": (c_int, [POINTER(MfgpBatch), POINTER(MfgpParams), c_double, c_int64, c_void_p]),

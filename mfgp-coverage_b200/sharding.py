@@ -9,6 +9,8 @@ Two axes, both taken from the reference's own parallelism (SURVEY.md section 2.1
     collective at all; chosen by measurement).  The coverage step all-reduces only O(agents) numbers:
     per-cell partial sums (SUM) and the per-cell (max variance, first index) pairs (all-gather + local merge, lowest
     global index wins ties exactly as np.argmax on the unsharded array).
+    Whole simulations run this way through simulator.lloyd / periodic / todescato / choi(..., group=); the Choi planner then
+    keeps only its slice's V cache on each rank (ShardPlanner, sharded_sample_points: one all-gather of a small slot per pick).
   * RUN sharding (config c5, replicate sweeps): independent simulations, `runner._map_sims` -- no collective.
 
 The merge logic is plain tensor code so that it is exercised on CPU with the gloo backend (tests/test_sharding_gloo.py).
@@ -241,39 +243,208 @@ class ShardedSim:
         self.var = torch.empty(self.grid.G, **f64)
         self._clip = [None, None]
 
-    def step(self, model, positions, centroids_t, voronoi="auto"):
-        """(loss, centroids[A,2], argmax grid indices[A], max variance[A]) -- global results, the same on every rank."""
+    def step(self, model, positions, centroids_t, voronoi="auto", weights=None):
+        """(loss, centroids[A,2], argmax grid indices[A], max variance[A]) -- global results, the same on every rank.
+        Lloyd form (model=None): the centroids are weighted by `weights` (this shard's slice, e.g. its truth) and no
+        variance is evaluated; the last two results are None."""
         from . import _coverage as cv
         from .gaussian_process import prior_variance
         bb = self.bounding_box
-        eng = model.engine
-        eng.lazy_check = eng.defer_fit = True
-        model.predict_device(self.grid.xy, self.mu, self.var, grid=self.grid)     # queued first; the host builds the cells meanwhile
+        eng = None if model is None else model.engine
+        if eng is not None:
+            eng.lazy_check = eng.defer_fit = True
+            model.predict_device(self.grid.xy, self.mu, self.var, grid=self.grid)   # queued first; the host builds the cells meanwhile
         if voronoi == "qhull":
             loss_vor, lloyd_vor = cv.BoundedVoronoi(positions, bb), cv.BoundedVoronoi(centroids_t, bb)
         else:
             loss_vor = cv.HybridVoronoi(positions, bb, reuse=self._clip[0])
             lloyd_vor = cv.HybridVoronoi(centroids_t, bb, reuse=self._clip[1])
             self._clip = [loss_vor, lloyd_vor]
-        k0 = prior_variance(model.params())
-        kw = dict(w=self.mu, var=self.var, amax_k0=k0, amax_rel=cv.AMAX_REL)
+        if eng is not None:
+            k0 = prior_variance(model.params())
+            kw = dict(w=self.mu, var=self.var, amax_k0=k0, amax_rel=cv.AMAX_REL)
+            info = eng.info.reshape(1)
+        else:
+            k0 = 0.0
+            kw = dict(w=weights)
+            info = torch.zeros(1, dtype=torch.int32, device=self.grid.device)
         extras = None
         if voronoi != "qhull" and self.grid.xy.is_cuda and len(loss_vor) and len(lloyd_vor):
             # this rank's cell areas, the clip flags and the Cholesky status ride home in the gathered results' copy
             extras = [lloyd_vor.dev_areas[:len(lloyd_vor)], loss_vor.dev_areas[:len(loss_vor)],
-                      torch.cat([eng.info.reshape(1), lloyd_vor.flag.reshape(1), loss_vor.flag.reshape(1)]).to(torch.float64)]
+                      torch.cat([info, lloyd_vor.flag.reshape(1), loss_vor.flag.reshape(1)]).to(torch.float64)]
         host = gather_results_to_host(self.grid.assign_reduce(lloyd_vor, loss_vor, **kw), self.group, k0, cv.AMAX_REL, extras)
         if extras is not None:
             ac, ap, st = host["extras"]
-            eng.raise_for_info(int(st[0]))
+            if eng is not None:
+                eng.raise_for_info(int(st[0]))
             if st[1] != 0 or st[2] != 0:
                 raise RuntimeError("cov_voronoi_clip: polygon capacity exceeded")
             lloyd_vor._areas_host, loss_vor._areas_host = ac.copy(), ap.copy()
         if host["ties"] and voronoi != "qhull":
             loss_vor.qhull(), lloyd_vor.qhull()
             host = gather_results_to_host(self.grid.assign_reduce(lloyd_vor, loss_vor, **kw), self.group, k0, cv.AMAX_REL)
-        if extras is None:
+        if extras is None and eng is not None:
             eng.check_factor(force=True)
         loss = cv.loss_from_partials(host["lossp"], loss_vor.areas())
         cent = cv.centroids_from_partials(host["cent"], lloyd_vor.areas(), bb[0], bb[1], bb[2], bb[3])
+        if eng is None:
+            return loss, cent, None, None
         return loss, cent, host["amax_idx"], host["amax_val"]
+
+
+def column_split(xy_host, world, rank):
+    """Whole-column slice of rank `rank` of the x-major tensor-product grid xy_host[G,2], split as the strong-scaling
+    benchmark splits it (columns [rank nx / world, (rank + 1) nx / world)).  Returns (lo, hi, ux, uy): the flat index range
+    [lo, hi) -- a multiple of ny, as the column-sweep coverage kernel needs -- and the grid's axes.  ValueError for a grid
+    that is not tensor-product or has fewer columns than ranks."""
+    from ._engine import detect_tensor_grid
+    tg = detect_tensor_grid(xy_host)
+    if tg is None:
+        raise ValueError("grid sharding needs an x-major tensor-product grid [[x, y] for x in ux for y in uy]")
+    ux, uy = tg
+    nx, ny = ux.size, uy.size
+    if world > nx:
+        raise ValueError(f"grid sharding needs at least one grid column per rank ({nx} columns, {world} ranks)")
+    c0, c1 = (rank * nx) // world, ((rank + 1) * nx) // world
+    return c0 * ny, c1 * ny, ux, uy
+
+
+# ---- grid-sharded Choi planner (csrc/choi.cu, choi_shard_*) ------------------------------------------------------------
+
+PLAN_BATCH = 16          # picks enqueued per host read of the planner's `done` flag, as choi_greedy does
+
+
+class ShardPlanner:
+    """Greedy-planner state of one grid shard: the V cache Vc[cap, G] of the shard's slice, q, var and the workspace.
+    One pick is append() -> propose() -> exchange of the send slots of all ranks (rank order) -> select(recv); see
+    include/mfgp_b200.h, choi_shard_*.  `grid`: the shard's CoverageGrid (base_index = global index of its first point,
+    axes = those of the whole grid).  The model is not changed."""
+
+    def __init__(self, model, grid, chunk=128):
+        from . import _native as nat
+        from ._coverage import AMAX_REL
+        eng = model.engine
+        if not eng.fitted:
+            model._refit()
+        self.nat, self.lib, self.eng, self.grid = nat, nat.lib(), eng, grid
+        self.G, self.base, self.tie_rel = grid.G, grid.base_index, AMAX_REL
+        self.n0 = eng.N
+        self.cap = self.n0 + chunk
+        f64 = dict(dtype=torch.float64, device=grid.device)
+        self.Vc = torch.empty((self.cap, self.G), **f64)
+        self.q = torch.empty(self.G, **f64)
+        _, self.var = model.predict_device(grid.xy, vcache=self.Vc if self.n0 else None, grid=grid, q_out=self.q)
+        eng.check_factor(force=True)
+        self._buffers()
+
+    def _buffers(self):
+        f64 = dict(dtype=torch.float64, device=self.grid.device)
+        self.work = torch.empty(int(self.lib.choi_shard_workspace_bytes(self.G, self.cap)) // 8 + 1, **f64)
+        self.send = torch.empty(self.cap + 4, **f64)
+
+    def _w(self):
+        return self.nat.ptr(self.work), self.work.numel() * 8, self.nat.stream_ptr()
+
+    def begin(self, n):
+        """Start planning with rows [0, n) of the cache valid: arg-max of the slice's var and the first send slot."""
+        import ctypes
+        nat = self.nat
+        nat.check(self.lib.choi_shard_begin(nat.ptr(self.grid.xy), self.G, self.base, nat.ptr(self.Vc), self.G, n, self.cap,
+                                            nat.ptr(self.var), ctypes.byref(self.eng.pstruct), ctypes.c_double(self.tie_rel),
+                                            nat.ptr(self.send), *self._w()), "choi_shard_begin")
+        return self.send
+
+    def append(self):
+        import ctypes
+        nat = self.nat
+        nat.check(self.lib.choi_shard_append(nat.ptr(self.grid.xy), self.G, self.base, nat.ptr(self.Vc), self.G, self.cap,
+                                             nat.ptr(self.var), nat.ptr(self.q), ctypes.byref(self.eng.pstruct),
+                                             ctypes.c_double(self.tie_rel), *self._w()), "choi_shard_append")
+
+    def propose(self):
+        """The shard's send slot (cap + 4 doubles) after the last append."""
+        import ctypes
+        nat = self.nat
+        nat.check(self.lib.choi_shard_propose(nat.ptr(self.grid.xy), self.G, self.base, nat.ptr(self.Vc), self.G, self.cap,
+                                              ctypes.byref(self.eng.pstruct), ctypes.c_double(self.tie_rel),
+                                              nat.ptr(self.send), *self._w()), "choi_shard_propose")
+        return self.send
+
+    def select(self, recv, threshold, max_picks):
+        """recv[world, cap + 4]: the send slots of all ranks in rank order."""
+        import ctypes
+        nat = self.nat
+        recv = recv.contiguous()
+        nat.check(self.lib.choi_shard_select(nat.ptr(recv), recv.shape[0], self.G, self.cap, ctypes.byref(self.eng.pstruct),
+                                             ctypes.c_double(float(threshold)), ctypes.c_double(self.tie_rel), int(max_picks),
+                                             *self._w()), "choi_shard_select")
+
+    def status(self, with_picks=False):
+        """(n, picks, done[, pick list]) -- synchronises the stream."""
+        import ctypes
+        st = (ctypes.c_int64 * 3)()
+        buf = (ctypes.c_int64 * self.cap)() if with_picks else None
+        self.nat.check(self.lib.choi_shard_status(self.G, self.cap, *self._w()[:2], st, buf, self.nat.stream_ptr()),
+                       "choi_shard_status")
+        out = (st[0], st[1], bool(st[2]))
+        return out + ([buf[i] for i in range(st[1])],) if with_picks else out
+
+    def grow(self, n, rows):
+        """Cache full: a larger one with rows [0, n) kept (every rank decides this from the same n)."""
+        bigger = torch.empty((self.cap + rows, self.G), dtype=torch.float64, device=self.grid.device)
+        bigger[:n].copy_(self.Vc[:n])
+        self.Vc, self.cap = bigger, self.cap + rows
+        self._buffers()
+
+
+def plan_shards(planners, exchange, threshold, chunk=128, console=False, max_picks=None):
+    """Greedy picks (global grid indices, selection order) of the shards of one grid.  `planners`: the ShardPlanners this
+    process drives (one per rank in a process group; all shards when one process emulates the group); `exchange(slots)`
+    turns their send slots into the slots of every rank, recv[world, cap + 4] in rank order (an all-gather).  Every shard
+    gets the same picks; the cache grows in lockstep since every shard sees the same n.  `max_picks`: stop after that many
+    picks even while the maximum variance is still above the threshold (None: no limit)."""
+    picks = []
+    n = planners[0].n0
+    while True:
+        room = planners[0].cap - n
+        limit = room if max_picks is None else min(room, max_picks - len(picks))
+        recv = exchange([p.begin(n) for p in planners])
+        for p in planners:
+            p.select(recv, threshold, limit)
+        while True:
+            for _ in range(PLAN_BATCH):
+                for p in planners:
+                    p.append()
+                recv = exchange([p.propose() for p in planners])
+                for p in planners:
+                    p.select(recv, threshold, limit)
+            _, _, done = planners[0].status()
+            if done:
+                break
+        n, k, _, got = planners[0].status(with_picks=True)
+        picks.extend(got)
+        print(f"Found {len(picks)} sample points so far") if console else None
+        if k < room or (max_picks is not None and len(picks) >= max_picks):
+            break
+        for p in planners:                  # V cache full: grow, resume
+            p.grow(n, chunk * 2)
+    return np.asarray(picks, dtype=np.int64)
+
+
+def sharded_sample_points(model, shard_grid, threshold, group=None, console=False):
+    """compute_sample_points on a grid sharded over `group`: this rank plans on its slice `shard_grid` (a CoverageGrid with
+    the base index and axes of a whole-column slice, see column_split), one all-gather of the shards' send slots per pick.
+    Returns (points[k, 2], global grid indices[k]), the same on every rank."""
+    world = dist.get_world_size(group)
+    planner = ShardPlanner(model, shard_grid)
+
+    def exchange(slots):
+        recv = torch.empty((world, slots[0].numel()), dtype=slots[0].dtype, device=slots[0].device)
+        dist.all_gather_into_tensor(recv, slots[0], group=group)
+        return recv
+
+    idx = plan_shards([planner], exchange, threshold, console=console)
+    axes = shard_grid.axes
+    pts = np.column_stack((axes.ux_host[idx // axes.ny], axes.uy_host[idx % axes.ny])) if idx.size else np.empty([0, 2])
+    return pts, idx

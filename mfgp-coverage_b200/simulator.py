@@ -412,6 +412,67 @@ class _Sim:
         return loss_t, centroids, argmax_xy, max_var, loss_vor, lloyd_vor
 
 
+class _ShardedSim:
+    """_Sim on a grid sharded over a process group: this rank keeps its whole-column slice of the grid resident
+    (sharding.column_split) and steps through sharding.ShardedSim, whose results are global and the same on every rank."""
+
+    def __init__(self, truth, group):
+        import torch.distributed as dist
+        from . import sharding
+        from ._engine import TensorAxes
+        self.truth_arr = np.vstack(truth.values.tolist()) if hasattr(truth, "values") else np.asarray(truth, dtype=np.float64)
+        self.x_star = self.truth_arr[:, [0, 1]]
+        self.bounding_box = np.array([np.amin(self.x_star[:, 0]), np.amax(self.x_star[:, 0]),
+                                      np.amin(self.x_star[:, 1]), np.amax(self.x_star[:, 1])])
+        if VORONOI == "clip":
+            raise ValueError("MFGP_VORONOI=clip is not available on a sharded grid: its cells fall back to Qhull at "
+                             "bisector ties (auto) or always use Qhull (qhull)")
+        self.group = group
+        lo, hi, ux, uy = sharding.column_split(self.x_star, dist.get_world_size(group), dist.get_rank(group))
+        axes = TensorAxes(ux, uy, torch.device("cuda", torch.cuda.current_device()))
+        self.state = sharding.ShardedSim(self.x_star[lo:hi], self.truth_arr[lo:hi, 2], axes, lo, self.bounding_box, group)
+        self.grid, self.mu, self.var = self.state.grid, self.state.mu, self.state.var
+        self._index_of = None
+
+    index_of = _Sim.index_of
+
+    def max_var(self):
+        """Global maximum of var (one all-reduce)."""
+        import torch.distributed as dist
+        v = self.grid.argmax(self.var)[0]
+        dist.all_reduce(v, op=dist.ReduceOp.MAX, group=self.group)
+        return float(v.item())
+
+    def step(self, model, positions, centroids_t, weights=None):
+        """_Sim.step's results; the partitions are not returned (None)."""
+        loss_t, centroids, idx, max_var = self.state.step(model, positions, centroids_t, weights=weights,
+                                                          voronoi="qhull" if VORONOI == "qhull" else "auto")
+        if model is None:
+            return loss_t, centroids, None, None, None, None
+        if np.any(idx < 0):
+            raise ValueError("zero-size array to reduction operation maximum which has no identity")   # np.amax([])
+        return loss_t, centroids, self.truth_arr[idx][:, [0, 1]], np.asarray(max_var).reshape(-1, 1), None, None
+
+
+def _sharded(group):
+    import torch.distributed as dist
+    return group is not None and dist.get_world_size(group) > 1
+
+
+def _shared_generators(rng, noise_rng, group):
+    """Generators of a sharded run: every rank must consume the same draws.  Given ones are used as passed; for missing
+    ones rank 0 draws one 64-bit seed from `random` and broadcasts it, and every rank builds random.Random(seed) /
+    np.random.default_rng(seed) from it."""
+    import torch.distributed as dist
+    if rng is not None and noise_rng is not None:
+        return rng, noise_rng
+    seed = np.array([random.getrandbits(64) if dist.get_rank(group) == 0 else 0], dtype=np.uint64)
+    t = torch.from_numpy(seed.view(np.int64)).to(torch.device("cuda", torch.cuda.current_device()))
+    dist.broadcast(t, src=dist.get_global_rank(group, 0), group=group)
+    seed = int(t.cpu().numpy().view(np.uint64)[0])
+    return (random.Random(seed) if rng is None else rng), (np.random.default_rng(seed) if noise_rng is None else noise_rng)
+
+
 def _coordinate_index(truth_arr):
     """{(x, y): row} for grids without repeated points (else None): the exact-equality lookup of simulator.py:875 in O(1)."""
     idx = {}
@@ -514,8 +575,10 @@ def _console(console, period, fidelity, loss_t, max_var_t, max_var_0, prob_explo
 #######################################################################################################################
 
 def lloyd(title, sim_num, iterations, agents, positions, truth, sigma_n, prior, hyp, console, plotter, log,
-          rng=None, noise_rng=None):
-    """reference simulator.py:508-616: Lloyd's algorithm with perfect knowledge (weights = ground truth)."""
+          rng=None, noise_rng=None, group=None):
+    """reference simulator.py:508-616: Lloyd's algorithm with perfect knowledge (weights = ground truth).
+    `group` (torch.distributed process group, all four algorithms): the grid is split into whole-column slices, one per
+    rank on its own GPU; every rank returns the same logs.  None or a group of one rank: the single-GPU path."""
     loss_log, agent_log, sample_log = [], [], [] if log else None
     fidelity = "NA"
     max_var_0 = 0
@@ -524,7 +587,7 @@ def lloyd(title, sim_num, iterations, agents, positions, truth, sigma_n, prior, 
     argmax_var_t = np.zeros((agents, 1))
     max_var_t = np.zeros((agents, 1))
     print(line_break + title + line_break)
-    sim = _Sim(truth)
+    sim = _ShardedSim(truth, group) if _sharded(group) else _Sim(truth)
     prev_positions = np.copy(positions)
     centroids_t = np.copy(positions)
     period = 0
@@ -546,17 +609,23 @@ def lloyd(title, sim_num, iterations, agents, positions, truth, sigma_n, prior, 
 
 
 def _explore_exploit(kind, title, sim_num, iterations, agents, positions, truth, sigma_n, prior, hyp, console, log,
-                     rng, noise_rng):
+                     rng, noise_rng, group=None):
     loss_log, agent_log, sample_log = [], [], [] if log else None
     fidelity = _fidelity_of(hyp)
     print(line_break + title + line_break)
+    sharded = _sharded(group)
+    if sharded:
+        rng, noise_rng = _shared_generators(rng, noise_rng, group)
     rng = random if rng is None else rng
     model, max_var_0 = _init_models(fidelity, hyp, prior)
     print("Max Initial Predictive Variance: " + str(max_var_0)) if console else None
-    sim = _Sim(truth)
+    sim = _ShardedSim(truth, group) if sharded else _Sim(truth)
     truth_arr = sim.truth_arr
     model.predict_device(sim.grid.xy, sim.mu, sim.var, grid=sim.grid)
-    max_var_t = float(sim.grid.argmax(sim.var)[0].item()) * np.ones((agents, 1))     # value only: ties irrelevant
+    if sharded:
+        max_var_t = sim.max_var() * np.ones((agents, 1))
+    else:
+        max_var_t = float(sim.grid.argmax(sim.var)[0].item()) * np.ones((agents, 1))     # value only: ties irrelevant
     prob_explore_t = todescato_prob(max_var_t, max_var_0) if kind == "todescato" else np.zeros((agents, 1))
     explore_t = np.zeros((agents, 1))
     prev_positions = np.copy(positions)
@@ -593,17 +662,17 @@ def _explore_exploit(kind, title, sim_num, iterations, agents, positions, truth,
 
 
 def periodic(title, sim_num, iterations, agents, positions, truth, sigma_n, prior, hyp, console, plotter, log,
-             rng=None, noise_rng=None):
-    """reference simulator.py:618-785."""
+             rng=None, noise_rng=None, group=None):
+    """reference simulator.py:618-785.  `group`: see lloyd."""
     return _explore_exploit("periodic", title, sim_num, iterations, agents, positions, truth, sigma_n, prior, hyp,
-                            console, log, rng, noise_rng)
+                            console, log, rng, noise_rng, group)
 
 
 def todescato(title, sim_num, iterations, agents, positions, truth, sigma_n, prior, hyp, console, plotter, log,
-              rng=None, noise_rng=None):
-    """reference simulator.py:788-954."""
+              rng=None, noise_rng=None, group=None):
+    """reference simulator.py:788-954.  `group`: see lloyd."""
     return _explore_exploit("todescato", title, sim_num, iterations, agents, positions, truth, sigma_n, prior, hyp,
-                            console, log, rng, noise_rng)
+                            console, log, rng, noise_rng, group)
 
 
 def run_batched(algo, sim_nums, iterations, agents, positions, truth, sigma_n, prior, hyp, uniforms=None, noise=None,
@@ -633,15 +702,19 @@ def run_batched(algo, sim_nums, iterations, agents, positions, truth, sigma_n, p
 
 
 def choi(title, sim_num, iterations, agents, positions, truth, sigma_n, prior, hyp, console, plotter, log,
-         rng=None, noise_rng=None):
-    """reference simulator.py:957-1161."""
+         rng=None, noise_rng=None, group=None):
+    """reference simulator.py:957-1161.  `group`: see lloyd; the planner's V cache is split with the grid
+    (sharding.sharded_sample_points), clustering and tours run on the same inputs on every rank."""
     loss_log, agent_log, sample_log = [], [], [] if log else None
     fidelity = _fidelity_of(hyp)
     print(line_break + title + line_break)
+    sharded = _sharded(group)
+    if sharded:
+        rng, noise_rng = _shared_generators(rng, noise_rng, group)
     model, max_var_0 = _init_models(fidelity, hyp, prior)
     threshold = max_var_0
     print("Max Initial Predictive Variance: " + str(max_var_0)) if console else None
-    sim = _Sim(truth)
+    sim = _ShardedSim(truth, group) if sharded else _Sim(truth)
     truth_arr, x_star, bounding_box = sim.truth_arr, sim.x_star, sim.bounding_box
     iteration = 0
     period = 0
@@ -652,7 +725,11 @@ def choi(title, sim_num, iterations, agents, positions, truth, sigma_n, prior, h
     while iteration < iterations:
         threshold = choi_threshold(threshold)
         sample_vor = voronoi_bounded(centroids_t, bounding_box)
-        sample_points = compute_sample_points(model, x_star, threshold, console)
+        if sharded:
+            from .sharding import sharded_sample_points
+            sample_points, _ = sharded_sample_points(model, sim.grid, threshold, group, console)
+        else:
+            sample_points = compute_sample_points(model, x_star, threshold, console)
         sample_clusters = compute_sample_clusters(sample_vor, sample_points)
         print("\nBegin TSP Computation") if console else None
         tsp_tours_t = compute_sample_tsp(sample_clusters)

@@ -115,6 +115,18 @@ int mfgp_posterior_grid(int64_t ny, int64_t g_lo, int64_t G, const double* TLx, 
                         int64_t ldw, const double* z, const mfgp_params* p_host, double* mu, double* var, double* qred,
                         double* Vc, int64_t ldv, void* stream);
 
+/* Joint / cross posterior covariance (SFGP.predict :121-148, MFGP.predict :401-438 return cov[G,G]; the default predict
+ * here returns its diagonal).  C[i*ldc + j] = k**(Xa_i, Xb_j) - sum_{n<N} Va[n*ldva + i] * Vb[n*ldvb + j], with V the
+ * whitened cross-covariance written by mfgp_posterior / mfgp_posterior_grid (their Vc output) and k** the prior covariance
+ * without noise or jitter, so diag(C) = k(0) - |v|^2.  Xb == NULL: B = A (Vb must be NULL and Gb == Ga), the symmetric
+ * Ga x Ga matrix (lower tiles computed and mirrored: exactly symmetric).  Otherwise the Ga x Gb cross block, which also
+ * gives block rows of a covariance too large to hold whole.  N = 0: C = k**, V is not read.  Va / Vb 16-byte aligned,
+ * ldva >= Ga, ldvb >= Gb, ldva, ldvb and ldc even (MFGP_ERR_INVALID otherwise, nothing enqueued); ldc >= Gb; nothing
+ * outside C[Ga][Gb] is written.  Deterministic: the same inputs give the same bits. */
+int mfgp_posterior_cov(const double* Xa, int64_t Ga, const double* Va, int64_t ldva,
+                       const double* Xb, int64_t Gb, const double* Vb, int64_t ldvb,
+                       int64_t N, const mfgp_params* p_host, double* C, int64_t ldc, void* stream);
+
 /* Incremental posterior after mfgp_cholesky_append: rows [row_lo, NL+NH) of V = W psi are new since mu / var / qred
  * were last computed; only their contributions are formed and ADDED (mu += v_new . z_new, var -= |v_new|^2,
  * qred += |v_new|^2).  Equal to a from-scratch mfgp_posterior up to rounding (~1e-13 k(0)); cost ~ G (N - row_lo) N

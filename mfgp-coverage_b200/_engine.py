@@ -405,6 +405,50 @@ class DeviceGP:
                   "mfgp_posterior")
         return mu, var
 
+    def posterior_cov(self, xs_a, xs_b=None, axes_a=None, g_lo_a=0, axes_b=None, g_lo_b=0, out=None):
+        """Joint posterior covariance of the points xs_a[Ga,2] (xs_b None: the symmetric Ga x Ga matrix, exactly symmetric)
+        or the cross block between xs_a and xs_b[Gb,2] -- the cov[G,G] of the reference's predict (gaussian_process.py:146,
+        :435-436), which the default `posterior` keeps only the diagonal of.  Returns device tensors (mu_a[Ga], C[Ga,Gb]).
+
+        V = W psi^T of each point set comes from `posterior(..., vcache=)` (on a tensor-product grid given by `axes_*` /
+        `g_lo_*`: the separable mfgp_posterior_grid), then mfgp_posterior_cov forms C = k** - V_A^T V_B.  mu_a comes from
+        that same dense call, so on a grid where `posterior` would take the Chebyshev-factored path it can differ from it in
+        the last bits.  C is a view with an even row pitch (the kernel's stores and TMA want 16-byte rows); `out`: a float64
+        [Ga, Gb] device tensor with unit column stride and an even row stride to write instead.
+        Raises MemoryError, before allocating anything, when V and C do not fit the free device memory; a covariance too
+        large to hold whole can be formed in block rows with the cross form, posterior_cov(xs_a[rows], xs_b=xs_a)."""
+        self.ensure_factor()
+        cross = xs_b is not None
+        Ga = int(xs_a.shape[0])
+        Gb = int(xs_b.shape[0]) if cross else Ga
+        N = self.N
+        lda, ldb = Ga + (Ga & 1), Gb + (Gb & 1)
+        if out is not None and (tuple(out.shape) != (Ga, Gb) or out.dtype != torch.float64 or out.device != self.device
+                                or (Gb > 1 and out.stride(1) != 1) or (Ga > 1 and out.stride(0) % 2)):
+            raise ValueError(f"posterior_cov: out must be a float64 [{Ga}, {Gb}] tensor on {self.device} with unit column "
+                             "stride and an even row stride")
+        need = 8 * ((0 if out is not None else Ga * ldb) + N * (lda + (ldb if cross else 0)) + 2 * (Ga + (Gb if cross else 0)))
+        free, _ = torch.cuda.mem_get_info(self.device)
+        free += torch.cuda.memory_reserved(self.device) - torch.cuda.memory_allocated(self.device)
+        if need > free:
+            raise MemoryError(f"posterior_cov: the {Ga} x {Gb} covariance and its V factors need {need / 1e9:.2f} GB, "
+                              f"{free / 1e9:.2f} GB of device memory is free; compute it in block rows with the cross form, "
+                              "posterior_cov(xs_a[rows], xs_b=xs_a)")
+        f64 = dict(dtype=torch.float64, device=self.device)
+        Va = torch.empty((N, lda), **f64)
+        mu_a, _ = self.posterior(xs_a, vcache=Va, axes=axes_a, g_lo=g_lo_a)
+        Vb = None
+        if cross:
+            Vb = torch.empty((N, ldb), **f64)
+            self.posterior(xs_b, vcache=Vb, axes=axes_b, g_lo=g_lo_b)
+        C = torch.empty((Ga, ldb), **f64)[:, :Gb] if out is None else out
+        ldc = int(C.stride(0)) if Ga > 1 else ldb
+        nat.check(nat.lib().mfgp_posterior_cov(nat.ptr(xs_a), Ga, nat.ptr(Va) if N else None, lda,
+                                               nat.ptr(xs_b) if cross else None, Gb, nat.ptr(Vb) if (cross and N) else None,
+                                               ldb if cross else 0, N, ctypes.byref(self.pstruct), nat.ptr(C), ldc,
+                                               nat.stream_ptr()), "mfgp_posterior_cov")
+        return mu_a, C
+
     # -- factored posterior on tensor-product grids (gp_factored.cu) ---------------------------------------------------------
     def _training_range(self):
         """(xmin, xmax, ymin, ymax) of the training points, tracked on the host by fit / append_hifi."""

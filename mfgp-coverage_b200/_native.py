@@ -55,6 +55,8 @@ SIGNATURES = {
     "mfgp_posterior_grid": (c_int, [c_int64, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64,
                                     c_int64, c_void_p, c_int64, c_int64, c_void_p, POINTER(MfgpParams), c_void_p,
                                     c_void_p, c_void_p, c_void_p, c_int64, c_void_p]),
+    "mfgp_posterior_cov": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_int64,
+                                   POINTER(MfgpParams), c_void_p, c_int64, c_void_p]),
     "mfgp_cholesky_append": (c_int, [c_void_p, c_int64, c_int64, c_int64, POINTER(MfgpParams), c_void_p, c_int64,
                                      c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64,
                                      c_void_p]),

@@ -79,6 +79,12 @@ __device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* map
         : "memory");
 }
 
+// register budget of a warpgroup after the role split of a warp-specialised kernel (every warp of the group executes it)
+template <int R>
+__device__ __forceinline__ void reg_alloc() { asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;\n" ::"n"(R)); }
+template <int R>
+__device__ __forceinline__ void reg_dealloc() { asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;\n" ::"n"(R)); }
+
 // 2D tensor map of a row-major FP64 matrix (rows x cols, row stride ld elements) with a box of box_cols x box_rows;
 // cuTensorMapEncodeTiled through the runtime's driver entry point query (no link-time dependency on libcuda).  The base
 // must be 16-byte aligned and ld even; boxes reaching past the matrix read zeros.
@@ -109,6 +115,25 @@ inline int make_tensor_map_2d(CUtensorMap* map, const double* base, int64_t rows
         set_last_error("cuTensorMapEncodeTiled failed", cudaErrorInvalidValue);
         return MFGP_ERR_CUDA;
     }
+    return MFGP_OK;
+}
+
+// A tensor map kept while the next call passes the same buffer and shape (a step re-uses the same buffers, so the maps are
+// encoded once).  Each cache slot serves one call site, whose box and swizzle are fixed.  The caller holds a mutex from the
+// lookup through the launch that copies the map into its parameters: otherwise another host thread could re-encode the
+// slot for its own buffers in between.
+struct CachedMap {
+    const double* base = nullptr;
+    int64_t rows = 0, cols = 0, ld = 0;
+    CUtensorMap map{};
+};
+inline int cached_tensor_map(CachedMap& m, const double* base, int64_t rows, int64_t cols, int64_t ld, int box_cols,
+                             int box_rows, CUtensorMapSwizzle swizzle) {
+    if (m.base == base && m.rows == rows && m.cols == cols && m.ld == ld) return MFGP_OK;
+    m.base = nullptr;
+    const int rc = make_tensor_map_2d(&m.map, base, rows, cols, ld, box_cols, box_rows, swizzle);
+    if (rc) return rc;
+    m.base = base; m.rows = rows; m.cols = cols; m.ld = ld;
     return MFGP_OK;
 }
 

@@ -1233,20 +1233,9 @@ extern "C" int mfgp_build_train_cov(const double* Xt, int64_t NL, int64_t NH, co
 }
 
 namespace {
-// A tensor map of chol_dataflow_kernel, kept while the next call passes the same buffer and shape (a step refactors the same
-// buffers, so the maps are encoded once).
-struct DfMap {
-    const double* base = nullptr;
-    int64_t rows = 0, cols = 0, ld = 0;
-    CUtensorMap map;
-};
-int df_cached_map(DfMap& m, const double* base, int64_t rows, int64_t cols, int64_t ld, int box_cols, int box_rows) {
-    if (m.base == base && m.rows == rows && m.cols == cols && m.ld == ld) return MFGP_OK;
-    m.base = nullptr;
-    const int rc = make_tensor_map_2d(&m.map, base, rows, cols, ld, box_cols, box_rows, CU_TENSOR_MAP_SWIZZLE_NONE);
-    if (rc) return rc;
-    m.base = base; m.rows = rows; m.cols = cols; m.ld = ld;
-    return MFGP_OK;
+// The tensor maps of chol_dataflow_kernel (a step refactors the same buffers, so they are encoded once): common.cuh
+int df_cached_map(CachedMap& m, const double* base, int64_t rows, int64_t cols, int64_t ld, int box_cols, int box_rows) {
+    return cached_tensor_map(m, base, rows, cols, ld, box_cols, box_rows, CU_TENSOR_MAP_SWIZZLE_NONE);
 }
 
 struct DfScratch {        // diagnostics (MFGP_DF_TRACE=1), the cached SM count and tensor maps; no data-path state
@@ -1255,7 +1244,7 @@ struct DfScratch {        // diagnostics (MFGP_DF_TRACE=1), the cached SM count 
     int trace_grid = 0;
     int sms = 0;
     std::mutex map_mu;    // held from the first map lookup through the launch that copies the maps into its parameters:
-    DfMap kmap, bmap, wmap;   // otherwise another host thread could re-encode them for its own buffers in between
+    CachedMap kmap, bmap, wmap;   // otherwise another host thread could re-encode them for its own buffers in between
 };
 DfScratch g_df[16];
 

@@ -61,14 +61,10 @@ struct PostArgs {
     DevParams p;
 };
 
-// ---- setmaxnreg / expect-tx primitives (PTX; mbarrier and TMA: common.cuh) --------------------------------------------
+// ---- expect-tx primitive (PTX; mbarrier, TMA and setmaxnreg: common.cuh) --------------------------------------------------
 __device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {   // adds to the tx-count, no arrival
     asm volatile("mbarrier.expect_tx.relaxed.cta.shared::cta.b64 [%0], %1;\n" ::"r"(bar), "r"(bytes) : "memory");
 }
-template <int R>
-__device__ __forceinline__ void reg_alloc() { asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;\n" ::"n"(R)); }
-template <int R>
-__device__ __forceinline__ void reg_dealloc() { asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;\n" ::"n"(R)); }
 
 // MMA row slot g (0..7) of an 8-row tile <-> row of the tile.  With the TMA 128B swizzle (16-byte chunk index XOR
 // row%8) a half-warp must touch rows whose row%8 differ in bits 1..2 to hit 16 distinct bank pairs: 0,2,4,6 | 1,3,5,7.

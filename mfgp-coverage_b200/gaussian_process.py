@@ -6,7 +6,9 @@ coverage algorithms use: construction from arrays, `hyp` assigned after construc
 
   * `predict(X_star)` returns `(mu[G,1], var[G])` -- the posterior VARIANCE VECTOR, not the G x G covariance matrix
     (gaussian_process.py:146, :435-436) of which the reference's callers only ever take `np.diag`
-    (simulator.py:301, :341, :685, :855).  A 1M-point grid would need an 8 TB matrix.
+    (simulator.py:301, :341, :685, :855).  A 1M-point grid would need an 8 TB matrix.  `predict(X_star, full_cov=True)`
+    returns the reference's `(mu[G,1], cov[G,G])`; `predict_cov_device` is its device form, with a cross form for
+    block rows of a covariance too large to hold whole.
   * `likelihood(hyp)` / `train()` (gaussian_process.py:81-119, :344-399) evaluate the negative log marginal likelihood
     AND its analytic gradient on the device (mfgp_nlml_grad) where the reference differentiates with autograd; the
     optimiser is the same scipy L-BFGS-B call.
@@ -134,8 +136,29 @@ class _GPBase:
         g_lo = grid.base_index if axes is not None else 0
         return self._dev.posterior(xs_dev, mu_out, var_out, vcache, axes=axes, g_lo=g_lo, q_out=q_out)
 
-    def predict(self, X_star):
-        """Posterior mean [G,1] and variance [G] at X_star[G,2] (host arrays in, host arrays out)."""
+    def predict_cov_device(self, xs_dev, xs2_dev=None, grid=None, grid2=None, out=None):
+        """Joint posterior covariance on device-resident points; returns device tensors (mu[G], C).  xs2_dev None: C is the
+        symmetric G x G matrix of xs_dev; otherwise the G x G2 cross block between xs_dev and xs2_dev.  `grid` / `grid2`:
+        the CoverageGrid each point set belongs to, as in predict_device.  See DeviceGP.posterior_cov."""
+        if not self._dev.fitted:
+            self._refit(check=True)
+
+        def axes_of(g):
+            axes = getattr(g, "axes", None) if (g is not None and self.use_separable) else None
+            return axes, (g.base_index if axes is not None else 0)
+
+        axes_a, g_lo_a = axes_of(grid)
+        axes_b, g_lo_b = axes_of(grid2)
+        return self._dev.posterior_cov(xs_dev, xs2_dev, axes_a=axes_a, g_lo_a=g_lo_a, axes_b=axes_b, g_lo_b=g_lo_b, out=out)
+
+    def predict(self, X_star, full_cov=False):
+        """Posterior mean [G,1] and variance [G] at X_star[G,2] (host arrays in, host arrays out).
+
+        full_cov=True: the reference's return value (gaussian_process.py:146, :435-436), mean [G,1] and the joint covariance
+        [G,G] (8 G^2 bytes on the device and on the host; MemoryError if they do not fit).  That mean comes from the dense
+        posterior call that also forms the whitened cross-covariance, so on tensor-product grids where the default call
+        takes the Chebyshev-factored path the two means can differ in the last bits; both are within 1e-9 of the exact
+        posterior."""
         from ._engine import TensorAxes, detect_tensor_grid
         # the reference's loops pass the SAME x_star array every iteration (simulator.py:892): its device copy and its
         # tensor-grid analysis are cached on the array's identity (the host array is kept alive by the cache)
@@ -154,6 +177,11 @@ class _GPBase:
             axes = None
         if not self._dev.fitted:
             self._refit(check=True)
+        if full_cov:
+            mu, C = self._dev.posterior_cov(xs_dev, axes_a=axes)
+            mu_h, C_h = mu.cpu().numpy(), C.cpu().numpy()
+            self._dev.check_factor(force=True)    # LinAlgError for a non-SPD covariance (deferred fit), as below
+            return mu_h.reshape(-1, 1), C_h
         mu, var = self._dev.posterior(xs_dev, axes=axes)
         mu_h, var_h = _to_host_pinned(mu), _to_host_pinned(var)
         self._dev.check_factor(force=True)        # synchronises; raises LinAlgError for a non-SPD covariance (deferred fit)

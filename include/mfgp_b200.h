@@ -127,6 +127,22 @@ int mfgp_posterior_cov(const double* Xa, int64_t Ga, const double* Va, int64_t l
                        const double* Xb, int64_t Gb, const double* Vb, int64_t ldvb,
                        int64_t N, const mfgp_params* p_host, double* C, int64_t ldc, void* stream);
 
+/* Factor of a joint posterior covariance for sampling.  C[npad, ld] holds mfgp_posterior_cov's symmetric output in its
+ * leading G x G block; adds `jitter` (absolute, >= 0) to its first G diagonal entries, writes the identity into rows /
+ * columns [G, npad), and factors it in place with the fused tiled Cholesky of mfgp_cholesky (lower triangle).
+ * W[npad, ldw]: receives the diagonal-block inverses (scratch for the caller); work: mfgp_workspace_bytes(npad).  info as
+ * mfgp_cholesky: 1 + index of the first non-positive pivot.  npad a multiple of MFGP_TILE with G <= npad <= 32768
+ * (npad = mfgp_npad(G)); 16-byte aligned C / W, even ld / ldw; otherwise MFGP_ERR_INVALID and nothing is enqueued. */
+int mfgp_posterior_cov_factor(double* C, int64_t G, int64_t npad, int64_t ld, double jitter, double* W, int64_t ldw,
+                              int32_t* info, void* work, void* stream);
+
+/* Joint posterior draws: F[g*ldf + s] = mu[g] + sum_{j<=g} L[g*ldl + j] * E[j*lde + s] for g < G, s < S, on DMMA.
+ * Only the lower triangle of L is read (its strict upper part may hold anything, NaN included); nothing outside
+ * F[G][S] is written.  16-byte aligned L / E / F, even ldl / lde / ldf, ldl >= G, lde >= S, ldf >= S (MFGP_ERR_INVALID
+ * otherwise, nothing enqueued).  Deterministic: the same inputs give the same bits. */
+int mfgp_posterior_sample(const double* L, int64_t G, int64_t ldl, const double* mu, const double* E, int64_t lde,
+                          int64_t S, double* F, int64_t ldf, void* stream);
+
 /* Incremental posterior after mfgp_cholesky_append: rows [row_lo, NL+NH) of V = W psi are new since mu / var / qred
  * were last computed; only their contributions are formed and ADDED (mu += v_new . z_new, var -= |v_new|^2,
  * qred += |v_new|^2).  Equal to a from-scratch mfgp_posterior up to rounding (~1e-13 k(0)); cost ~ G (N - row_lo) N

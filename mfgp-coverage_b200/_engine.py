@@ -449,6 +449,77 @@ class DeviceGP:
                                                nat.stream_ptr()), "mfgp_posterior_cov")
         return mu_a, C
 
+    SAMPLE_MAX_G = 32768      # largest point set posterior_sample factors (mfgp_posterior_cov_factor's npad limit)
+
+    def posterior_sample(self, xs, normals, axes=None, g_lo=0, jitter=None, out=None):
+        """Joint posterior draws of the latent f_H at xs[G,2]: F = mu[:, None] + L E with L = chol(C + jitter I) and
+        C = k** - V^T V, the symmetric matrix of `posterior_cov`.  `normals`: E, a float64 [G, S] device tensor of
+        standard normals.  Returns device tensors (mu[G], F[G, S]); `out`: a float64 [G, S] device tensor with unit column
+        stride and an even row stride to write F into.  `jitter` (absolute, default 1e-8 k(0)) is added to C's diagonal.
+
+        Needs C and the factor's scratch (about 16 mfgp_npad(G)^2 bytes) besides V and F: raises MemoryError before
+        allocating anything when they do not fit the free device memory, LinAlgError when C + jitter I has a non-positive
+        pivot (no retry: pass a larger `jitter`)."""
+        self.ensure_factor()
+        G = int(xs.shape[0])
+        if G > self.SAMPLE_MAX_G:
+            raise ValueError(f"posterior_sample: {G} points; at most {self.SAMPLE_MAX_G} can be drawn jointly")
+        if normals.dtype != torch.float64 or normals.device != self.device or normals.dim() != 2 or normals.shape[0] != G:
+            raise ValueError(f"posterior_sample: normals must be a float64 [{G}, S] tensor on {self.device}")
+        S = int(normals.shape[1])
+        if out is not None and (tuple(out.shape) != (G, S) or out.dtype != torch.float64 or out.device != self.device
+                                or (S > 1 and out.stride(1) != 1) or (G > 1 and out.stride(0) % 2)):
+            raise ValueError(f"posterior_sample: out must be a float64 [{G}, {S}] tensor on {self.device} with unit column "
+                             "stride and an even row stride")
+        p = self.params
+        if jitter is None:
+            jitter = 1e-8 * ((p["rho"] ** 2 * p["s_L"] + p["s_H"]) if p["multi"] else p["s_H"])
+        jitter = float(jitter)
+        if not (jitter >= 0.0 and np.isfinite(jitter)):
+            raise ValueError(f"posterior_sample: jitter must be finite and >= 0, got {jitter}")
+        if S < 1:
+            raise ValueError("posterior_sample: normals must have at least one column")
+        f64 = dict(dtype=torch.float64, device=self.device)
+        if G == 0:
+            return torch.empty(0, **f64), (torch.empty((0, S), **f64) if out is None else out)
+        lib = nat.lib()
+        npad = nat.npad(G)
+        work_bytes = int(lib.mfgp_workspace_bytes(npad))
+        lde = S + (S & 1)
+        need = (8 * (2 * npad * npad + self.N * (G + (G & 1)) + 2 * G + (0 if out is not None else G * lde))
+                + work_bytes)
+        free, _ = torch.cuda.mem_get_info(self.device)
+        free += torch.cuda.memory_reserved(self.device) - torch.cuda.memory_allocated(self.device)
+        if need > free:
+            raise MemoryError(f"posterior_sample: {G} points x {S} draws need {need / 1e9:.2f} GB (covariance, its factor's "
+                              f"scratch, V, F), {free / 1e9:.2f} GB of device memory is free")
+        C = torch.empty((npad, npad), **f64)
+        mu, _ = self.posterior_cov(xs, axes_a=axes, g_lo_a=g_lo, out=C[:G, :G])
+        W = torch.empty((npad, npad), **f64)
+        work = torch.empty(work_bytes // 8 + 1, **f64)
+        info = torch.zeros(1, dtype=torch.int32, device=self.device)
+        st = nat.stream_ptr()
+        nat.check(lib.mfgp_posterior_cov_factor(nat.ptr(C), G, npad, npad, jitter, nat.ptr(W), npad, nat.ptr(info),
+                                                nat.ptr(work), st), "mfgp_posterior_cov_factor")
+        del W, work
+        code = int(info.item())
+        if code < 0:
+            self.raise_for_info(code)
+        if code > 0:
+            raise np.linalg.LinAlgError(f"posterior_sample: the posterior covariance plus jitter {jitter:.3g} is not positive "
+                                        f"definite (pivot {code - 1}); pass a larger jitter")
+        F = torch.empty((G, lde), **f64)[:, :S] if out is None else out
+        # the kernel's TMA reads E with a 16-byte aligned base and an even row pitch; other layouts are copied once
+        if (S == 1 or normals.stride(1) == 1) and (G == 1 or normals.stride(0) % 2 == 0) and normals.data_ptr() % 16 == 0:
+            E, ld_e = normals, (int(normals.stride(0)) if G > 1 else lde)
+        else:
+            E = torch.empty((G, lde), **f64)[:, :S].copy_(normals)
+            ld_e = lde
+        ldf = int(F.stride(0)) if G > 1 else lde
+        nat.check(lib.mfgp_posterior_sample(nat.ptr(C), G, npad, nat.ptr(mu), nat.ptr(E), ld_e, S, nat.ptr(F), ldf, st),
+                  "mfgp_posterior_sample")
+        return mu, F
+
     # -- factored posterior on tensor-product grids (gp_factored.cu) ---------------------------------------------------------
     def _training_range(self):
         """(xmin, xmax, ymin, ymax) of the training points, tracked on the host by fit / append_hifi."""

@@ -57,6 +57,10 @@ SIGNATURES = {
                                     c_void_p, c_void_p, c_void_p, c_int64, c_void_p]),
     "mfgp_posterior_cov": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_int64,
                                    POINTER(MfgpParams), c_void_p, c_int64, c_void_p]),
+    "mfgp_posterior_cov_factor": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_double, c_void_p, c_int64, c_void_p,
+                                          c_void_p, c_void_p]),
+    "mfgp_posterior_sample": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_int64,
+                                      c_void_p]),
     "mfgp_cholesky_append": (c_int, [c_void_p, c_int64, c_int64, c_int64, POINTER(MfgpParams), c_void_p, c_int64,
                                      c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64,
                                      c_void_p]),

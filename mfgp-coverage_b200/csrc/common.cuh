@@ -79,6 +79,12 @@ __device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* map
         : "memory");
 }
 
+// Row g (0..7) of DMMA tile half h inside a 16-column box of a [k][n] slab loaded with 128B swizzle (gp_cov.cu,
+// gp_sample.cu).  The swizzle puts 16-byte chunk c of slab row k at chunk c ^ (k % 8); a half-warp loads rows k = 4p + t
+// (t = 0..3) of the four g it holds, so the g must spread over both halves of the chunk range for the 16 loads to hit 16
+// distinct bank pairs: g -> {0, 1, 8, 9, 2, 3, 10, 11} (+4 for h = 1).
+__device__ __forceinline__ int cv_perm(int g, int h) { return (g & 1) | (((g >> 2) & 1) << 1) | (h << 2) | (((g >> 1) & 1) << 3); }
+
 // register budget of a warpgroup after the role split of a warp-specialised kernel (every warp of the group executes it)
 template <int R>
 __device__ __forceinline__ void reg_alloc() { asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;\n" ::"n"(R)); }

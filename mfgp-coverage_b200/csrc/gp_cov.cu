@@ -45,11 +45,6 @@ struct CovArgs {
     DevParams p;
 };
 
-// Row g (0..7) of DMMA tile half h inside a 16-column box.  The 128B swizzle puts 16-byte chunk c of slab row k at chunk
-// c ^ (k % 8); a half-warp loads rows k = 4p + t (t = 0..3) of the four g it holds, so the g must spread over both halves of
-// the chunk range for the 16 loads to hit 16 distinct bank pairs: g -> {0, 1, 8, 9, 2, 3, 10, 11} (+4 for h = 1).
-__device__ __forceinline__ int cv_perm(int g, int h) { return (g & 1) | (((g >> 2) & 1) << 1) | (h << 2) | (((g >> 1) & 1) << 3); }
-
 __device__ __forceinline__ void cv_coords(double* dst, const double* X, int64_t g0, int64_t G, const DevParams& p) {
     for (int e = threadIdx.x; e < CV_BM; e += CV_THREADS) {
         int64_t g = g0 + e;

@@ -8,7 +8,8 @@ coverage algorithms use: construction from arrays, `hyp` assigned after construc
     (gaussian_process.py:146, :435-436) of which the reference's callers only ever take `np.diag`
     (simulator.py:301, :341, :685, :855).  A 1M-point grid would need an 8 TB matrix.  `predict(X_star, full_cov=True)`
     returns the reference's `(mu[G,1], cov[G,G])`; `predict_cov_device` is its device form, with a cross form for
-    block rows of a covariance too large to hold whole.
+    block rows of a covariance too large to hold whole.  `sample_posterior` (an addition) draws from that joint
+    posterior: mu + chol(cov + jitter I) E, with an absolute jitter (default 1e-8 k(0)) and mu the full_cov mean.
   * `likelihood(hyp)` / `train()` (gaussian_process.py:81-119, :344-399) evaluate the negative log marginal likelihood
     AND its analytic gradient on the device (mfgp_nlml_grad) where the reference differentiates with autograd; the
     optimiser is the same scipy L-BFGS-B call.
@@ -151,6 +152,59 @@ class _GPBase:
         axes_b, g_lo_b = axes_of(grid2)
         return self._dev.posterior_cov(xs_dev, xs2_dev, axes_a=axes_a, g_lo_a=g_lo_a, axes_b=axes_b, g_lo_b=g_lo_b, out=out)
 
+    def sample_posterior_device(self, xs_dev, normals, grid=None, jitter=None, out=None):
+        """Joint posterior draws of the latent f_H on device-resident points: F[G, S] = mu[:, None] + L normals with
+        L = chol(C + jitter I), C the joint covariance of predict_cov_device.  `normals`: a float64 [G, S] device tensor of
+        standard normals; `jitter`: absolute, added to C's diagonal (default 1e-8 k(0)); `grid` as in predict_device.
+        Returns device tensors (mu[G], F[G, S]).  See DeviceGP.posterior_sample."""
+        if not self._dev.fitted:
+            self._refit(check=True)
+        axes = getattr(grid, "axes", None) if (grid is not None and self.use_separable) else None
+        g_lo = grid.base_index if axes is not None else 0
+        return self._dev.posterior_sample(xs_dev, normals, axes=axes, g_lo=g_lo, jitter=jitter, out=out)
+
+    def sample_posterior(self, X_star, n_samples=1, rng=None, jitter=None):
+        """`n_samples` joint draws of the latent f_H at X_star[G,2] from the posterior (no observation noise): a numpy
+        array [G, n_samples], column s = mu + L E[:, s] with E = rng.standard_normal((G, n_samples)) and
+        L = chol(C + jitter I), C the covariance of predict(X_star, full_cov=True) and mu its mean.  `rng`: a numpy
+        Generator (default np.random.default_rng()), so a seeded generator replays the same draws.  `jitter`: absolute,
+        added to C's diagonal, default 1e-8 k(0) (prior_variance).  G <= 32768.  Raises LinAlgError for a non-SPD training
+        covariance or when C + jitter I is not positive definite (no retry: pass a larger jitter), MemoryError when C and
+        its factor do not fit the device."""
+        if int(n_samples) != n_samples or n_samples < 1:
+            raise ValueError(f"sample_posterior: n_samples must be a positive integer, got {n_samples}")
+        if jitter is not None and not (float(jitter) >= 0.0 and np.isfinite(float(jitter))):
+            raise ValueError(f"sample_posterior: jitter must be finite and >= 0, got {jitter}")
+        X_star = np.asarray(X_star)
+        G = X_star.reshape(-1, 2).shape[0]
+        if G > self._dev.SAMPLE_MAX_G:
+            raise ValueError(f"sample_posterior: {G} points; at most {self._dev.SAMPLE_MAX_G} can be drawn jointly")
+        rng = np.random.default_rng() if rng is None else rng
+        E = rng.standard_normal((G, int(n_samples)))
+        xs_dev, axes = self._device_points(X_star)
+        if not self._dev.fitted:
+            self._refit(check=True)
+        self._dev.check_factor(force=True)        # LinAlgError for a non-SPD training covariance (deferred fit), as predict
+        E_dev = torch.from_numpy(E).to(self._dev.device)
+        _, F = self._dev.posterior_sample(xs_dev, E_dev, axes=axes, jitter=jitter)
+        return F.cpu().numpy()
+
+    def _device_points(self, X_star):
+        """Device copy of X_star and its tensor-product axes (None if it is not such a grid, or use_separable is off)."""
+        from ._engine import TensorAxes, detect_tensor_grid
+        # the reference's loops pass the SAME x_star array every iteration (simulator.py:892): its device copy and its
+        # tensor-grid analysis are cached on the array's identity (the host array is kept alive by the cache)
+        from ._coverage import host_array_key
+        key = host_array_key(X_star)
+        if self._grid_key == key:
+            xs_dev, axes, _ = self._grid_dev
+        else:
+            xs_dev = self._upload_grid(X_star)
+            t = detect_tensor_grid(X_star)
+            axes = TensorAxes(t[0], t[1], self._dev.device) if t is not None else None
+            self._grid_key, self._grid_dev = key, (xs_dev, axes, X_star)
+        return xs_dev, (axes if self.use_separable else None)
+
     def predict(self, X_star, full_cov=False):
         """Posterior mean [G,1] and variance [G] at X_star[G,2] (host arrays in, host arrays out).
 
@@ -159,22 +213,7 @@ class _GPBase:
         posterior call that also forms the whitened cross-covariance, so on tensor-product grids where the default call
         takes the Chebyshev-factored path the two means can differ in the last bits; both are within 1e-9 of the exact
         posterior."""
-        from ._engine import TensorAxes, detect_tensor_grid
-        # the reference's loops pass the SAME x_star array every iteration (simulator.py:892): its device copy and its
-        # tensor-grid analysis are cached on the array's identity (the host array is kept alive by the cache)
-        X_star = np.asarray(X_star)
-        from ._coverage import host_array_key
-        key = host_array_key(X_star)
-        if self._grid_key == key:
-            xs_dev, axes, _ = self._grid_dev
-        else:
-            xs_dev = self._upload_grid(X_star)
-            axes = None
-            t = detect_tensor_grid(X_star)
-            axes = TensorAxes(t[0], t[1], self._dev.device) if t is not None else None
-            self._grid_key, self._grid_dev = key, (xs_dev, axes, X_star)
-        if not self.use_separable:
-            axes = None
+        xs_dev, axes = self._device_points(np.asarray(X_star))
         if not self._dev.fitted:
             self._refit(check=True)
         if full_cov:

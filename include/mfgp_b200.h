@@ -143,6 +143,42 @@ int mfgp_posterior_cov_factor(double* C, int64_t G, int64_t npad, int64_t ld, do
 int mfgp_posterior_sample(const double* L, int64_t G, int64_t ldl, const double* mu, const double* E, int64_t lde,
                           int64_t S, double* F, int64_t ldf, void* stream);
 
+/* Joint posterior draws over whole tensor-product grids by pathwise conditioning (csrc/gp_sample_grid.cu): no posterior
+ * covariance is formed or factored, so there is no G limit and no jitter.  Draw s is
+ *   F[g][s] = mean_H + f_s(x_g) + k(x_g, X) K^-1 (y - m - f_s(X) - eps_s),
+ * f_s a prior draw (per kernel part, the Chebyshev interpolant on [xlo,xhi] x [ylo,yhi] of a draw at the r_x x r_y
+ * Chebyshev nodes) and eps_s ~ N(0, diag(noise + jitter)); F = mu + A E, as mfgp_posterior_sample.  The box must cover the
+ * grid and the training points; at the orders the host picks (5e-15 convergence of the kernel's interpolant) the draws'
+ * covariance is the exact posterior covariance to ~1e-14 k(0).
+ * Normals E[d][lde], d = rxL*ryL + rxH*ryH + NL + NH rows, S columns:
+ *   rows [0, rxL*ryL)                 lofi part, term (i, j) (i-th x node root, j-th y node root) at row i*ryL + j;
+ *   rows [rxL*ryL, + rxH*ryH)         hifi part, same layout with ryH;
+ *   then one observation-noise row per training point, in the order [X_L; X_H].
+ * Single fidelity: rxL = ryL = 0 (no lofi block), NL = 0.
+ * Q matrices: Qx_P[rx_P][rx_P], Qy_P[ry_P][ry_P] row-major, Q = DCT sqrt(K_nodes) with DCT[k][j] = (k ? 2 : 1) / r
+ * cos(pi k (j + 1/2) / r) and K_nodes the unit-scale RBF of the part's length scale at the nodes mid + half cos(pi (j + 1/2) / r).
+ *
+ * mfgp_grid_sample_coef: the coefficient matrices C[S][ry][kpad] (ry = max(ryL, ryH), kpad = max(rxL, rxH) rounded up to 4)
+ * of the draws, term (l, k) = T_l(ty) T_k(tx).  W[npad, ldw] = L^-1 of the standing fit (mfgp_tri_inverse done),
+ * npad = mfgp_npad(NL + NH).  NL + NH = 0: prior draws (Xt, y, W not read).  ryL, ryH multiples of 4, every order <= 64;
+ * 16-byte aligned E / C / W / work, even lde >= S and ldw (MFGP_ERR_INVALID otherwise, nothing enqueued).
+ * work: mfgp_grid_sample_coef_workspace_bytes(NL + NH, rxL, ryL, rxH, ryH, S).
+ * mfgp_grid_sample_eval: F[((ix - ix0) * ny + iy) * ldf + s] = mean + sum_l T_l(ty_iy) sum_k T_k(tx_ix) C[s][l][k] for the
+ * whole columns [ix0, ix0 + ncols), on DMMA; nothing outside F[ncols * ny][S] is written.  rx = max(rxL, rxH), ry as above;
+ * 16-byte aligned C / F / work, even ldf >= S (MFGP_ERR_INVALID otherwise, nothing enqueued).
+ * work: mfgp_grid_sample_eval_workspace_bytes(ncols, ny, rx, ry, S).
+ * Deterministic: the same inputs give the same bits, and column slices give the same bits as the whole grid. */
+int mfgp_grid_sample_coef(const double* Xt, const double* y, int64_t NL, int64_t NH, const double* W, int64_t npad, int64_t ldw,
+                          const mfgp_params* p_host, int64_t rxL, int64_t ryL, int64_t rxH, int64_t ryH,
+                          double xlo, double xhi, double ylo, double yhi, const double* QxL, const double* QyL,
+                          const double* QxH, const double* QyH, const double* E, int64_t lde, int64_t S, double* C,
+                          void* work, int64_t work_bytes, void* stream);
+int64_t mfgp_grid_sample_coef_workspace_bytes(int64_t N, int64_t rxL, int64_t ryL, int64_t rxH, int64_t ryH, int64_t S);
+int mfgp_grid_sample_eval(const double* ux, int64_t nx, const double* uy, int64_t ny, int64_t ix0, int64_t ncols,
+                          double xlo, double xhi, double ylo, double yhi, int64_t rx, int64_t ry, const double* C, int64_t S,
+                          double mean, double* F, int64_t ldf, void* work, int64_t work_bytes, void* stream);
+int64_t mfgp_grid_sample_eval_workspace_bytes(int64_t ncols, int64_t ny, int64_t rx, int64_t ry, int64_t S);
+
 /* Incremental posterior after mfgp_cholesky_append: rows [row_lo, NL+NH) of V = W psi are new since mu / var / qred
  * were last computed; only their contributions are formed and ADDED (mu += v_new . z_new, var -= |v_new|^2,
  * qred += |v_new|^2).  Equal to a from-scratch mfgp_posterior up to rounding (~1e-13 k(0)); cost ~ G (N - row_lo) N

@@ -112,6 +112,18 @@ def detect_tensor_grid(xy):
     return ux, uy
 
 
+def node_root(length, lo, hi, r):
+    """Q[r, r] = DCT V sqrt(max(Lambda, 0)) V^T for the unit-scale RBF kernel matrix V Lambda V^T at the r Chebyshev nodes
+    mid + half cos(pi (j + 1/2) / r) of [lo, hi], DCT[k][j] = (k ? 2 : 1) / r cos(pi k (j + 1/2) / r) (cheb_coef_kernel's
+    node-values-to-coefficients map): Q xi, xi ~ N(0, I), are the Chebyshev coefficients of the interpolant of a prior draw."""
+    j = np.arange(r) + 0.5
+    node = 0.5 * (lo + hi) + 0.5 * (hi - lo) * np.cos(np.pi * j / r)
+    d = (node[:, None] - node[None, :]) / length
+    lam, V = np.linalg.eigh(np.exp(-0.5 * d * d))
+    dct = np.cos(np.pi * np.outer(np.arange(r), j) / r) * np.where(np.arange(r) == 0, 1.0, 2.0)[:, None] / r
+    return np.ascontiguousarray(dct @ ((V * np.sqrt(np.maximum(lam, 0.0))) @ V.T))
+
+
 def params_struct(p):
     """p: dict with the evaluated parameters (see gaussian_process.evaluate_hyp)."""
     return nat.MfgpParams(p["s_L"], p["l_L"], p["s_H"], p["l_H"], p["rho"], p["noise_L"], p["noise_H"],
@@ -157,6 +169,7 @@ class DeviceGP:
         self.lazy_check = False       # True: the caller reads `info` itself (cov_finish carries it home): no sync per fit
         self.epoch = 0                # bumped by every FULL refactor: standing posteriors become stale
         self._post = None             # (buffer key, epoch, N covered)
+        self._splan = None            # plan of the pathwise grid sampler (_grid_sample_plan)
 
     # -- memory -------------------------------------------------------------------------------------------------------
     def _reserve(self, n, keep_factor=False):
@@ -519,6 +532,108 @@ class DeviceGP:
         nat.check(lib.mfgp_posterior_sample(nat.ptr(C), G, npad, nat.ptr(mu), nat.ptr(E), ld_e, S, nat.ptr(F), ldf, st),
                   "mfgp_posterior_sample")
         return mu, F
+
+    # -- pathwise posterior draws on tensor-product grids (gp_sample_grid.cu) -------------------------------------------------
+    def _grid_sample_plan(self, axes):
+        """Box (the grid and the training points), Chebyshev orders and node roots Q = DCT K_nodes^(1/2) of the pathwise grid
+        sampler, uploaded; cached per grid, hyper-parameters and training hull.  ValueError when an order would exceed 64."""
+        p = self.params
+        if self.N:
+            t = self._training_range()
+            box = (min(axes.xlo, t[0]), max(axes.xhi, t[1]), min(axes.ylo, t[2]), max(axes.yhi, t[3]))
+        else:
+            box = (axes.xlo, axes.xhi, axes.ylo, axes.yhi)
+        key = (axes.uid, box, p["l_L"], p["l_H"], int(p["multi"]))
+        if self._splan is not None and self._splan["key"] == key:
+            return self._splan
+        if not (box[1] > box[0] and box[3] > box[2]):
+            raise ValueError("sample_posterior_grid: the grid and the training points span no area; use sample_posterior")
+        f64 = dict(dtype=torch.float64, device=self.device)
+        Q, orders = {}, {}
+        for part, length in ((("L", p["l_L"]), ("H", p["l_H"])) if p["multi"] else (("H", p["l_H"]),)):
+            for ax, lo, hi in (("x", box[0], box[1]), ("y", box[2], box[3])):
+                r = chebyshev_order(length, lo, hi, lo, hi)
+                if r is None:
+                    raise ValueError(f"sample_posterior_grid: length scale {length:.4g} needs more than 64 Chebyshev terms over "
+                                     f"[{lo:.4g}, {hi:.4g}]; draw at point sets of up to {self.SAMPLE_MAX_G} points with "
+                                     "sample_posterior instead")
+                orders[part + ax] = r
+                Q[part + ax] = torch.from_numpy(node_root(length, lo, hi, r)).to(**f64)
+        rxL, ryL = orders.get("Lx", 0), orders.get("Ly", 0)
+        rxH, ryH = orders["Hx"], orders["Hy"]
+        self._splan = dict(key=key, box=box, orders=(rxL, ryL, rxH, ryH), Q=Q, d0=rxL * ryL + rxH * ryH,
+                           rx=max(rxL, rxH), ry=max(ryL, ryH))
+        return self._splan
+
+    def grid_sample_dim(self, axes):
+        """Rows d of the normals that posterior_sample_grid takes for the tensor-product grid `axes` (TensorAxes)."""
+        self.ensure_factor(need_inverse=False)
+        return self._grid_sample_plan(axes)["d0"] + self.N
+
+    def posterior_sample_grid(self, axes, normals, ix0=0, ncols=None, out=None):
+        """Joint posterior draws of the latent f_H over the whole columns [ix0, ix0 + ncols) of the tensor-product grid `axes`
+        (TensorAxes), by pathwise conditioning (mfgp_grid_sample_coef, mfgp_grid_sample_eval): F = mu + A E with A A^T the
+        posterior covariance of the whole grid.  `normals`: E, a float64 [d, S] device tensor of standard normals,
+        d = grid_sample_dim(axes) (layout: include/mfgp_b200.h).  Returns F[ncols * ny, S] (row (ix - ix0) * ny + iy); `out`: a
+        float64 tensor of that shape with unit column stride and an even row stride to write it into.  The same E gives the
+        same bits for the whole grid and for any column slice of it.
+        Raises MemoryError before allocating anything when the draws and the scratch do not fit the free device memory."""
+        self.ensure_factor(need_inverse=True)
+        plan = self._grid_sample_plan(axes)
+        ix0 = int(ix0)
+        ncols = axes.nx - ix0 if ncols is None else int(ncols)
+        if not (0 <= ix0 and ncols >= 1 and ix0 + ncols <= axes.nx):
+            raise ValueError(f"posterior_sample_grid: columns [{ix0}, {ix0 + ncols}) are not inside the grid's {axes.nx}")
+        d = plan["d0"] + self.N
+        if (normals.dtype != torch.float64 or normals.device != self.device or normals.dim() != 2 or normals.shape[0] != d
+                or normals.shape[1] < 1):
+            raise ValueError(f"posterior_sample_grid: normals must be a float64 [{d}, S] tensor on {self.device}, S >= 1")
+        S = int(normals.shape[1])
+        rows = ncols * axes.ny
+        if out is not None and (tuple(out.shape) != (rows, S) or out.dtype != torch.float64 or out.device != self.device
+                                or (S > 1 and out.stride(1) != 1) or (rows > 1 and out.stride(0) % 2) or out.data_ptr() % 16):
+            raise ValueError(f"posterior_sample_grid: out must be a float64 [{rows}, {S}] tensor on {self.device} with unit "
+                             "column stride, an even row stride and a 16-byte aligned base")
+        lib = nat.lib()
+        rxL, ryL, rxH, ryH = plan["orders"]
+        rx, ry = plan["rx"], plan["ry"]
+        lde = S + (S & 1)
+        copy_e = not ((S == 1 or normals.stride(1) == 1) and (d == 1 or normals.stride(0) % 2 == 0)
+                      and normals.data_ptr() % 16 == 0)
+        cw = int(lib.mfgp_grid_sample_coef_workspace_bytes(self.N, rxL, ryL, rxH, ryH, S))
+        ew = int(lib.mfgp_grid_sample_eval_workspace_bytes(ncols, axes.ny, rx, ry, S))
+        ncoef = S * ry * (-(-rx // 4) * 4)
+        need = cw + ew + 8 * (ncoef + (rows * lde if out is None else 0) + (d * lde if copy_e else 0)) + 1024
+        free, _ = torch.cuda.mem_get_info(self.device)
+        free += torch.cuda.memory_reserved(self.device) - torch.cuda.memory_allocated(self.device)
+        if need > free:
+            raise MemoryError(f"posterior_sample_grid: {ncols} columns x {axes.ny} rows x {S} draws need {need / 1e9:.2f} GB "
+                              f"(draws, coefficients, scratch), {free / 1e9:.2f} GB of device memory is free; draw the grid in "
+                              "column slices (ix0, ncols) with the same normals")
+        f64 = dict(dtype=torch.float64, device=self.device)
+        if copy_e:
+            E, lde_e = torch.empty((d, lde), **f64), lde
+            E[:, :S].copy_(normals)
+        else:
+            E, lde_e = normals, (int(normals.stride(0)) if d > 1 else lde)
+        F = torch.empty((rows, lde), **f64)[:, :S] if out is None else out
+        ldf = int(F.stride(0)) if rows > 1 else lde
+        C = torch.empty(ncoef + 2, **f64)
+        work = torch.empty(max(cw, ew) // 8 + 2, **f64)
+        Q = plan["Q"]
+        st = nat.stream_ptr()
+        xlo, xhi, ylo, yhi = (ctypes.c_double(v) for v in plan["box"])
+        N = self.N
+        nat.check(lib.mfgp_grid_sample_coef(nat.ptr(self.Xt) if N else None, nat.ptr(self.y) if N else None, self.NL, self.NH,
+                                            nat.ptr(self.W) if N else None, self.npad if N else 0, self.cap if N else 0,
+                                            ctypes.byref(self.pstruct), rxL, ryL, rxH, ryH, xlo, xhi, ylo, yhi,
+                                            nat.ptr(Q.get("Lx")), nat.ptr(Q.get("Ly")), nat.ptr(Q["Hx"]), nat.ptr(Q["Hy"]),
+                                            nat.ptr(E), lde_e, S, nat.ptr(C), nat.ptr(work), work.numel() * 8, st),
+                  "mfgp_grid_sample_coef")
+        nat.check(lib.mfgp_grid_sample_eval(nat.ptr(axes.ux), axes.nx, nat.ptr(axes.uy), axes.ny, ix0, ncols, xlo, xhi, ylo, yhi,
+                                            rx, ry, nat.ptr(C), S, ctypes.c_double(self.params["mean_H"]), nat.ptr(F), ldf,
+                                            nat.ptr(work), work.numel() * 8, st), "mfgp_grid_sample_eval")
+        return F
 
     # -- factored posterior on tensor-product grids (gp_factored.cu) ---------------------------------------------------------
     def _training_range(self):

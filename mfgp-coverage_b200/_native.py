@@ -61,6 +61,15 @@ SIGNATURES = {
                                           c_void_p, c_void_p]),
     "mfgp_posterior_sample": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_int64,
                                       c_void_p]),
+    "mfgp_grid_sample_coef": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_int64, c_int64, POINTER(MfgpParams),
+                                      c_int64, c_int64, c_int64, c_int64, c_double, c_double, c_double, c_double, c_void_p,
+                                      c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int64,
+                                      c_void_p]),
+    "mfgp_grid_sample_coef_workspace_bytes": (c_int64, [c_int64, c_int64, c_int64, c_int64, c_int64, c_int64]),
+    "mfgp_grid_sample_eval": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_int64, c_int64, c_double, c_double, c_double,
+                                      c_double, c_int64, c_int64, c_void_p, c_int64, c_double, c_void_p, c_int64, c_void_p,
+                                      c_int64, c_void_p]),
+    "mfgp_grid_sample_eval_workspace_bytes": (c_int64, [c_int64, c_int64, c_int64, c_int64, c_int64]),
     "mfgp_cholesky_append": (c_int, [c_void_p, c_int64, c_int64, c_int64, POINTER(MfgpParams), c_void_p, c_int64,
                                      c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64,
                                      c_void_p]),

@@ -14,7 +14,8 @@ enum GemmMode : int {
     GEMM_A_LOWER = 2,      // A[M,K=M] lower triangular: k < m0 + 64
     GEMM_B_LOWER = 3,      // B[K=N,N] (not transposed) lower triangular: k >= n0
     GEMM_BT_LOWER = 4,     // B[N,K=N] (transposed operand) lower triangular: k < n0 + 64
-    GEMM_SYRK_LOWER_AUPPER = 5   // C = A A^T lower tiles with A[M,K=M] UPPER triangular: k >= m0 (>= n0)
+    GEMM_SYRK_LOWER_AUPPER = 5,  // C = A A^T lower tiles with A[M,K=M] UPPER triangular: k >= m0 (>= n0)
+    GEMM_AT_LOWER = 6            // A_TRANS operand given as a lower triangular [K=M][M] matrix (op(A) upper): k >= m0
 };
 
 struct GemmArgs {
@@ -54,7 +55,7 @@ __global__ void __launch_bounds__(128) gemm_f64_kernel(GemmArgs g) {
     if (g.mode == GEMM_A_LOWER) kend = min(g.K, m0 + GT);
     if (g.mode == GEMM_B_LOWER) kbeg = n0;
     if (g.mode == GEMM_BT_LOWER) kend = min(g.K, n0 + GT);
-    if (g.mode == GEMM_SYRK_LOWER_AUPPER) kbeg = m0;
+    if (g.mode == GEMM_SYRK_LOWER_AUPPER || g.mode == GEMM_AT_LOWER) kbeg = m0;
     if (splitk) {
         kbeg = max(kbeg, (int)blockIdx.z * g.kchunk);
         kend = min(kend, ((int)blockIdx.z + 1) * g.kchunk);
@@ -160,6 +161,15 @@ static __global__ void splitk_reduce_kernel(const double* __restrict__ part, int
 inline int launch_syrk_ata(const GemmArgs& g, int nsplit, cudaStream_t st) {
     if (g.M <= 0 || g.N <= 0 || nsplit <= 0) return MFGP_OK;
     dim3 grid((g.N + GT - 1) / GT, g.M / GT, nsplit);
+    gemm_f64_kernel<false, true><<<grid, 128, 0, st>>>(g);
+    MFGP_LAUNCH_CHECK();
+    return MFGP_OK;
+}
+
+// C[M,N] = alpha * A^T * B + beta * C for A[K,M] and B[K,N] row-major (modes GEMM_GENERAL, GEMM_AT_LOWER)
+inline int launch_gemm_at(const GemmArgs& g, cudaStream_t st) {
+    if (g.M <= 0 || g.N <= 0) return MFGP_OK;
+    dim3 grid((g.N + GT - 1) / GT, g.M / GT, 1);
     gemm_f64_kernel<false, true><<<grid, 128, 0, st>>>(g);
     MFGP_LAUNCH_CHECK();
     return MFGP_OK;

@@ -10,6 +10,8 @@ coverage algorithms use: construction from arrays, `hyp` assigned after construc
     returns the reference's `(mu[G,1], cov[G,G])`; `predict_cov_device` is its device form, with a cross form for
     block rows of a covariance too large to hold whole.  `sample_posterior` (an addition) draws from that joint
     posterior: mu + chol(cov + jitter I) E, with an absolute jitter (default 1e-8 k(0)) and mu the full_cov mean.
+    `sample_posterior_grid` draws over whole tensor-product grids of any size by pathwise conditioning, without a
+    covariance or a jitter.
   * `likelihood(hyp)` / `train()` (gaussian_process.py:81-119, :344-399) evaluate the negative log marginal likelihood
     AND its analytic gradient on the device (mfgp_nlml_grad) where the reference differentiates with autograd; the
     optimiser is the same scipy L-BFGS-B call.
@@ -187,6 +189,57 @@ class _GPBase:
         self._dev.check_factor(force=True)        # LinAlgError for a non-SPD training covariance (deferred fit), as predict
         E_dev = torch.from_numpy(E).to(self._dev.device)
         _, F = self._dev.posterior_sample(xs_dev, E_dev, axes=axes, jitter=jitter)
+        return F.cpu().numpy()
+
+    @staticmethod
+    def _grid_axes(grid):
+        from ._engine import TensorAxes
+        axes = grid if isinstance(grid, TensorAxes) else getattr(grid, "axes", None)
+        if axes is None or getattr(grid, "base_index", 0):
+            raise ValueError("sample_posterior_grid: the points are not a whole x-major tensor-product grid "
+                             "[[x, y] for x in ux for y in uy]; use sample_posterior for point sets")
+        return axes
+
+    def grid_sample_dim(self, grid):
+        """Rows d of the normals sample_posterior_grid_device takes for `grid` (a CoverageGrid of a whole tensor-product grid,
+        or its TensorAxes)."""
+        if not self._dev.fitted:
+            self._refit(check=True)
+        return self._dev.grid_sample_dim(self._grid_axes(grid))
+
+    def sample_posterior_grid_device(self, grid, normals, ix0=0, ncols=None, out=None):
+        """Joint posterior draws of the latent f_H over a whole tensor-product grid, or its columns [ix0, ix0 + ncols), by
+        pathwise conditioning: F = mu + A E with A A^T the posterior covariance, no jitter and no limit on the grid's size.
+        `grid`: a CoverageGrid of the whole grid (or its TensorAxes); `normals`: a float64 [grid_sample_dim(grid), S] device
+        tensor of standard normals.  Returns F[ncols * ny, S] on the device.  See DeviceGP.posterior_sample_grid."""
+        if not self._dev.fitted:
+            self._refit(check=True)
+        return self._dev.posterior_sample_grid(self._grid_axes(grid), normals, ix0=ix0, ncols=ncols, out=out)
+
+    def sample_posterior_grid(self, X_star, n_samples=1, rng=None):
+        """`n_samples` joint draws of the latent f_H over the tensor-product grid X_star[G,2] (x-major,
+        `[[x, y] for x in ux for y in uy]`): a numpy array [G, n_samples], F = mu + A E with E = rng.standard_normal((d,
+        n_samples)), d = grid_sample_dim, and A A^T the posterior covariance of predict(X_star, full_cov=True).  Pathwise
+        conditioning on a prior draw at Chebyshev nodes: unlike sample_posterior, no G x G covariance is formed, so whole 1M-point
+        grids can be drawn, and no jitter is added.  `rng`: a numpy Generator (default np.random.default_rng()).  Raises
+        ValueError when X_star is not such a grid or the length scales are too short for 64 Chebyshev terms over the grid and the
+        training points (sample_posterior covers both), LinAlgError for a non-SPD training covariance, MemoryError when the
+        draws do not fit the device."""
+        if int(n_samples) != n_samples or n_samples < 1:
+            raise ValueError(f"sample_posterior_grid: n_samples must be a positive integer, got {n_samples}")
+        X_star = np.asarray(X_star)
+        self._device_points(X_star)
+        axes = self._grid_dev[1]
+        if axes is None:
+            raise ValueError("sample_posterior_grid: X_star is not an x-major tensor-product grid [[x, y] for x in ux for y in uy]; "
+                             "use sample_posterior for point sets")
+        if not self._dev.fitted:
+            self._refit(check=True)
+        self._dev.check_factor(force=True)        # LinAlgError for a non-SPD training covariance (deferred fit), as predict
+        d = self._dev.grid_sample_dim(axes)
+        rng = np.random.default_rng() if rng is None else rng
+        E = rng.standard_normal((d, int(n_samples)))
+        F = self._dev.posterior_sample_grid(axes, torch.from_numpy(E).to(self._dev.device))
         return F.cpu().numpy()
 
     def _device_points(self, X_star):

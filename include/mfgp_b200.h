@@ -355,6 +355,38 @@ int cov_finish(const double* cent, const double* areas_c, int64_t Ac, const doub
                const int32_t* flag0, const int32_t* flag1, const int32_t* flag2, const int32_t* flag3, double* out,
                void* stream);
 
+/* Per-cell centroids of joint posterior draws (Thompson sampling), reduced in Chebyshev coefficient space.  A draw of
+ * mfgp_grid_sample_coef is F_s(ix, iy) = mean + sum_l sum_k T_l(ty) T_k(tx) C[s][l][k] over the box [xlo,xhi] x [ylo,yhi];
+ * the Lloyd partials of a cell are linear in it, so they are dot products of C' = C + mean on term (0, 0) with per-cell
+ * moment tensors, and no draw is evaluated.
+ *
+ * cov_cell_moments: for the x-major tensor-product grid xy[nx*ny, 2] (point g = ix*ny + iy, as cov_assign_reduce_grid) and
+ * one partition (seeds[A,2], poly_xy / poly_off as cov_assign_reduce, 1 <= A <= 256), writes
+ *   mom[A][3][ry][kpad] (kpad = rx rounded up to 4; the term layout of mfgp_grid_sample_coef's C[S][ry][kpad]):
+ *   mom[i][w][l][k] = sum over the points p of cell i of w(p) T_l(ty_p) T_k(tx_p), w = 1, x, y.
+ * The T are taken of the grid's own coordinates on the box.  Membership is cov_assign_reduce_grid's: nearest seed with
+ * the runner-up, and the crossings test against every polygon when the gap is <= tie_tol (a tie point counts in every
+ * cell the test puts it in, possibly none; tie_tol = +inf: the crossings test everywhere).  tie_count (optional device
+ * int32) receives the number of points whose gap is <= tie_tol / 10, as cov_assign_reduce_grid's.  Deterministic (fixed
+ * summation order, no floating-point atomics).  xy, poly_xy, mom and work must be 16-byte aligned.
+ *
+ * cov_cell_moments_centroids: for S coefficient matrices C[S][ry][kpad] (contiguous, mfgp_grid_sample_coef's output) and
+ * the draws' constant mean, writes cent[S][A][4] = {sum F_s, sum F_s x, sum F_s y, n} of every cell (cov_assign_reduce's
+ * `cent` with w = F_s) and centroids[S][A][2] with cov_finish's arithmetic: ((sum F_s x / n) area) / ((sum F_s / n) area),
+ * then the one-sided clamps to [xmin,xmax] x [ymin,ymax]; an empty cell gives NaN.  areas[A]: the cells' areas.  Needs
+ * no scratch: its workspace query returns 0 and `work` may be NULL.  mom, C, cent and centroids must be 16-byte aligned.
+ *
+ * Both return MFGP_ERR_INVALID and enqueue nothing on bad sizes, orders outside [1, 64], misaligned buffers or a short
+ * workspace. */
+int64_t cov_cell_moments_workspace_bytes(int64_t nx, int64_t ny, int64_t A, int64_t rx, int64_t ry);
+int cov_cell_moments(const double* xy, int64_t nx, int64_t ny, const double* seeds, int64_t A, const double* poly_xy,
+                     const int32_t* poly_off, double tie_tol, double xlo, double xhi, double ylo, double yhi, int64_t rx,
+                     int64_t ry, double* mom, int32_t* tie_count, void* work, int64_t work_bytes, void* stream);
+int64_t cov_cell_moments_centroids_workspace_bytes(int64_t A, int64_t rx, int64_t ry, int64_t S);
+int cov_cell_moments_centroids(const double* mom, int64_t A, int64_t rx, int64_t ry, const double* C, int64_t S, double mean,
+                               const double* areas, double xmin, double xmax, double ymin, double ymax, double* cent,
+                               double* centroids, void* work, int64_t work_bytes, void* stream);
+
 /* Global first-index argmax of v[G] (np.argmax at simulator.py:352): out_val[1], out_idx[1]. */
 int cov_argmax(const double* v, int64_t G, int64_t base_index, double k0, double rel, double* out_val, int64_t* out_idx,
                void* work, int64_t work_bytes, void* stream);

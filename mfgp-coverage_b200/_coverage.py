@@ -502,6 +502,70 @@ class CoverageGrid:
              h[1 + 3 * Ac:1 + 4 * Ac].astype(np.int64))
         return r + (int(h[4 + 4 * Ac]),) if with_ties else r
 
+    def cell_moments(self, vor, box, orders, tie_tol=None):
+        """Moment tensors mom[A, 3, ry, kpad] of the partition `vor` over this whole tensor-product grid (cov_cell_moments) on
+        the Chebyshev basis of `box` = (xlo, xhi, ylo, yhi) with `orders` = (rx, ry), and the device int32 tie count.
+        Returns (mom, ties, partition used), the partition as CoverageGrid.upload gives it."""
+        if self.axes is None or self.base_index:
+            raise ValueError("sample_centroids: the grid is not a whole x-major tensor-product grid [[x, y] for x in ux for y in uy]")
+        P = self.upload(vor)
+        if P is None:
+            raise ValueError("sample_centroids: the partition has no cell")
+        if tie_tol is None:
+            tie_tol = TIE_TOL if P.seeds_inside else math.inf
+        rx, ry = int(orders[0]), int(orders[1])
+        lib = nat.lib()
+        nx, ny, A = self.axes.nx, self.axes.ny, P.A
+        wb = int(lib.cov_cell_moments_workspace_bytes(nx, ny, A, rx, ry))
+        f64 = dict(dtype=torch.float64, device=self.device)
+        mom = torch.empty((A, 3, ry, -(-rx // 4) * 4), **f64)
+        ties = torch.empty(2, dtype=torch.int32, device=self.device)[:1]
+        work = torch.empty(wb // 8 + 2, **f64)
+        nat.check(lib.cov_cell_moments(nat.ptr(self.xy), nx, ny, nat.ptr(P.seeds), A, nat.ptr(P.poly), nat.ptr(P.off),
+                                       ctypes.c_double(tie_tol), *(ctypes.c_double(v) for v in box), rx, ry, nat.ptr(mom),
+                                       nat.ptr(ties), nat.ptr(work), wb, nat.stream_ptr()), "cov_cell_moments")
+        return mom, ties, P
+
+    def sample_centroids(self, model, vor, normals, bbox=None):
+        """Per-cell Lloyd partials and centroids of joint posterior draws over this whole tensor-product grid, without
+        evaluating the draws: the draws are DeviceGP.posterior_sample_grid's at the same `normals` (a float64 [d, S] device
+        tensor, d = model.grid_sample_dim(grid)), their coefficients are contracted with the partition's moment tensors
+        (cov_cell_moments, cov_cell_moments_centroids).  `model`: an MFGP / SFGP; `vor`: the partition (any type
+        assign_reduce takes); `bbox`: the clamp box of the centroids, default the grid's extent.
+        Returns device tensors cent[S, A, 4] = {sum F_s, sum F_s x, sum F_s y, n} (assign_reduce's `cent` with w = F_s) and
+        centroids[S, A, 2] (compute_centroids' arithmetic; NaN for an empty cell).  Like reduce_to_host, a HybridVoronoi
+        partition whose pass meets hard ties is passed again on Qhull's polygons.  Raises the sampler's errors: ValueError
+        for a grid that is not a whole tensor-product grid or orders above 64, MemoryError before allocating, LinAlgError for
+        a non-SPD fit."""
+        eng = model._dev
+        axes = model._grid_axes(self)
+        if not eng.fitted:
+            model._refit(check=True)
+        eng.check_factor(force=True)
+        plan = eng._grid_sample_plan(axes)
+        A = len(vor)
+        rx, ry = plan["rx"], plan["ry"]
+        kpad = -(-rx // 4) * 4
+        S = int(normals.shape[1]) if normals.dim() == 2 else 0
+        extra = int(nat.lib().cov_cell_moments_workspace_bytes(axes.nx, axes.ny, max(A, 1), rx, ry)) + \
+            8 * (3 * A * ry * kpad + 6 * S * A)
+        C, plan = eng.posterior_sample_grid_coef(axes, normals, extra_bytes=extra)
+        mom, ties, _ = self.cell_moments(vor, plan["box"], (rx, ry))
+        if isinstance(vor, HybridVoronoi) and vor._qhull is None and int(ties.item()):
+            vor.qhull()          # tie points: their membership is decided by Qhull's vertices, as in the reference
+            mom, ties, _ = self.cell_moments(vor, plan["box"], (rx, ry))
+        areas = torch.from_numpy(np.ascontiguousarray(vor.areas(), dtype=np.float64)).to(self.device)
+        if bbox is None:
+            bbox = (axes.xlo, axes.xhi, axes.ylo, axes.yhi)
+        f64 = dict(dtype=torch.float64, device=self.device)
+        cent = torch.empty((S, A, 4), **f64)
+        cen = torch.empty((S, A, 2), **f64)
+        nat.check(nat.lib().cov_cell_moments_centroids(nat.ptr(mom), A, rx, ry, nat.ptr(C), S,
+                                                       ctypes.c_double(eng.params["mean_H"]), nat.ptr(areas),
+                                                       *(ctypes.c_double(v) for v in bbox), nat.ptr(cent), nat.ptr(cen),
+                                                       None, 0, nat.stream_ptr()), "cov_cell_moments_centroids")
+        return cent, cen
+
     def argmax(self, v_dev, k0=0.0, rel=0.0):
         """First-index argmax of a device vector (np.argmax semantics): returns (value, index) device tensors."""
         val = torch.empty(1, dtype=torch.float64, device=self.device)

@@ -635,6 +635,50 @@ class DeviceGP:
                                             nat.ptr(work), work.numel() * 8, st), "mfgp_grid_sample_eval")
         return F
 
+    def posterior_sample_grid_coef(self, axes, normals, extra_bytes=0):
+        """The coefficients of the draws posterior_sample_grid evaluates, without evaluating them: C[S, ry * kpad] (term (l, k) in
+        column l * kpad + k, kpad = rx rounded up to 4) with F_s = mean_H + sum T_l(ty) T_k(tx) C[s][l][k] on plan["box"].
+        Returns (C, plan).  `extra_bytes`: the caller's own allocations, included in the memory check (MemoryError before
+        anything is allocated)."""
+        self.ensure_factor(need_inverse=True)
+        plan = self._grid_sample_plan(axes)
+        d = plan["d0"] + self.N
+        if (normals.dtype != torch.float64 or normals.device != self.device or normals.dim() != 2 or normals.shape[0] != d
+                or normals.shape[1] < 1):
+            raise ValueError(f"posterior_sample_grid: normals must be a float64 [{d}, S] tensor on {self.device}, S >= 1")
+        S = int(normals.shape[1])
+        lib = nat.lib()
+        rxL, ryL, rxH, ryH = plan["orders"]
+        R = plan["ry"] * (-(-plan["rx"] // 4) * 4)
+        lde = S + (S & 1)
+        copy_e = not ((S == 1 or normals.stride(1) == 1) and (d == 1 or normals.stride(0) % 2 == 0)
+                      and normals.data_ptr() % 16 == 0)
+        cw = int(lib.mfgp_grid_sample_coef_workspace_bytes(self.N, rxL, ryL, rxH, ryH, S))
+        need = cw + int(extra_bytes) + 8 * (S * R + (d * lde if copy_e else 0)) + 1024
+        free, _ = torch.cuda.mem_get_info(self.device)
+        free += torch.cuda.memory_reserved(self.device) - torch.cuda.memory_allocated(self.device)
+        if need > free:
+            raise MemoryError(f"posterior_sample_grid: {S} draws need {need / 1e9:.2f} GB (coefficients, moments, scratch), "
+                              f"{free / 1e9:.2f} GB of device memory is free")
+        f64 = dict(dtype=torch.float64, device=self.device)
+        if copy_e:
+            E, lde_e = torch.empty((d, lde), **f64), lde
+            E[:, :S].copy_(normals)
+        else:
+            E, lde_e = normals, (int(normals.stride(0)) if d > 1 else lde)
+        C = torch.empty((S, R), **f64)
+        work = torch.empty(cw // 8 + 2, **f64)
+        Q = plan["Q"]
+        xlo, xhi, ylo, yhi = (ctypes.c_double(v) for v in plan["box"])
+        N = self.N
+        nat.check(lib.mfgp_grid_sample_coef(nat.ptr(self.Xt) if N else None, nat.ptr(self.y) if N else None, self.NL, self.NH,
+                                            nat.ptr(self.W) if N else None, self.npad if N else 0, self.cap if N else 0,
+                                            ctypes.byref(self.pstruct), rxL, ryL, rxH, ryH, xlo, xhi, ylo, yhi,
+                                            nat.ptr(Q.get("Lx")), nat.ptr(Q.get("Ly")), nat.ptr(Q["Hx"]), nat.ptr(Q["Hy"]),
+                                            nat.ptr(E), lde_e, S, nat.ptr(C), nat.ptr(work), work.numel() * 8,
+                                            nat.stream_ptr()), "mfgp_grid_sample_coef")
+        return C, plan
+
     # -- factored posterior on tensor-product grids (gp_factored.cu) ---------------------------------------------------------
     def _training_range(self):
         """(xmin, xmax, ymin, ymax) of the training points, tracked on the host by fit / append_hifi."""

@@ -138,6 +138,14 @@ SIGNATURES = {
                                  c_int64, c_void_p, c_void_p, c_void_p, c_int64, c_void_p]),
     "cov_finish": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_double,
                            c_double, c_double, c_double, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "cov_cell_moments_workspace_bytes": (c_int64, [c_int64, c_int64, c_int64, c_int64, c_int64]),
+    "cov_cell_moments": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_double, c_double,
+                                 c_double, c_double, c_double, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_int64,
+                                 c_void_p]),
+    "cov_cell_moments_centroids_workspace_bytes": (c_int64, [c_int64, c_int64, c_int64, c_int64]),
+    "cov_cell_moments_centroids": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int64, c_double, c_void_p,
+                                           c_double, c_double, c_double, c_double, c_void_p, c_void_p, c_void_p, c_int64,
+                                           c_void_p]),
     "cov_argmax": (c_int, [c_void_p, c_int64, c_int64, c_double, c_double, c_void_p, c_void_p, c_void_p, c_int64,
                            c_void_p]),
     "choi_greedy": (c_int64, [c_void_p, c_int64, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_void_p,

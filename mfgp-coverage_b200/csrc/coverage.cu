@@ -13,6 +13,7 @@
 // per-block partials in global memory, and a second kernel that adds the block partials in block order.
 #include <cfloat>
 #include <climits>
+#include <cmath>
 
 #include "common.cuh"
 #include "argmax.cuh"
@@ -1053,6 +1054,341 @@ extern "C" int cov_voronoi_clip(const double* seeds, int64_t A, double xmin, dou
                                                                                          ymax + h, scratch, counts, areas, flag);
     MFGP_LAUNCH_CHECK();
     cov_voronoi_pack_kernel<<<1, 256, 0, st>>>(scratch, counts, (int)A, poly_xy, poly_off, (int)cap_vertices, areas, flag);
+    MFGP_LAUNCH_CHECK();
+    return MFGP_OK;
+}
+
+namespace mfgp {
+
+// ---- per-cell centroids of posterior draws, reduced in Chebyshev coefficient space ------------------------------------------
+// A draw over a tensor-product grid is F_s(ix, iy) = mean + sum_l sum_k Uy[iy][l] Ux[ix][k] C_s[l][k] (mfgp_grid_sample_coef's
+// coefficients, basis T_l(ty) T_k(tx) on the sampler's box).  The Lloyd partials of cell i are linear in the draw:
+//   sum_{p in cell i} w(p) F_s(p) = <C'_s, Mom_i^w>,   Mom_i^w[l][k] = sum_ix Ux[ix][k] sum_{iy in cell i, column ix} w Uy[iy][l]
+// with w in {1, x, y} and C' = C + mean on term (0, 0) (T_0 = 1).  So the moments are formed once per partition and every draw
+// costs 3 dot products of length ry kpad per cell; no draw is evaluated.
+//   cov_moment_basis_kernel    Ux[ix][k] (zero for k >= rx), Uy[iy][l] from the grid's own coordinates
+//   cov_moment_columns_kernel  one CTA per column: membership as cov_assign_reduce_grid (nearest seed + runner-up, the
+//                              crossings test for ties), then Sy[i][ix][0][l] = sum Uy[iy][l], Sy[i][ix][1][l] = sum y Uy[iy][l]
+//                              over the column's points of cell i; thread (m, l) owns those sums and adds in row order
+//   cov_moment_reduce_kernel   one CTA per cell over the columns it touches: Mom_i^{1,x,y} = Ux^T Sy_i (x weights per column)
+//   cov_moment_centroid_kernel one CTA per (cell, 32 draws): the three dot products, then cov_finish's centroid arithmetic
+// Every sum runs in a fixed order (no floating-point atomics): the same inputs give the same bits.
+constexpr int CM_MAXR = 64;            // largest Chebyshev order per axis (the sampler's limit)
+constexpr int CM_THREADS = 2 * CM_MAXR; // column kernel: thread (m, l) owns moment m of y term l
+constexpr int CM_ROWS = 512;           // rows of a column classified per pass
+constexpr int CM_WORDS = COV_MAX_CELLS / 64;
+constexpr int CR_COLS = 16;            // columns staged per step of the reduction kernel
+constexpr int CC_WARPS = 8, CC_DRAWS = 32;   // centroid kernel: draws per CTA (CC_DRAWS / CC_WARPS per warp)
+
+struct MomArgs {
+    const double* xy; int64_t nx, ny;
+    const double* seeds; int A; const double* poly_xy; const int32_t* poly_off;
+    double tie_tol;
+    const uint4* buckets; const double* geom; int nb;
+    const double* Uy; int ry;
+    double* Sy;             // [A][nx][2][ry]
+    int* colr;              // [A][2]: first and last column that holds a point of the cell
+    int* tie_count;
+};
+
+__global__ void cov_moment_basis_kernel(const double* __restrict__ xy, int64_t nx, int64_t ny, double xlo, double xhi, double ylo,
+                                        double yhi, int rx, int kpad, int ry, double* __restrict__ Ux, double* __restrict__ Xc,
+                                        double* __restrict__ Uy) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= nx + ny) return;
+    const bool isx = i < nx;
+    const double u = isx ? xy[2 * (i * ny)] : xy[2 * (i - nx) + 1];
+    const double lo = isx ? xlo : ylo, hi = isx ? xhi : yhi;
+    const int r = isx ? rx : ry, w = isx ? kpad : ry;
+    double* row = isx ? Ux + i * kpad : Uy + (i - nx) * ry;
+    if (isx) Xc[i] = u;
+    const double t = (2.0 * u - (lo + hi)) / (hi - lo);      // the recurrence of cheb_basis_kernel (cheb.cuh)
+    double t0 = 1.0, t1 = t;
+    for (int k = 0; k < w; k++) {
+        row[k] = k < r ? t0 : 0.0;
+        const double t2 = 2.0 * t * t1 - t0;
+        t0 = t1; t1 = t2;
+    }
+}
+
+__global__ void __launch_bounds__(CM_THREADS) cov_moment_columns_kernel(MomArgs a) {
+    __shared__ double s_seeds[2 * COV_MAX_CELLS];
+    __shared__ int s_cell[CM_ROWS];
+    __shared__ double s_y[CM_ROWS];
+    __shared__ unsigned long long s_mask[CM_ROWS][CM_WORDS];
+    const int tid = threadIdx.x, lane = tid & 31;
+    const int64_t ix = blockIdx.x;
+    for (int i = tid; i < 2 * a.A; i += CM_THREADS) s_seeds[i] = a.seeds[i];
+    const BucketGrid bg{a.buckets, a.nb, a.geom[0], a.geom[1], a.geom[2]};
+    const bool polygon_mode = !(a.tie_tol < 1e300);
+    const int ry = a.ry;
+    const bool owner = tid < 2 * ry;
+    const int m = tid < ry ? 0 : 1, l = tid < ry ? tid : tid - ry;
+    const bool ranges = tid == 0;          // thread (0, 0) sees every run of every cell: it keeps the column ranges
+    double* __restrict__ sy = a.Sy + (ix * 2 + m) * ry + l;           // + cell * nx * 2 * ry
+    const int64_t cstride = a.nx * 2 * ry;
+    double acc = 0.0;
+    int cur = CELL_NONE;
+    auto flush = [&]() {
+        if (cur >= 0) {
+            sy[cur * cstride] += acc;
+            if (ranges) { atomicMin(a.colr + 2 * cur, (int)ix); atomicMax(a.colr + 2 * cur + 1, (int)ix); }
+        }
+        acc = 0.0;
+        cur = CELL_NONE;
+    };
+    for (int64_t r0 = 0; r0 < a.ny; r0 += CM_ROWS) {
+        const int nr = (int)min((int64_t)CM_ROWS, a.ny - r0);
+        __syncthreads();                   // the previous pass's rows are consumed (and the seeds are in)
+        for (int rb = 0; rb < CM_ROWS; rb += CM_THREADS) {
+            const int r = rb + tid;
+            const bool valid = r < nr;
+            int cell = CELL_NONE;
+            double x = 0.0, y = 0.0;
+            if (valid) {
+                const double2 p = __ldg(reinterpret_cast<const double2*>(a.xy) + ix * a.ny + r0 + r);
+                x = p.x; y = p.y;
+                cell = polygon_mode ? CELL_TIE : classify_point(bg, s_seeds, a.A, x, y, a.tie_tol);
+            }
+            const unsigned hm = __ballot_sync(0xffffffffu, cell == CELL_TIE_HARD);
+            if (hm && a.tie_count != nullptr && lane == 0) atomicAdd(a.tie_count, __popc(hm));
+            if (cell == CELL_TIE_HARD) cell = CELL_TIE;
+            if (cell == CELL_TIE) {        // the reference's crossings test against every cell polygon: 0, 1 or several cells
+                unsigned long long k0 = 0ull, k1 = 0ull, k2 = 0ull, k3 = 0ull;
+                for (int c = 0; c < a.A; c++) {
+                    const int o = a.poly_off[c];
+                    if (crossings_inside(a.poly_xy + 2 * o, a.poly_off[c + 1] - o, x, y)) {
+                        const unsigned long long bit = 1ull << (c & 63);
+                        const int w = c >> 6;
+                        k0 |= w == 0 ? bit : 0ull; k1 |= w == 1 ? bit : 0ull; k2 |= w == 2 ? bit : 0ull; k3 |= w == 3 ? bit : 0ull;
+                    }
+                }
+                s_mask[r][0] = k0; s_mask[r][1] = k1; s_mask[r][2] = k2; s_mask[r][3] = k3;
+            }
+            if (valid) { s_cell[r] = cell; s_y[r] = y; }
+        }
+        __syncthreads();
+        if (owner) {
+            const double* __restrict__ uy = a.Uy + r0 * ry + l;
+            for (int r = 0; r < nr; r++) {
+                const int c = s_cell[r];
+                const double u = __ldg(uy + (int64_t)r * ry);
+                const double v = m ? s_y[r] * u : u;
+                if (c >= 0) {
+                    if (c != cur) { flush(); cur = c; }
+                    acc += v;
+                } else {
+                    flush();
+#pragma unroll
+                    for (int w = 0; w < CM_WORDS; w++) {
+                        unsigned long long mk = s_mask[r][w];
+                        while (mk) {
+                            const int cc = 64 * w + __ffsll((long long)mk) - 1;
+                            mk &= mk - 1;
+                            sy[cc * cstride] += v;
+                            if (ranges) { atomicMin(a.colr + 2 * cc, (int)ix); atomicMax(a.colr + 2 * cc + 1, (int)ix); }
+                        }
+                    }
+                }
+            }
+        }
+    }
+    if (owner) flush();
+}
+
+__global__ void cov_moment_init_kernel(int* __restrict__ colr, int A) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < A) { colr[2 * i] = INT_MAX; colr[2 * i + 1] = -1; }
+}
+
+// Mom[i][0] = Ux^T Sy_i[., 0], Mom[i][1] = (x Ux)^T Sy_i[., 0], Mom[i][2] = Ux^T Sy_i[., 1] over the columns cell i touches.
+// Thread (tl, tk) owns the terms l = tl + 16 a, k = tk + 16 b (a, b < 4): 48 accumulators in registers, columns in order.
+__global__ void __launch_bounds__(256) cov_moment_reduce_kernel(const double* __restrict__ Sy, const int* __restrict__ colr,
+                                                                const double* __restrict__ Ux, const double* __restrict__ Xc,
+                                                                int64_t nx, int ry, int kpad, double* __restrict__ mom) {
+    __shared__ double s_sy[CR_COLS][2][CM_MAXR];
+    __shared__ double s_ux[CR_COLS][CM_MAXR];
+    __shared__ double s_x[CR_COLS];
+    const int c = blockIdx.x, tid = threadIdx.x;
+    const int tl = tid >> 4, tk = tid & 15;
+    const int c0 = colr[2 * c], c1 = colr[2 * c + 1];
+    double acc[3][4][4];
+#pragma unroll
+    for (int q = 0; q < 3; q++)
+#pragma unroll
+        for (int i = 0; i < 4; i++)
+#pragma unroll
+            for (int j = 0; j < 4; j++) acc[q][i][j] = 0.0;
+    const double* syc = Sy + (int64_t)c * nx * 2 * ry;
+    for (int64_t b0 = c0; b0 <= c1; b0 += CR_COLS) {      // empty cell: c1 = -1 < c0, no iteration
+        const int nc = (int)min((int64_t)CR_COLS, (int64_t)c1 + 1 - b0);
+        __syncthreads();
+        for (int e = tid; e < nc * 2 * ry; e += 256) {
+            const int q = e / (2 * ry), rem = e % (2 * ry);
+            s_sy[q][rem / ry][rem % ry] = syc[(b0 + q) * 2 * ry + rem];
+        }
+        for (int e = tid; e < nc * kpad; e += 256) s_ux[e / kpad][e % kpad] = Ux[(b0 + e / kpad) * kpad + e % kpad];
+        if (tid < nc) s_x[tid] = Xc[b0 + tid];
+        __syncthreads();
+        for (int q = 0; q < nc; q++) {
+            double a0[4], a1[4], u[4], ux[4];
+            const double xq = s_x[q];
+#pragma unroll
+            for (int i = 0; i < 4; i++) {
+                const int ll = tl + 16 * i;
+                a0[i] = ll < ry ? s_sy[q][0][ll] : 0.0;
+                a1[i] = ll < ry ? s_sy[q][1][ll] : 0.0;
+            }
+#pragma unroll
+            for (int j = 0; j < 4; j++) {
+                const int k = tk + 16 * j;
+                u[j] = k < kpad ? s_ux[q][k] : 0.0;
+                ux[j] = xq * u[j];
+            }
+#pragma unroll
+            for (int i = 0; i < 4; i++)
+#pragma unroll
+                for (int j = 0; j < 4; j++) {
+                    acc[0][i][j] = fma(a0[i], u[j], acc[0][i][j]);
+                    acc[1][i][j] = fma(a0[i], ux[j], acc[1][i][j]);
+                    acc[2][i][j] = fma(a1[i], u[j], acc[2][i][j]);
+                }
+        }
+    }
+    const int64_t R = (int64_t)ry * kpad;
+#pragma unroll
+    for (int i = 0; i < 4; i++) {
+        const int ll = tl + 16 * i;
+        if (ll >= ry) continue;
+#pragma unroll
+        for (int j = 0; j < 4; j++) {
+            const int k = tk + 16 * j;
+            if (k >= kpad) continue;
+#pragma unroll
+            for (int q = 0; q < 3; q++) mom[((int64_t)c * 3 + q) * R + ll * kpad + k] = acc[q][i][j];
+        }
+    }
+}
+
+// cent[s][i] = (sum F_s, sum F_s x, sum F_s y, n) of cell i = <C'_s, Mom_i^{1,x,y}>, n = Mom_i^1[0][0] (an exact count: T_0 = 1);
+// centroids[s][i] with cov_finish's arithmetic: ((m/n) area) / ((m0/n) area), then the one-sided clamps (NaN stays NaN).
+__global__ void __launch_bounds__(CC_WARPS * 32) cov_moment_centroid_kernel(const double* __restrict__ mom, int A, int R,
+                                                                            const double* __restrict__ C, int S, double mean,
+                                                                            const double* __restrict__ areas, double xmin,
+                                                                            double xmax, double ymin, double ymax,
+                                                                            double* __restrict__ cent, double* __restrict__ cen) {
+    extern __shared__ __align__(16) double s_mom[];     // [3][R]
+    const int c = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    for (int e = tid; e < 3 * R; e += CC_WARPS * 32) s_mom[e] = mom[(int64_t)c * 3 * R + e];
+    __syncthreads();
+    const double n = s_mom[0], area = areas[c];
+    for (int si = warp; si < CC_DRAWS; si += CC_WARPS) {
+        const int s = blockIdx.y * CC_DRAWS + si;
+        if (s >= S) break;
+        const double* cs = C + (int64_t)s * R;
+        double m0 = 0.0, m1 = 0.0, m2 = 0.0;
+        for (int e = lane; e < R; e += 32) {
+            const double v = e == 0 ? cs[0] + mean : cs[e];
+            m0 = fma(v, s_mom[e], m0);
+            m1 = fma(v, s_mom[R + e], m1);
+            m2 = fma(v, s_mom[2 * R + e], m2);
+        }
+        m0 = warp_sum(m0); m1 = warp_sum(m1); m2 = warp_sum(m2);
+        if (lane == 0) {
+            double* o = cent + ((int64_t)s * A + c) * 4;
+            o[0] = m0; o[1] = m1; o[2] = m2; o[3] = n;
+            const double f_int = __dmul_rn(__ddiv_rn(m0, n), area);
+            double cx = __ddiv_rn(__dmul_rn(__ddiv_rn(m1, n), area), f_int);
+            double cy = __ddiv_rn(__dmul_rn(__ddiv_rn(m2, n), area), f_int);
+            if (cx < xmin) cx = xmin;
+            if (cx > xmax) cx = xmax;
+            if (cy < ymin) cy = ymin;
+            if (cy > ymax) cy = ymax;
+            cen[((int64_t)s * A + c) * 2] = cx;
+            cen[((int64_t)s * A + c) * 2 + 1] = cy;
+        }
+    }
+}
+
+struct MomLayout { double *Sy, *Ux, *Xc, *Uy; int* colr; uint4* buckets; double* geom; int64_t bytes; };
+inline int64_t cm_rup(int64_t v) { return (v + 255) / 256 * 256; }
+inline MomLayout cm_layout(int64_t nx, int64_t ny, int64_t A, int64_t rx, int64_t ry, void* work) {
+    const int64_t kpad = (rx + 3) / 4 * 4;
+    char* base = static_cast<char*>(work);
+    int64_t used = 0;
+    auto carve = [&](int64_t bytes) { char* p = base ? base + used : nullptr; used += cm_rup(bytes); return p; };
+    MomLayout L{};
+    L.Sy = reinterpret_cast<double*>(carve(A * nx * 2 * ry * 8));
+    L.Ux = reinterpret_cast<double*>(carve(nx * kpad * 8));
+    L.Xc = reinterpret_cast<double*>(carve(nx * 8));
+    L.Uy = reinterpret_cast<double*>(carve(ny * ry * 8));
+    L.colr = reinterpret_cast<int*>(carve(A * 2 * 4));
+    L.buckets = reinterpret_cast<uint4*>(carve((int64_t)COV_BUCKETS_MAX * COV_BUCKETS_MAX * 16));
+    L.geom = reinterpret_cast<double*>(carve(64));
+    L.bytes = used;
+    return L;
+}
+inline bool cm_al(const void* p, uintptr_t a) { return (reinterpret_cast<uintptr_t>(p) & (a - 1)) == 0; }
+inline bool cm_box_ok(double lo, double hi) { return hi > lo && std::isfinite(hi - lo); }
+}  // namespace mfgp
+
+extern "C" int64_t cov_cell_moments_workspace_bytes(int64_t nx, int64_t ny, int64_t A, int64_t rx, int64_t ry) {
+    if (nx <= 0 || ny <= 0 || A <= 0 || A > COV_MAX_CELLS || rx <= 0 || rx > CM_MAXR || ry <= 0 || ry > CM_MAXR) return 0;
+    return cm_layout(nx, ny, A, rx, ry, nullptr).bytes;
+}
+
+extern "C" int cov_cell_moments(const double* xy, int64_t nx, int64_t ny, const double* seeds, int64_t A, const double* poly_xy,
+                                const int32_t* poly_off, double tie_tol, double xlo, double xhi, double ylo, double yhi, int64_t rx,
+                                int64_t ry, double* mom, int32_t* tie_count, void* work, int64_t work_bytes, void* stream) {
+    if (!xy || !seeds || !poly_xy || !poly_off || !mom || !work) return MFGP_ERR_INVALID;
+    if (nx <= 0 || ny <= 0 || nx >= (1LL << 31) - 1 || ny >= (1LL << 40) / nx || A <= 0 || A > COV_MAX_CELLS) return MFGP_ERR_INVALID;
+    if (rx <= 0 || rx > CM_MAXR || ry <= 0 || ry > CM_MAXR || tie_tol != tie_tol || tie_tol < 0.0) return MFGP_ERR_INVALID;
+    if (!cm_box_ok(xlo, xhi) || !cm_box_ok(ylo, yhi)) return MFGP_ERR_INVALID;
+    if (!cm_al(xy, 16) || !cm_al(poly_xy, 16) || !cm_al(seeds, 8) || !cm_al(poly_off, 4) || !cm_al(mom, 16) || !cm_al(work, 16) ||
+        !cm_al(tie_count, 4))
+        return MFGP_ERR_INVALID;
+    if (work_bytes < cm_layout(nx, ny, A, rx, ry, nullptr).bytes) return MFGP_ERR_INVALID;
+    const MomLayout L = cm_layout(nx, ny, A, rx, ry, work);
+    const int kpad = (int)((rx + 3) / 4 * 4);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (tie_count) MFGP_CUDA_CHECK(cudaMemsetAsync(tie_count, 0, sizeof(int32_t), st));
+    MFGP_CUDA_CHECK(cudaMemsetAsync(L.Sy, 0, sizeof(double) * A * nx * 2 * ry, st));
+    cov_moment_init_kernel<<<(unsigned)((A + 255) / 256), 256, 0, st>>>(L.colr, (int)A);
+    MFGP_LAUNCH_CHECK();
+    const int nb = cov_bucket_side(A);
+    BucketBuild bb{seeds, (int)A, poly_xy, poly_off, nb, L.buckets, L.geom};
+    cov_build_buckets_kernel<<<dim3((unsigned)((nb * nb + 7) / 8), 1), 256, 0, st>>>(bb, bb, tie_tol);
+    MFGP_LAUNCH_CHECK();
+    cov_moment_basis_kernel<<<(unsigned)((nx + ny + 127) / 128), 128, 0, st>>>(xy, nx, ny, xlo, xhi, ylo, yhi, (int)rx, kpad, (int)ry,
+                                                                              L.Ux, L.Xc, L.Uy);
+    MFGP_LAUNCH_CHECK();
+    MomArgs a{xy, nx, ny, seeds, (int)A, poly_xy, poly_off, tie_tol, L.buckets, L.geom, nb, L.Uy, (int)ry, L.Sy, L.colr, tie_count};
+    cov_moment_columns_kernel<<<(unsigned)nx, CM_THREADS, 0, st>>>(a);
+    MFGP_LAUNCH_CHECK();
+    cov_moment_reduce_kernel<<<(unsigned)A, 256, 0, st>>>(L.Sy, L.colr, L.Ux, L.Xc, nx, (int)ry, kpad, mom);
+    MFGP_LAUNCH_CHECK();
+    return MFGP_OK;
+}
+
+extern "C" int64_t cov_cell_moments_centroids_workspace_bytes(int64_t A, int64_t rx, int64_t ry, int64_t S) {
+    (void)A; (void)rx; (void)ry; (void)S;
+    return 0;
+}
+
+extern "C" int cov_cell_moments_centroids(const double* mom, int64_t A, int64_t rx, int64_t ry, const double* C, int64_t S, double mean,
+                                          const double* areas, double xmin, double xmax, double ymin, double ymax, double* cent,
+                                          double* centroids, void* work, int64_t work_bytes, void* stream) {
+    (void)work;
+    if (!mom || !C || !areas || !cent || !centroids || work_bytes < 0) return MFGP_ERR_INVALID;
+    if (A <= 0 || A > COV_MAX_CELLS || rx <= 0 || rx > CM_MAXR || ry <= 0 || ry > CM_MAXR || S <= 0 || S >= (1LL << 21))
+        return MFGP_ERR_INVALID;
+    if (!cm_al(mom, 16) || !cm_al(C, 16) || !cm_al(areas, 8) || !cm_al(cent, 16) || !cm_al(centroids, 16)) return MFGP_ERR_INVALID;
+    const int R = (int)(ry * ((rx + 3) / 4 * 4));
+    const int smem = 3 * R * (int)sizeof(double);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    MFGP_CUDA_CHECK(cudaFuncSetAttribute(cov_moment_centroid_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    cov_moment_centroid_kernel<<<dim3((unsigned)A, (unsigned)((S + CC_DRAWS - 1) / CC_DRAWS)), CC_WARPS * 32, smem, st>>>(
+        mom, (int)A, R, C, (int)S, mean, areas, xmin, xmax, ymin, ymax, cent, centroids);
     MFGP_LAUNCH_CHECK();
     return MFGP_OK;
 }

@@ -24,7 +24,7 @@ eps = 0.1
 
 def run_sim(args):
     """reference runner.py:33-69."""
-    from .simulator import choi, lloyd, periodic, todescato
+    from .simulator import choi, lloyd, periodic, thompson, todescato
     (out_name, algo, sim_num, iterations, agents, truth, sigma_n, prior, hyp, console, plotter, log) = args
     print(line_break + f"Start Simulation {sim_num} : {algo}" + line_break)
     sim_start = time.time()
@@ -39,6 +39,8 @@ def run_sim(args):
         fn = lloyd
     elif "periodic" in algo:
         fn = periodic
+    elif "thompson" in algo:
+        fn = thompson
     else:
         raise ValueError("Invalid simulation algorithm specified.")
     loss_log_t, agent_log_t, sample_log_t = fn(algo, sim_num, iterations, agents, positions, truth, sigma_n, prior,

@@ -152,6 +152,22 @@ def compute_centroids(vor, x_star, mu_star):
     return cv.centroids_from_partials(host["cent"], vor.areas(), *grid.extent)
 
 
+def compute_centroids_samples(vor, x_star, model, n_samples=1, rng=None):
+    """compute_centroids under `n_samples` joint posterior draws of `model` over the whole tensor-product grid x_star instead
+    of its posterior mean: centroids[n_samples, A, 2], row s with w = draw s.  The draws are
+    model.sample_posterior_grid(x_star, n_samples, rng)'s (normals E = rng.standard_normal((d, n_samples)), `rng` a numpy
+    Generator, default np.random.default_rng()), but they are never evaluated: their Chebyshev coefficients are contracted
+    with per-cell moment tensors on the device (CoverageGrid.sample_centroids)."""
+    if int(n_samples) != n_samples or n_samples < 1:
+        raise ValueError(f"compute_centroids_samples: n_samples must be a positive integer, got {n_samples}")
+    grid = _grid_for(np.asarray(x_star))
+    d = model.grid_sample_dim(grid)
+    rng = np.random.default_rng() if rng is None else rng
+    E = rng.standard_normal((d, int(n_samples)))
+    _, cen = grid.sample_centroids(model, vor, torch.from_numpy(E).to(grid.device), bbox=grid.extent)
+    return cen.cpu().numpy()
+
+
 def _as_var_vector(var_star, device):
     if torch.is_tensor(var_star):
         return var_star
@@ -673,6 +689,79 @@ def todescato(title, sim_num, iterations, agents, positions, truth, sigma_n, pri
     """reference simulator.py:788-954.  `group`: see lloyd."""
     return _explore_exploit("todescato", title, sim_num, iterations, agents, positions, truth, sigma_n, prior, hyp,
                             console, log, rng, noise_rng, group)
+
+
+def _nearest_index(u, v):
+    """Index of the axis value nearest v; ties go to the lower index."""
+    return int(np.argmin(np.abs(u - v)))
+
+
+def snap_to_grid(targets, positions, ux, uy):
+    """Grid point of every agent for Thompson sampling, in agent order: the point of the grid [[x, y] for x in ux for y in uy]
+    nearest its target (per axis; ties go to the lower index).  When a lower-index agent already took that point, or the
+    target is NaN, the agent goes to the grid point nearest its current position instead."""
+    taken = set()
+    out = np.empty((targets.shape[0], 2))
+    for i in range(targets.shape[0]):
+        t = targets[i]
+        g = (_nearest_index(ux, t[0]), _nearest_index(uy, t[1])) if np.all(np.isfinite(t)) else None
+        if g is None or g in taken:
+            g = (_nearest_index(ux, positions[i, 0]), _nearest_index(uy, positions[i, 1]))
+        taken.add(g)
+        out[i] = (ux[g[0]], uy[g[1]])
+    return out
+
+
+def thompson(title, sim_num, iterations, agents, positions, truth, sigma_n, prior, hyp, console, plotter, log,
+             rng=None, noise_rng=None, group=None):
+    """Thompson-sampling coverage.  Every iteration each agent samples the truth at its position (not at iteration 0: the
+    start positions are not grid points), the model is updated, and the step's loss and cell variances are logged as in
+    periodic / todescato.  Then one independent joint posterior draw per agent is taken over the whole grid, and agent i
+    heads for the centroid of its own Voronoi cell under draw i, snapped to the grid (snap_to_grid).  The draws are never
+    evaluated (CoverageGrid.sample_centroids).  `rng`: a numpy Generator for the draws' normals (default: seeded from
+    random.getrandbits(64), so runner.run(seed=...) replays the run); `noise_rng` as in periodic.  XCentroid / YCentroid log
+    the unsnapped targets, ProbExplore = Explore = 1.  Needs a tensor-product grid; a process group of more than one rank
+    raises ValueError."""
+    if _sharded(group):
+        raise ValueError("thompson does not run on a sharded grid: use a process group of one rank")
+    loss_log, agent_log, sample_log = [], [], [] if log else None
+    fidelity = _fidelity_of(hyp)
+    print(line_break + title + line_break)
+    rng = np.random.default_rng(random.getrandbits(64)) if rng is None else rng
+    sim = _Sim(truth)
+    if sim.grid.axes is None:
+        raise ValueError("thompson needs a tensor-product grid [[x, y] for x in ux for y in uy]")
+    ux, uy = sim.grid.axes.ux_host, sim.grid.axes.uy_host
+    model, max_var_0 = _init_models(fidelity, hyp, prior)
+    print("Max Initial Predictive Variance: " + str(max_var_0)) if console else None
+    truth_arr = sim.truth_arr
+    ones = np.ones((agents, 1))
+    prev_positions = np.copy(positions)
+    centroids_t = np.copy(positions)
+    period = 0
+    for iteration in range(iterations):
+        print(f"\nBegin Iteration {iteration} of Simulation {sim_num} of {title}") if console else None
+        explore_t = ones if iteration else np.zeros((agents, 1))
+        x_new, y_new, id_new = _take_samples(agents, positions, explore_t, truth_arr, sigma_n, noise_rng, console,
+                                             centroids_t, iteration, sim.index_of())
+        distance = np.sqrt(np.sum((positions - prev_positions) ** 2, axis=1)).reshape(-1, 1)
+        if fidelity == "S":
+            model.updt(x_new, y_new)
+        else:
+            model.updt_hifi(x_new, y_new)
+        loss_t, _, argmax_var_t, max_var_t, _, lloyd_vor = sim.step(model, positions, positions)
+        if len(lloyd_vor) != agents:
+            raise ValueError("thompson: every agent must lie inside the cushioned bounding box")
+        normals = rng.standard_normal((model.grid_sample_dim(sim.grid), agents))
+        _, cen = sim.grid.sample_centroids(model, lloyd_vor, torch.from_numpy(normals).to(sim.grid.device),
+                                           bbox=tuple(sim.bounding_box))
+        centroids_t = cen.cpu().numpy()[np.arange(agents), np.arange(agents)]      # agent i: its own cell under draw i
+        _console(console, period, fidelity, loss_t, max_var_t, max_var_0, ones, ones, iteration)
+        _log_rows(log, loss_log, agent_log, sample_log, sim_num, iteration, period, fidelity, agents, positions,
+                  argmax_var_t, max_var_t, max_var_0, centroids_t, ones, ones, distance, loss_t, id_new, x_new, y_new)
+        prev_positions = np.copy(positions)
+        positions[...] = snap_to_grid(centroids_t, prev_positions, ux, uy)
+    return loss_log, agent_log, sample_log
 
 
 def run_batched(algo, sim_nums, iterations, agents, positions, truth, sigma_n, prior, hyp, uniforms=None, noise=None,

@@ -442,7 +442,7 @@ int choi_shard_status(int64_t G, int64_t cap, const void* work, int64_t work_byt
  * Logs: log_loss[iterations], log_agent[iterations, A, 11] (X, Y, XMax, YMax, VarMax, Var0, XCentroid, YCentroid, ProbExplore,
  * Explore, Distance: the reference's agent row), log_sample[max_samples, 5] (Iteration, Agent, X, Y, Sample). */
 typedef struct mfgp_batch {
-    int64_t runs, G, nx, ny, A, NL, cap, algo /* 0 lloyd, 1 periodic, 2 todescato, 3 choi */, iterations, max_samples;
+    int64_t runs, G, nx, ny, A, NL, cap, algo /* 0 lloyd, 1 periodic, 2 todescato, 3 choi, 4 thompson */, iterations, max_samples;
     double xmin, xmax, ymin, ymax, eps, tie_tol, amax_rel;
     const double* xy; const double* f; const double* ux; const double* uy;
     double* Xt; double* y; double* W; double* z;
@@ -462,6 +462,17 @@ typedef struct mfgp_batch {
      * tour_cur[runs*A] (next entry to visit). */
     double* q; int64_t* picks; int32_t* nplan; int32_t* plan_state; int32_t* pmask; int32_t* ccount; int32_t* cties;
     int32_t* tour_off; int32_t* tour_cur; int64_t* tour;
+    /* Thompson only (algo 4; NULL / 0 otherwise).  seed[runs]: the run's draw seed (64 bits).  Written by the coverage step:
+     * cmask[G] (membership bit mask of every grid point in the cells seeded by the positions, bit c = agent c),
+     * ccell[A][2] (point count and area of each of those cells), rowidx[cap] (grid index of training row n, -1 for the
+     * off-grid prior rows, which the caller sets).  The pathwise sampler's plan of the shared initial model (the box covers
+     * the grid and the prior points and stays fixed, every later training point being a grid point): orders rxL, ryL, rxH,
+     * ryH (lofi orders 0 for a single-fidelity model), box [bxlo, bxhi] x [bylo, byhi], node roots QxL[rxL][rxL],
+     * QyL[ryL][ryL], QxH[rxH][rxH], QyH[ryH][ryH] (as mfgp_grid_sample_coef takes them). */
+    const int64_t* seed; uint16_t* cmask; double* ccell; int32_t* rowidx;
+    int64_t rxL, ryL, rxH, ryH;
+    double bxlo, bxhi, bylo, byhi;
+    const double* QxL; const double* QyL; const double* QxH; const double* QyH;
 } mfgp_batch;
 
 /* One iteration of every run: take the exploring agents' samples (:698-713), append them to the model by a block-bordered
@@ -492,6 +503,23 @@ int mfgp_batch_choi_cluster(const mfgp_batch* b_host, void* stream);
  * into ord[n_total] (work / work_bytes: as choi_tsp_tours), and stored as grid indices in b->tour; tour_cur = tour_off. */
 int mfgp_batch_choi_tours(const mfgp_batch* b_host, int64_t n_total, int64_t n_max, double* pts, int64_t* gidx, int32_t* ord,
                           void* work, int64_t work_bytes, void* stream);
+
+/* ---- batched Thompson sampling (algo 4): the draw stage of simulator.thompson for every run, after mfgp_batch_step ---------
+ * Per run r and draw s = agent i, the joint posterior draw over the whole grid that mfgp_grid_sample_coef defines,
+ *   F_s(g) = mu(g) + f_s(g) - k(g, X) beta_s,   beta_s = W^T W (f_s(X) + sqrt(noise + jitter) eta_s),
+ * with f_s the Chebyshev-node prior draw of the plan in the batch struct, mu the stepper's standing posterior mean and
+ * k(g, X) read from its axis tables.  Only the statistics sum F_i {1, x, y} over cell i (cmask) are formed; the target of
+ * agent i is cov_finish's centroid of them (NaN for an empty cell), snapped to the grid in agent order as
+ * simulator.snap_to_grid does.  The move sets pos, pos_idx, prev and cen (= the unsnapped target) and the log's XCentroid /
+ * YCentroid.  The normals are generated on the device by a counter-based generator (Philox4x32-10 keyed by the run's seed,
+ * counter (row, agent, iteration, 0), one Box-Muller normal per counter); rows follow mfgp_grid_sample_coef's layout at
+ * the run's training-set size: a run's normals depend on its seed only.  `iteration` must be the one just stepped.
+ * work: mfgp_batch_thompson_workspace_bytes(b_host) bytes. */
+int64_t mfgp_batch_thompson_workspace_bytes(const mfgp_batch* b_host);
+int mfgp_batch_thompson(const mfgp_batch* b_host, const mfgp_params* p_host, int64_t iteration, void* work, int64_t work_bytes,
+                        void* stream);
+/* The normals the draw stage of `iteration` uses for rows [0, rows) of every run: out[runs][rows][A]. */
+int mfgp_batch_thompson_normals(const mfgp_batch* b_host, int64_t iteration, int64_t rows, double* out, void* stream);
 
 /* ---- hyper-parameter training: replaces SFGP.likelihood / MFGP.likelihood gaussian_process.py:81-105, :344-384 and the
  *      autograd gradient behind SFGP.train / MFGP.train :107-119, :386-399 ------------------------------------------- */

@@ -22,8 +22,20 @@ agent's tour has points left).  The buffers grow between pick rounds when a run'
 lies within TIE_TOL/10 of a bisector of the centroid cells (which agent visits it is then decided by Qhull's vertex
 rounding in the single-run path) makes the run's result depend on Qhull: such runs are re-run on the single-run path with
 the same start positions and noise draws (`tie_reruns`).
+
+Thompson sampling (simulator.thompson) runs whole on the device: after each iteration's step, a draw stage
+(`mfgp_batch_thompson`, csrc/batched_thompson.cu) takes one joint posterior draw per agent over the whole grid, reduces
+agent i's draw over agent i's cell to its centroid and moves the agents to their snapped targets.  The draws' normals come
+from a counter-based generator on the device keyed by each run's 64-bit seed (`seeds`; default: one
+random.getrandbits(64) per run, which is what simulator.thompson seeds its numpy Generator with).  They are NOT the numpy
+stream simulator.thompson draws from the same seed; `draw_normals(t)` returns the ones a run used at iteration t.
+Parity contract: a batched Thompson run equals simulator.thompson run with simulator.VORONOI = "clip" at equal normals
+(an `rng` whose standard_normal returns draw_normals) and equal noise.  Agents sit on grid points, and on uniform grids
+grid points lie exactly on the bisectors between them: under the default VORONOI = "auto", simulator.thompson passes those
+iterations again on Qhull's polygons, which the device loop does not follow, so the two differ at such grid points only.
 """
 import ctypes
+import random
 
 import numpy as np
 import torch
@@ -32,7 +44,7 @@ from . import _coverage as cv
 from . import _native as nat
 from .gaussian_process import evaluate_hyp, prior_variance
 
-ALGOS = {"lloyd": 0, "periodic": 1, "todescato": 2, "choi": 3}
+ALGOS = {"lloyd": 0, "periodic": 1, "todescato": 2, "choi": 3, "thompson": 4}
 LOG_COLS = ("X", "Y", "XMax", "YMax", "VarMax", "Var0", "XCentroid", "YCentroid", "ProbExplore", "Explore", "Distance")
 CHOI_ROUNDS = 16          # planner pick rounds launched between two reads of the runs' planning state
 CHOI_GROW = 32            # training rows added per run when a planner reaches the capacity
@@ -40,6 +52,8 @@ BUFFER_NAMES = ("xy", "f", "ux", "uy", "Xt", "y", "W", "z", "TxL", "TyL", "TxH",
                 "pos_idx", "prob", "explore", "Ncur", "knew", "status", "noise_used", "nsamples", "ties", "noise", "unif",
                 "log_loss", "log_agent", "log_sample")
 CHOI_BUFFER_NAMES = ("q", "picks", "nplan", "plan_state", "pmask", "ccount", "cties", "tour_off", "tour_cur", "tour")
+THOMPSON_BUFFER_NAMES = ("seed", "cmask", "ccell", "rowidx", "QxL", "QyL", "QxH", "QyH")
+APPEND_STAGING_BYTES = 200 * 1024      # shared-memory staging of the sample append (mfgp_batch_step): 2 A cap doubles
 
 
 def choi_schedule(iterations):
@@ -67,13 +81,13 @@ class _NoiseRow:
 
 class BatchedRuns:
     def __init__(self, algo, truth_arr, prior_arr, hyp, agents, iterations, positions0, sigma_n=0.1, uniforms=None, noise=None,
-                 noise_rngs=None, raw_means=False, device=None, cap=None):
-        """algo: "lloyd" | "periodic" | "todescato" | "choi".  positions0[R, A, 2]: start positions of the R runs.
+                 noise_rngs=None, raw_means=False, device=None, cap=None, seeds=None):
+        """algo: "lloyd" | "periodic" | "todescato" | "choi" | "thompson".  positions0[R, A, 2]: start positions of the R runs.
         uniforms[R, iterations, A]: todescato's Bernoulli draws (random.random(), simulator.py:943), in consumption order.
         noise[R, iterations * A]: the N(0, sigma_n) sample noise in consumption order -- or `noise_rngs`, one numpy Generator
         per run, from which it is drawn here (the reference draws one normal per sample, :707).  Choi logs
         len(choi_schedule(iterations)) iterations and needs that many times A draws.  cap (Choi): initial training rows per
-        run; the buffers grow when the planner needs more."""
+        run; the buffers grow when the planner needs more.  seeds[R] (Thompson): the runs' 64-bit draw seeds."""
         from . import simulator as sim
         from ._engine import TensorAxes, detect_tensor_grid
         nat.require_cuda()
@@ -93,6 +107,8 @@ class BatchedRuns:
         if A != agents or A > 16:
             raise ValueError("positions0 must be [runs, agents, 2] with at most 16 agents")
         G, nx, ny, T = xy.shape[0], len(ux), len(uy), int(iterations)
+        if self.code == 4:
+            box = self._thompson_checks(xy, positions0, prior_arr, hyp, raw_means, T)
         self.iterations, self.positions0 = T, positions0.copy()
         if self.code == 3:
             self.period = choi_schedule(T)
@@ -133,6 +149,10 @@ class BatchedRuns:
             eng.ensure_factor(need_inverse=True)
             eng.check_factor(force=True)
             cap = -(-(N0 + T * A) // 8) * 8
+            if self.code == 4:              # iteration 0 takes no samples
+                cap = max(-(-(N0 + (T - 1) * A) // 8) * 8, 8)
+                self.splan = eng._grid_sample_plan(grid.axes)
+                assert self.splan["box"] == box and self.splan["orders"] == self._orders      # fixed: later samples are grid points
             if self.code == 3:
                 cap = -(-max(N0 + CHOI_GROW if cap_arg is None else int(cap_arg), N0 + 1) // 8) * 8
             k0 = prior_variance(self.params)
@@ -201,13 +221,55 @@ class BatchedRuns:
             self.tour = torch.zeros(1, dtype=torch.int64, device=self.dev)
             self.cluster_ties = np.zeros((R, int(self.period[-1]) + 1 if T else 0), dtype=np.int64)
             self.phase_ms = {"plan": 0.0, "cluster_tours": 0.0, "step": 0.0}
+        if self.code == 4:
+            seeds = [random.getrandbits(64) for _ in range(R)] if seeds is None else seeds
+            self.seeds = np.asarray(seeds, dtype=np.uint64).reshape(R)
+            self.seed = t(self.seeds.view(np.int64))
+            self.cmask = torch.zeros((R, G), dtype=torch.int16, device=self.dev)
+            self.ccell = z(R, A, 2)
+            self.rowidx = torch.full((R, cap), -1, dtype=torch.int32, device=self.dev)
+            Q = self.splan["Q"]
+            self.QxL, self.QyL = Q.get("Lx", Q["Hx"]), Q.get("Ly", Q["Hy"])
+            self.QxH, self.QyH = Q["Hx"], Q["Hy"]
+            b.rxL, b.ryL, b.rxH, b.ryH = self.splan["orders"]
+            b.bxlo, b.bxhi, b.bylo, b.byhi = self.splan["box"]
+            self.d0 = int(self.splan["d0"])
         self._bind()
+        if self.code == 4:
+            self.work = torch.empty(int(nat.lib().mfgp_batch_thompson_workspace_bytes(ctypes.byref(b))) // 8, **f64)
 
     def _bind(self):
         b = self._b
         b.cap = self.cap
-        for name in BUFFER_NAMES + (CHOI_BUFFER_NAMES if self.code == 3 else ()):
+        for name in BUFFER_NAMES + (CHOI_BUFFER_NAMES if self.code == 3 else ()) + \
+                (THOMPSON_BUFFER_NAMES if self.code == 4 else ()):
             setattr(b, name, getattr(self, name).data_ptr())
+
+    def _thompson_checks(self, xy, positions0, prior_arr, hyp, raw_means, T):
+        """The errors of a Thompson batch, raised before anything is launched.  Returns the sampler's box: the grid and the
+        prior points.  It stays fixed for the whole run, because every later training point is a grid point."""
+        from . import simulator as sim
+        from ._engine import grid_sample_orders
+        bb = np.array([xy[:, 0].min(), xy[:, 0].max(), xy[:, 1].min(), xy[:, 1].max()])
+        for p in positions0:
+            if not np.all(cv.in_box(p, bb)):
+                raise ValueError("thompson: every agent must lie inside the cushioned bounding box")
+        X0 = sim._prior_arrays(prior_arr)[0]
+        A, N0 = positions0.shape[1], X0.shape[0]
+        cap = -(-(N0 + (T - 1) * A) // 8) * 8
+        if 2 * A * cap * 8 > APPEND_STAGING_BYTES:
+            raise ValueError(f"a batched Thompson run needs {cap} training rows, more than the stepper's sample append can stage "
+                             f"with {A} agents ({APPEND_STAGING_BYTES // (16 * A)} rows); run this experiment with "
+                             "simulator.thompson")
+        box = (float(bb[0]), float(bb[1]), float(bb[2]), float(bb[3]))
+        if N0:
+            box = (min(box[0], float(X0[:, 0].min())), max(box[1], float(X0[:, 0].max())),
+                   min(box[2], float(X0[:, 1].min())), max(box[3], float(X0[:, 1].max())))
+        h = np.asarray(hyp.values.tolist()[0] if hasattr(hyp, "values") else hyp, dtype=np.float64).reshape(-1)
+        p = evaluate_hyp(h, raw_means)
+        o = grid_sample_orders(p, box)
+        self._orders = (o.get("Lx", 0), o.get("Ly", 0), o["Hx"], o["Hy"])
+        return box
 
     def _grow(self, cap):
         """Choi: room for `cap` training rows per run (the rows in use and the factor are copied over)."""
@@ -230,6 +292,22 @@ class BatchedRuns:
     def step(self, it):
         nat.check(nat.lib().mfgp_batch_step(ctypes.byref(self._b), ctypes.byref(self.pstruct), int(it), nat.stream_ptr()),
                   "mfgp_batch_step")
+        if self.code == 4:
+            nat.check(nat.lib().mfgp_batch_thompson(ctypes.byref(self._b), ctypes.byref(self.pstruct), int(it),
+                                                    nat.ptr(self.work), self.work.numel() * 8, nat.stream_ptr()),
+                      "mfgp_batch_thompson")
+
+    def draw_normals(self, t):
+        """Thompson: the standard normals the draw stage of iteration t used, [R, d_t, A] (float64, device), in the layout of
+        mfgp_grid_sample_coef's normals at the run's training-set size N0 + A t: row d of run r is what
+        simulator.thompson's `rng.standard_normal((d_t, A))` returns at iteration t of an equal run."""
+        if self.code != 4:
+            raise ValueError("draw_normals: only Thompson runs draw normals on the device")
+        rows = self.d0 + self.N0 + self.A * int(t)
+        out = torch.empty((self.R, rows, self.A), dtype=torch.float64, device=self.dev)
+        nat.check(nat.lib().mfgp_batch_thompson_normals(ctypes.byref(self._b), int(t), rows, nat.ptr(out), nat.stream_ptr()),
+                  "mfgp_batch_thompson_normals")
+        return out
 
     def plan(self, threshold):
         """Choi, every run: greedy picks on the run's own factor until its max variance is <= threshold

@@ -124,6 +124,23 @@ def node_root(length, lo, hi, r):
     return np.ascontiguousarray(dct @ ((V * np.sqrt(np.maximum(lam, 0.0))) @ V.T))
 
 
+def grid_sample_orders(p, box):
+    """Chebyshev orders {"Lx", "Ly" (multi-fidelity only), "Hx", "Hy"} of the pathwise grid sampler on `box` (xlo, xhi, ylo,
+    yhi) for the evaluated parameters `p`.  ValueError when the box spans no area or an order would exceed 64."""
+    if not (box[1] > box[0] and box[3] > box[2]):
+        raise ValueError("sample_posterior_grid: the grid and the training points span no area; use sample_posterior")
+    orders = {}
+    for part, length in ((("L", p["l_L"]), ("H", p["l_H"])) if p["multi"] else (("H", p["l_H"]),)):
+        for ax, lo, hi in (("x", box[0], box[1]), ("y", box[2], box[3])):
+            r = chebyshev_order(length, lo, hi, lo, hi)
+            if r is None:
+                raise ValueError(f"sample_posterior_grid: length scale {length:.4g} needs more than 64 Chebyshev terms over "
+                                 f"[{lo:.4g}, {hi:.4g}]; draw at point sets of up to {DeviceGP.SAMPLE_MAX_G} points with "
+                                 "sample_posterior instead")
+            orders[part + ax] = r
+    return orders
+
+
 def params_struct(p):
     """p: dict with the evaluated parameters (see gaussian_process.evaluate_hyp)."""
     return nat.MfgpParams(p["s_L"], p["l_L"], p["s_H"], p["l_H"], p["rho"], p["noise_L"], p["noise_H"],
@@ -546,19 +563,12 @@ class DeviceGP:
         key = (axes.uid, box, p["l_L"], p["l_H"], int(p["multi"]))
         if self._splan is not None and self._splan["key"] == key:
             return self._splan
-        if not (box[1] > box[0] and box[3] > box[2]):
-            raise ValueError("sample_posterior_grid: the grid and the training points span no area; use sample_posterior")
+        orders = grid_sample_orders(p, box)
         f64 = dict(dtype=torch.float64, device=self.device)
-        Q, orders = {}, {}
+        Q = {}
         for part, length in ((("L", p["l_L"]), ("H", p["l_H"])) if p["multi"] else (("H", p["l_H"]),)):
             for ax, lo, hi in (("x", box[0], box[1]), ("y", box[2], box[3])):
-                r = chebyshev_order(length, lo, hi, lo, hi)
-                if r is None:
-                    raise ValueError(f"sample_posterior_grid: length scale {length:.4g} needs more than 64 Chebyshev terms over "
-                                     f"[{lo:.4g}, {hi:.4g}]; draw at point sets of up to {self.SAMPLE_MAX_G} points with "
-                                     "sample_posterior instead")
-                orders[part + ax] = r
-                Q[part + ax] = torch.from_numpy(node_root(length, lo, hi, r)).to(**f64)
+                Q[part + ax] = torch.from_numpy(node_root(length, lo, hi, orders[part + ax])).to(**f64)
         rxL, ryL = orders.get("Lx", 0), orders.get("Ly", 0)
         rxH, ryH = orders["Hx"], orders["Hy"]
         self._splan = dict(key=key, box=box, orders=(rxL, ryL, rxH, ryH), Q=Q, d0=rxL * ryL + rxH * ryH,

@@ -31,7 +31,10 @@ class MfgpBatch(Structure):      # struct mfgp_batch (include/mfgp_b200.h)
                                         "prev", "cen", "pos_idx", "prob", "explore", "Ncur", "knew", "status", "noise_used",
                                         "nsamples", "ties", "noise", "unif", "log_loss", "log_agent", "log_sample",
                                         "q", "picks", "nplan", "plan_state", "pmask", "ccount", "cties", "tour_off", "tour_cur",
-                                        "tour")]
+                                        "tour", "seed", "cmask", "ccell", "rowidx")] + \
+               [(n, c_int64) for n in ("rxL", "ryL", "rxH", "ryH")] + \
+               [(n, c_double) for n in ("bxlo", "bxhi", "bylo", "byhi")] + \
+               [(n, c_void_p) for n in ("QxL", "QyL", "QxH", "QyH")]
 
 
 # name -> (restype, argtypes); this table is also what tests/test_abi.py checks against include/mfgp_b200.h
@@ -167,6 +170,9 @@ SIGNATURES = {
     "mfgp_batch_choi_cluster": (c_int, [POINTER(MfgpBatch), c_void_p]),
     "mfgp_batch_choi_tours": (c_int, [POINTER(MfgpBatch), c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int64,
                                       c_void_p]),
+    "mfgp_batch_thompson_workspace_bytes": (c_int64, [POINTER(MfgpBatch)]),
+    "mfgp_batch_thompson": (c_int, [POINTER(MfgpBatch), POINTER(MfgpParams), c_int64, c_void_p, c_int64, c_void_p]),
+    "mfgp_batch_thompson_normals": (c_int, [POINTER(MfgpBatch), c_int64, c_int64, c_void_p, c_void_p]),
     "mfgp_nlml_workspace_bytes": (c_int64, [c_int64]),
     "mfgp_nlml_grad": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_int64, c_int64,
                                POINTER(MfgpParams), c_void_p, c_void_p, c_int64, c_void_p]),

@@ -24,41 +24,11 @@
 // vertex rounding -- those (run, iteration) pairs are counted in `ties` for the host to re-evaluate if it needs them bit-exact.
 #include <cfloat>
 
-#include "common.cuh"
 #include "argmax.cuh"
+#include "batched.cuh"
 #include "cov_device.cuh"
 
 namespace mfgp {
-
-constexpr int BT_THREADS = 256;
-constexpr int BT_MAXA = 16;          // agents per run
-constexpr int BT_LOGC = 11;          // X, Y, XMax, YMax, VarMax, Var0, XCentroid, YCentroid, ProbExplore, Explore, Distance
-
-struct BatchArgs {
-    int runs, G, nx, ny, A, NL, cap, algo, iterations, max_samples;      // algo: 0 lloyd, 1 periodic, 2 todescato
-    double xmin, xmax, ymin, ymax, eps, tie_tol, amax_rel;
-    DevParams p;
-    const double* xy; const double* f; const double* ux; const double* uy;
-    double* Xt; double* y; double* W; double* z;                         // [runs][cap(,2 | ,cap)]
-    double* TxL; double* TyL; double* TxH; double* TyH;                  // [runs][cap][nx | ny]
-    double* mu; double* var;                                             // [runs][G]
-    double* pos; double* prev; double* cen;                              // [runs][A][2]
-    long long* pos_idx;                                                  // [runs][A] grid index of the position, or -1
-    double* prob; int* explore;                                          // [runs][A]
-    int* Ncur; int* knew; int* status; int* noise_used; int* nsamples;   // [runs]
-    int* ties;                                                           // [runs][iterations]
-    const double* noise; const double* unif;                             // [runs][max_samples], [runs][iterations][A]
-    double* log_loss; double* log_agent; double* log_sample;             // [runs][it], [runs][it][A][BT_LOGC], [runs][max_samples][5]
-    double* q; long long* picks; int* nplan; int* plan_state;            // Choi planner: [runs][G], [runs][cap], [runs], [runs]
-    int* pmask; int* ccount; int* cties;                                 // Choi clusters: [runs][cap], [runs][A], [runs]
-    int* tour_off; int* tour_cur; long long* tour;                       // Choi tours: [runs*A+1], [runs*A], [tour_off[runs*A]]
-};
-
-__device__ __forceinline__ double warp_sum_d(double v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
 
 // training covariance entry between a NEW hifi point (x, y) and training point n of the run -- the operations of
 // build_train_cov_kernel (gp_fit.cu), i.e. of gaussian_process.py:523-528 / :253
@@ -357,7 +327,12 @@ __global__ void __launch_bounds__(BT_THREADS) batch_coverage_kernel(BatchArgs a,
     double* pos = a.pos + (int64_t)r * A * 2;
     double* prev = a.prev + (int64_t)r * A * 2;
     double* cen = a.cen + (int64_t)r * A * 2;
-    if (tid < 2 * A) { s_seed[0][tid >> 1][tid & 1] = cen[tid]; s_seed[1][tid >> 1][tid & 1] = pos[tid]; }
+    const bool thompson = a.algo == 4;          // both partitions seeded by the positions; the draw stage moves the agents
+    if (tid < 2 * A) { s_seed[0][tid >> 1][tid & 1] = thompson ? pos[tid] : cen[tid]; s_seed[1][tid >> 1][tid & 1] = pos[tid]; }
+    if (thompson) {          // grid index of the training rows this iteration appended (every agent samples, in agent order)
+        const int q = a.knew[r];
+        if (tid < q) a.rowidx[(int64_t)r * a.cap + a.Ncur[r] - q + tid] = (int)a.pos_idx[r * A + tid];
+    }
     if (tid == 0) { s_ties = 0; s_bad = 0; }
     __syncthreads();
     // bounded Voronoi cells of both partitions: the box inflated by eps/2 clipped by the bisectors (simulator.py:154-191)
@@ -413,6 +388,7 @@ __global__ void __launch_bounds__(BT_THREADS) batch_coverage_kernel(BatchArgs a,
                     if (crossings_inside(s_poly[part][c], s_cnt[part][c], x, y)) mask |= 1u << c;
             }
             s_mask[part * a.G + g] = (unsigned short)mask;
+            if (thompson && part == 0) a.cmask[(int64_t)r * a.G + g] = (unsigned short)mask;
         }
     }
     if (hard) atomicAdd(&s_ties, hard);
@@ -471,6 +447,14 @@ __global__ void __launch_bounds__(BT_THREADS) batch_coverage_kernel(BatchArgs a,
         double* row = a.log_agent + (((int64_t)r * a.iterations + it) * A + i) * BT_LOGC;
         row[0] = px; row[1] = py; row[2] = axm; row[3] = py; row[4] = mv; row[5] = with_var ? a.p.k0 : 0.0;
         row[6] = cx; row[7] = cy; row[8] = a.prob[r * A + i]; row[9] = (double)a.explore[r * A + i]; row[10] = dist;
+        if (thompson) {          // every agent samples from the next iteration on; the draw stage fills XCentroid / YCentroid
+            row[8] = 1.0; row[9] = 1.0;
+            a.prob[r * A + i] = 1.0;
+            a.explore[r * A + i] = 1;
+            a.ccell[((int64_t)r * A + i) * 2] = n;
+            a.ccell[((int64_t)r * A + i) * 2 + 1] = ar;
+            return;
+        }
         int ex = 0;
         double pr = 0.0;
         long long tgi = -1;
@@ -503,15 +487,6 @@ __global__ void __launch_bounds__(BT_THREADS) batch_coverage_kernel(BatchArgs a,
 // unchanged and the next real sample overwrites the row.  The planner's variance is k0 - q with q = |W psi|^2 accumulated from
 // a recomputation at the period start, never the stepper's decremented var: far from the data q ~ ulp(k0), and the first
 // index of the top 1-ulp plateau is what the reference picks (argmax.cuh).
-
-// cross-covariance of training row n of run r with grid point (ix, iy), from the axis tables (batch_posterior_kernel)
-__device__ __forceinline__ double bt_psi(const BatchArgs& a, int r, int n, int ix, int iy) {
-    const int64_t t = (int64_t)r * a.cap + n;
-    double psi = 0.0;
-    if (n >= a.NL) psi = a.p.s_H * (a.TxH[t * a.nx + ix] * a.TyH[t * a.ny + iy]);
-    if (a.p.multi) psi = fma(n < a.NL ? a.p.rho * a.p.s_L : a.p.rho2 * a.p.s_L, a.TxL[t * a.nx + ix] * a.TyL[t * a.ny + iy], psi);
-    return psi;
-}
 
 constexpr int CQ_ROWS = 8;
 
@@ -736,24 +711,13 @@ __global__ void batch_choi_order_kernel(BatchArgs a, const long long* gidx, cons
     for (int t = o0; t < o1; t++) a.tour[t] = gidx[o0 + ord[t]];
 }
 
-}  // namespace mfgp
-
-using namespace mfgp;
-
-// Layout of the caller-provided state block (doubles unless noted), per run r and in this order:
-//   Xt[cap*2] y[cap] W[cap*cap] z[cap] TxL[cap*nx] TyL[cap*ny] TxH[cap*nx] TyH[cap*ny] mu[G] var[G] pos[2A] prev[2A] cen[2A]
-//   prob[A] | int64: pos_idx[A] | int32: explore[A] Ncur knew status noise_used nsamples ties[iterations]
-// (the host module mfgp-coverage_b200/_batched.py owns the buffers; this file only receives pointers)
-extern "C" {
-
-/* struct mfgp_batch: include/mfgp_b200.h */
-
-static bool batch_valid(const mfgp_batch* b, const mfgp_params* p_host) {
+bool batch_valid(const mfgp_batch* b, const mfgp_params* p_host) {
     return b && p_host && b->runs > 0 && b->A > 0 && b->A <= BT_MAXA && b->G > 0 && b->nx * b->ny == b->G && b->cap > 0 &&
-           b->algo >= 0 && b->algo <= 3 && (b->algo != 3 || (b->tour_off && b->tour_cur));
+           b->algo >= 0 && b->algo <= 4 && (b->algo != 3 || (b->tour_off && b->tour_cur)) &&
+           (b->algo != 4 || (b->seed && b->cmask && b->ccell && b->rowidx));
 }
 
-static BatchArgs batch_args(const mfgp_batch* b, const mfgp_params* p_host) {
+BatchArgs batch_args(const mfgp_batch* b, const mfgp_params* p_host) {
     BatchArgs a{};
     a.runs = (int)b->runs; a.G = (int)b->G; a.nx = (int)b->nx; a.ny = (int)b->ny; a.A = (int)b->A; a.NL = (int)b->NL;
     a.cap = (int)b->cap; a.algo = (int)b->algo; a.iterations = (int)b->iterations; a.max_samples = (int)b->max_samples;
@@ -768,8 +732,22 @@ static BatchArgs batch_args(const mfgp_batch* b, const mfgp_params* p_host) {
     a.q = b->q; a.picks = reinterpret_cast<long long*>(b->picks); a.nplan = b->nplan; a.plan_state = b->plan_state;
     a.pmask = b->pmask; a.ccount = b->ccount; a.cties = b->cties; a.tour_off = b->tour_off; a.tour_cur = b->tour_cur;
     a.tour = reinterpret_cast<long long*>(b->tour);
+    a.seed = reinterpret_cast<const long long*>(b->seed); a.cmask = reinterpret_cast<unsigned short*>(b->cmask); a.ccell = b->ccell;
+    a.rowidx = b->rowidx;
     return a;
 }
+
+}  // namespace mfgp
+
+using namespace mfgp;
+
+// Layout of the caller-provided state block (doubles unless noted), per run r and in this order:
+//   Xt[cap*2] y[cap] W[cap*cap] z[cap] TxL[cap*nx] TyL[cap*ny] TxH[cap*nx] TyH[cap*ny] mu[G] var[G] pos[2A] prev[2A] cen[2A]
+//   prob[A] | int64: pos_idx[A] | int32: explore[A] Ncur knew status noise_used nsamples ties[iterations]
+// (the host module mfgp-coverage_b200/_batched.py owns the buffers; this file only receives pointers)
+extern "C" {
+
+/* struct mfgp_batch: include/mfgp_b200.h */
 
 int mfgp_batch_step(const mfgp_batch* b, const mfgp_params* p_host, int64_t iteration, void* stream) {
     if (!batch_valid(b, p_host) || iteration < 0 || iteration >= b->iterations) return MFGP_ERR_INVALID;

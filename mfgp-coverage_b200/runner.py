@@ -52,10 +52,11 @@ def run_sim(args):
 
 
 # MFGP_BATCHED=1 (or runner.BATCHED = True, or run(batched=True)): the replicate simulations of lloyd / periodic / todescato /
-# choi experiments are stepped TOGETHER on the device (simulator.run_batched: three kernel launches advance every run by one
-# iteration; Choi plans all runs' tours on the device once per period) instead of one host loop per simulation.  The random
-# streams are consumed exactly as the sequential loop consumes them: per simulation the 2 A start coordinates, then
-# (todescato) one uniform per agent and iteration.
+# choi / thompson experiments are stepped TOGETHER on the device (simulator.run_batched: three kernel launches advance every
+# run by one iteration; Choi plans all runs' tours on the device once per period; Thompson adds its draw stage) instead of
+# one host loop per simulation.  The random streams are consumed exactly as the sequential loop consumes them: per
+# simulation the 2 A start coordinates, then (todescato) one uniform per agent and iteration, or (thompson) the one
+# random.getrandbits(64) that seeds the run's draws.
 BATCHED = os.environ.get("MFGP_BATCHED", "0") == "1"
 BATCH_RUNS = 512          # simulations per device batch (state: ~4 MB per run at 64x64 points, 520 samples)
 
@@ -63,7 +64,8 @@ BATCH_RUNS = 512          # simulations per device batch (state: ~4 MB per run a
 def _batchable(args):
     algos = {a[1] for a in args}
     return len(args) > 1 and len(algos) == 1 and \
-        any(k in next(iter(algos)) for k in ("choi", "todescato", "lloyd", "periodic")) and all(a[10] is None for a in args)
+        any(k in next(iter(algos)) for k in ("choi", "todescato", "lloyd", "periodic", "thompson")) and \
+        all(a[10] is None for a in args)
 
 
 def run_sims_batched(args):
@@ -73,17 +75,20 @@ def run_sims_batched(args):
     for b0 in range(0, len(args), BATCH_RUNS):
         chunk = args[b0:b0 + BATCH_RUNS]
         (_, algo, _, iterations, agents, truth, sigma_n, prior, hyp, _, _, _) = chunk[0]
-        pos, unif = [], []
-        for a in chunk:                                   # the draws of run_sim (:41-43) and of todescato (:943), in order
+        pos, unif, seeds = [], [], []
+        thompson = not any(k in algo for k in ("choi", "todescato", "lloyd", "periodic"))
+        for a in chunk:                                   # the draws of run_sim (:41-43), todescato (:943) and thompson, in order
             x_positions = [random.random() for i in range(agents)]
             y_positions = [random.random() for i in range(agents)]
             pos.append(np.column_stack((x_positions, y_positions)))
             if "todescato" in algo and "choi" not in algo:
                 unif.append([[random.random() for i in range(agents)] for t in range(iterations)])
+            if thompson:
+                seeds.append(random.getrandbits(64))
         print(line_break + f"Start Simulations {chunk[0][2]}..{chunk[-1][2]} : {algo} (batched)" + line_break)
         sim_start = time.time()
         logs = run_batched(algo, [a[2] for a in chunk], iterations, agents, np.array(pos), truth, sigma_n, prior, hyp,
-                           uniforms=np.array(unif) if unif else None)
+                           uniforms=np.array(unif) if unif else None, seeds=seeds if thompson else None)
         print(line_break + f"End Simulations : {algo}\nTime : {time.time() - sim_start}" + line_break)
         out.extend(logs)
     return out

@@ -765,25 +765,28 @@ def thompson(title, sim_num, iterations, agents, positions, truth, sigma_n, prio
 
 
 def run_batched(algo, sim_nums, iterations, agents, positions, truth, sigma_n, prior, hyp, uniforms=None, noise=None,
-                noise_rngs=None, exact_tie_loss=False, use_graph=False):
+                noise_rngs=None, exact_tie_loss=False, use_graph=False, seeds=None):
     """Many independent runs of ONE experiment stepped together on the device (config c5, the replicate sweeps of
-    runner.py:100, :131-147): `algo` names lloyd, periodic, todescato or choi (as runner.run_sim dispatches), `positions[R, A,
+    runner.py:100, :131-147): `algo` names lloyd, periodic, todescato, choi or thompson (as runner.run_sim dispatches), `positions[R, A,
     2]` the runs' start positions (updated in place to the final ones, like the single-run functions do).  Returns a list of R
     (loss_log, agent_log, sample_log) triples with the reference's row schemas.  See _batched.BatchedRuns for the
     random-number and tie conventions; `exact_tie_loss=True` re-evaluates the losses that involve exact bisector ties with
-    Qhull cells.  Choi runs come back to the host once per period, so `use_graph` is not available for them."""
+    Qhull cells.  Choi runs come back to the host once per period, so `use_graph` is not available for them.  `seeds[R]`
+    (thompson): the runs' 64-bit draw seeds; the draws themselves come from a generator on the device, so a batched run equals
+    thompson(..., VORONOI "clip") at the normals BatchedRuns.draw_normals returns, not at a numpy stream of the same seed."""
     from ._batched import BatchedRuns
     kind = "choi" if "choi" in algo else ("todescato" if "todescato" in algo else ("lloyd" if "lloyd" in algo else
-                                          ("periodic" if "periodic" in algo else None)))
+                                          ("periodic" if "periodic" in algo else ("thompson" if "thompson" in algo else None))))
     if kind is None:
-        raise ValueError("run_batched supports lloyd, periodic, todescato and choi")
+        raise ValueError("run_batched supports lloyd, periodic, todescato, choi and thompson")
     if kind == "choi" and use_graph:
         raise ValueError("Choi runs return to the host once per period: use_graph is not available for them")
     truth_arr = np.vstack(truth.values.tolist()) if hasattr(truth, "values") else np.asarray(truth, dtype=np.float64)
     prior_arr = None
     if prior is not None and len(prior) > 0:
         prior_arr = np.vstack(prior.values.tolist()) if hasattr(prior, "values") else np.asarray(prior, dtype=np.float64)
-    br = BatchedRuns(kind, truth_arr, prior_arr, hyp, agents, iterations, positions, sigma_n, uniforms, noise, noise_rngs)
+    br = BatchedRuns(kind, truth_arr, prior_arr, hyp, agents, iterations, positions, sigma_n, uniforms, noise, noise_rngs,
+                     seeds=seeds)
     br.run(use_graph=use_graph)          # use_graph: the whole device-resident loop replayed from one CUDA graph
     logs = br.logs(sim_nums, exact_tie_loss)
     np.asarray(positions)[...] = br.final_positions()
